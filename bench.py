@@ -18,6 +18,10 @@ One JSON line on stdout (rank 0).  A "step" is one outer iteration over the whol
   cpu_baseline  = the reference's race-free `omp-pmf-train-rf` (oracle/_ref) on two bounded user samples, extrapolated with
                   the affine model t(n) = a + b n they determine (the plain nnz-ratio figure is kept as `linear_value`);
   parity        = the engine vs the unmodified reference (race-free harness) on the first ~2 M ratings of the same data.
+
+--dump-outputs DIR writes what the timed path returned after its last step (objective, counters, U and V; rows of a
+factor larger than its budget are a fixed seeded sample, indices beside them) as DIR/*.npy, so two builds can be compared
+output for output: the workload and the init are deterministic functions of the arguments.
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing of a bench run lands in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -315,6 +320,36 @@ def shim_e2e(shard, args, iters):
                     "H2D, setup, Iter-0 objective + %d iterations, D2H, un-flattening) / iterations" % iters}
 
 
+# --------------------------------------------------------------------------------------------- output dump
+
+# per-factor byte budgets of --dump-outputs (64 MB in all with the indices): Netflix-shape V (14 MB) fits whole,
+# U (384 MB) is sampled
+DUMP_U_BYTES, DUMP_V_BYTES = 32_000_000, 24_000_000
+DUMP_SEED = 20170813
+
+
+def dump_rows(n, k, budget, seed):
+    """Sorted row indices of an (n, k) float64 factor to dump: all of them if they fit `budget` bytes, else a seeded sample."""
+    cap = max(1, budget // (8 * k))
+    if n <= cap:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).choice(n, size=cap, replace=False))
+
+
+def dump_outputs(path, obj, counters, U_rows, U, V, k):
+    """Writes the last step's outputs as float64 .npy files: objective (1,), counters (8, api.Counters order; rank 0's), U / V
+    rows and their global indices."""
+    os.makedirs(path, exist_ok=True)
+    v_rows = dump_rows(V.shape[0], k, DUMP_V_BYTES, DUMP_SEED + 1)
+    out = {"objective": np.array([obj], np.float64),
+           "counters": np.array(list(counters.values()), np.float64),
+           "U": U, "U_rows": U_rows.astype(np.float64), "V": V[v_rows], "V_rows": v_rows.astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, np.float64))
+    log("[bench] outputs of the last timed step written to %s (%s, %.1f MB)" % (
+        path, ", ".join("%s%s" % (n, list(a.shape)) for n, a in out.items()), sum(a.nbytes for a in out.values()) / 1e6))
+
+
 # --------------------------------------------------------------------------------------------- our arm
 
 def main_ours(args):
@@ -418,6 +453,13 @@ def main_ours(args):
     prof = eng.profile()
     eng.profile_enable(False)
     dev_bytes = eng.device_bytes()
+    dump = None
+    if args.dump_outputs:       # copied back after the timed window
+        U_out, V_out = eng.get_factors()
+        rows = dump_rows(ds.d1, k, DUMP_U_BYTES, DUMP_SEED)
+        rows = rows[(rows >= u0) & (rows < u1)]
+        dump = (rows, U_out[rows - u0], V_out)
+        del U_out
     eng.close(); del eng
     torch.cuda.empty_cache()
 
@@ -451,6 +493,14 @@ def main_ours(args):
         gathered = [None] * world
         dist.all_gather_object(gathered, mine)
         per_rank = gathered
+    if dump is not None:
+        rows, U_rows = dump[0], dump[1]
+        if world > 1:           # each rank holds the sampled rows of its own users
+            parts = [None] * world
+            dist.all_gather_object(parts, (rows, U_rows))
+            rows = np.concatenate([p[0] for p in parts]); U_rows = np.concatenate([p[1] for p in parts])
+        if rank == 0:
+            dump_outputs(args.dump_outputs, objs[-1], counters[-1], rows, U_rows, dump[2], k)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -566,7 +616,11 @@ def main():
                     help="ratings in the reference's timing sample (0: 10 %% of the workload, less if that would not fit the run)")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline and parity legs")
     ap.add_argument("--no-shim-e2e", action="store_true", help="skip the e2e run through the C++ drop-in shim")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     global METRIC
     if not (args.workload == "netflix" and args.k == 100):
         METRIC = "sec_per_outer_iter_primalcrpp_k%d_%s_shape" % (args.k, args.workload)

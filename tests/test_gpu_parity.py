@@ -242,8 +242,6 @@ def test_line_search_branches(stepsize, solver):
                                               ("ml1m", 100, 5000.0, 1)])
 def test_training_trajectory(name, k, lam, iters, solver):
     """The pcrpp()/pcr() driver: objective per outer iteration, pairwise error and NDCG@10 vs the oracle."""
-    if name == "ml1m" and solver == 1:
-        pytest.skip("the O(len^2) CPU oracle of Primal-CR on ml1m-shape takes minutes; covered by the golden test")
     ds = dataset(name)
     U, V = init_factors(ds.d1, ds.d2, k)
     O = ob.oracle()
