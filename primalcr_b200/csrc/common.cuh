@@ -93,8 +93,8 @@ struct Profiler {
 // RAII device buffer bookkeeping.  Stream-ordered allocation (cudaMallocAsync from the device's default memory pool,
 // release threshold raised so that freed blocks are kept for the next engine of the process): a plain cudaMalloc gets
 // ~10x slower once NCCL has enabled peer access, because every allocation is then mapped into all peers
-// (measured at 2 GPUs: 0.74 s for the ~100 buffers of a 50 M-rating shard vs 0.08 s).  PRIMALCR_SYNC_ALLOC=1 restores
-// cudaMalloc / cudaFree.
+// (measured at 2 GPUs: 0.74 s for the ~100 buffers of a 50 M-rating shard vs 0.08 s).  Falls back to cudaMalloc / cudaFree
+// when the default memory pool cannot be obtained.
 struct DevPool {
     std::vector<void *> ptrs;
     i64 bytes = 0;
@@ -102,13 +102,11 @@ struct DevPool {
     bool async = false;
     void init(cudaStream_t s) {
         stream = s;
-        async = getenv("PRIMALCR_SYNC_ALLOC") == nullptr;
-        if (async) {
-            int dev = 0; cudaMemPool_t mp;
-            if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetDefaultMemPool(&mp, dev) != cudaSuccess) { async = false; cudaGetLastError(); return; }
-            unsigned long long keep = ~0ull;
-            cudaMemPoolSetAttribute(mp, cudaMemPoolAttrReleaseThreshold, &keep);
-        }
+        int dev = 0; cudaMemPool_t mp;
+        if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetDefaultMemPool(&mp, dev) != cudaSuccess) { cudaGetLastError(); return; }
+        async = true;
+        unsigned long long keep = ~0ull;
+        cudaMemPoolSetAttribute(mp, cudaMemPoolAttrReleaseThreshold, &keep);
     }
     void *raw_alloc(size_t b) {
         void *p = nullptr;
@@ -160,9 +158,7 @@ struct DevCsr {
     i64 *pt_ptr = nullptr;       // [d1+1] first work item of each user
     // row-sum work units over this CSR (segments = users)
     int32_t *un_seg = nullptr; i64 *un_start = nullptr; i64 n_units = 0;   // un_start[n_units+1]
-    i64 *un_end = nullptr;       // only when the units are item-block ordered (then un_start is not contiguous)
     i64 *seg_unit_ptr = nullptr; // [d1+1]
-    int32_t *seg_unit_idx = nullptr;   // unit ids grouped by user (item-block order), else nullptr
 };
 
 struct SortedMeta {          // per rating, in (user, ascending score) order

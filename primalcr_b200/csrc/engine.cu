@@ -69,7 +69,7 @@ struct Engine {
     primalcr_config cfg;
     cudaStream_t stream = nullptr;
     // side stream: the chunk-parallel heavy-user kernels (few, small grids) run beside the tile kernels of the same stage
-    cudaStream_t aux = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr; Ctx ctx_aux; bool use_aux = false;
+    cudaStream_t aux = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr; Ctx ctx_aux;
     Profiler prof;
     DevPool pool;
     Ctx ctx;
@@ -86,7 +86,7 @@ struct Engine {
     // CSC of the training set (by item)
     i64 *col_ptr = nullptr; int32_t *csc_user = nullptr, *csc2csr = nullptr;
     int32_t *cu_seg = nullptr; i64 *cu_start = nullptr, *cu_end = nullptr; i64 n_cunits = 0; i64 *col_unit_ptr = nullptr;
-    int32_t *col_unit_idx = nullptr; int n_user_blocks = 1, n_item_blocks = 1;
+    int32_t *col_unit_idx = nullptr; int n_user_blocks = 1;
     // multi-GPU, large item sets: V-side vectors are reduce-scattered by item rows, the CG algebra runs on this rank's row
     // slice and the search direction is all-gathered (see update_V); d2p = d2 rounded up to a multiple of the world size
     bool sharded_cg = false; i64 d2p = 0, vs_row0 = 0, vs_rows = 0;
@@ -146,7 +146,6 @@ struct Engine {
         }
         PCR_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
         PCR_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
-        use_aux = getenv("PRIMALCR_NO_AUX_STREAM") == nullptr;
         k = cfg.k; ld = ceil4(k);
         PCR_CUDA(cudaMallocHost(&h_slots, sizeof(double) * 32));
         PCR_CUDA(cudaMallocHost(&h_counters, sizeof(int) * 4));
@@ -174,7 +173,6 @@ struct Engine {
     }
     void bind() { PCR_CUDA(cudaSetDevice(cfg.device)); }
     // heavy-user work of a stage goes to the side stream between fork and join (disjoint users => disjoint outputs)
-    bool heavy_on_aux() const { return use_aux && heavy_chunked && X.n_cls[2] > 0; }
     void fork_aux() { PCR_CUDA(cudaEventRecord(ev_fork, stream)); PCR_CUDA(cudaStreamWaitEvent(aux, ev_fork, 0)); }
     void join_aux() { PCR_CUDA(cudaEventRecord(ev_join, aux)); PCR_CUDA(cudaStreamWaitEvent(stream, ev_join, 0)); }
     void sync() { PCR_CUDA(cudaStreamSynchronize(stream)); prof.resolve(); }
@@ -316,7 +314,7 @@ struct Engine {
         std::vector<int32_t> cls[3];
         std::vector<i64> hoff((size_t)d1, -1), hb, he;
         i64 htot = 0;
-        use_tiles = (T <= 8) && (getenv("PRIMALCR_NO_TILES") == nullptr);
+        use_tiles = T <= 8;
         // tiles: runs of consecutive users; geometry 0 takes users with len <= TILE_CAP, geometry 1 users with
         // TILE_CAP < len <= TILE_CAP_M, geometry 2 users with TILE_CAP_M < len <= TILE_CAP_L; anything longer is heavy
         struct Builder { std::vector<int32_t> first, num; i64 cur_first = -1, cur_nnz = 0, cur_users = 0, nnz = 0; i64 cap;
@@ -325,11 +323,10 @@ struct Engine {
             void add(i64 u, i64 len) { if (cur_first >= 0 && (cur_nnz + len > cap || cur_users + 1 > TILE_MAX_USERS)) close();
                                        if (cur_first < 0) cur_first = u; cur_nnz += len; cur_users += 1; } };
         Builder tb[3]; tb[0].cap = TILE_CAP; tb[1].cap = TILE_CAP_M; tb[2].cap = TILE_CAP_L;
-        const bool one_geometry = getenv("PRIMALCR_NO_TILE_M") != nullptr;     // A/B: medium users in the large tiles
         for (i64 u = 0; u < d1; ++u) {
             const i64 len = X.h_row_ptr[u + 1] - X.h_row_ptr[u];
             if (use_tiles && len <= TILE_CAP) { tb[1].close(); tb[2].close(); tb[0].add(u, len); continue; }
-            if (use_tiles && T <= 5 && len <= TILE_CAP_M && !one_geometry) { tb[0].close(); tb[2].close(); tb[1].add(u, len); continue; }   // T>5: smem
+            if (use_tiles && T <= 5 && len <= TILE_CAP_M) { tb[0].close(); tb[2].close(); tb[1].add(u, len); continue; }   // T>5: smem
             if (use_tiles && T <= 5 && len <= TILE_CAP_L) { tb[0].close(); tb[1].close(); tb[2].add(u, len); continue; }
             tb[0].close(); tb[1].close(); tb[2].close();
             if (len == 0) continue;
@@ -368,7 +365,7 @@ struct Engine {
             hsort.tmp_s = pool.alloc<double>((size_t)run); hsort.tmp_pos = pool.alloc<int32_t>((size_t)run);
             sync();
         }
-        heavy_chunked = use_tiles && getenv("PRIMALCR_NO_LM") == nullptr && getenv("PRIMALCR_HEAVY_LEGACY") == nullptr && !cls[2].empty();
+        heavy_chunked = use_tiles && !cls[2].empty();
         if (heavy_chunked) {
             std::vector<i64> hoff_h; std::vector<int32_t> cu, clo, c0;
             for (size_t q = 0; q < cls[2].size(); ++q) {
@@ -388,49 +385,10 @@ struct Engine {
             hv.csum = pool.alloc<double>((size_t)hv.n_chunks * 2);
             sync();
         } else {
-            alloc_heavy_legacy();
+            alloc_heavy_cta_scratch();
         }
         // ---- row-sum work units over the CSR
-        const double blk_bytes = getenv("PRIMALCR_UBLOCK_MB") ? atof(getenv("PRIMALCR_UBLOCK_MB")) * 1e6 : 24e6;
-        const double v_bytes = (double)d2 * ld * 8.0;
-        if (v_bytes > 4.0 * blk_bytes && getenv("PRIMALCR_ITEM_BLOCKS") != nullptr) {
-            // OPT-IN EXPERIMENT (PRIMALCR_ITEM_BLOCKS=1): when V does not fit L2 (Yahoo shape, 500 MB) order the
-            // user-major units ITEM-BLOCK-major so that the V rows gathered by dots / the user-major row sum come from one
-            // <= 24 MB block at a time (items ascend inside a user, so a user's entries of one block are contiguous) --
-            // the mirror image of the CSC user blocks below.  Measured on the full Yahoo shape: 1.26 s vs 1.14 s per
-            // iteration WITHOUT it: 21 blocks x 1 M users give 21 M units of ~12 ratings, and re-fetching the user's row
-            // per unit costs more than the L2 hits save.  Off by default; parity-tested.
-            int nb = (int)std::ceil(v_bytes / blk_bytes);
-            if (nb > 64) nb = 64;
-            const i64 bi = (d2 + nb - 1) / nb;
-            n_item_blocks = nb;
-            std::vector<i64> bpos((size_t)d1 * (nb + 1));
-            i64 *bpos_d = nullptr;
-            bpos_d = (i64 *)pool.raw_alloc(sizeof(i64) * std::max<size_t>(bpos.size(), 1));
-            k_csc_block_bounds(ctx, X.row_ptr, X.item, d1, nb, bi, bpos_d);
-            PCR_CUDA(cudaMemcpyAsync(bpos.data(), bpos_d, sizeof(i64) * bpos.size(), cudaMemcpyDeviceToHost, stream));
-            sync();
-            pool.raw_free(bpos_d);
-            std::vector<int32_t> useg, uidx; std::vector<i64> ustart, uend, supt((size_t)d1 + 1, 0);
-            useg.reserve((size_t)d1 * 4); ustart.reserve((size_t)d1 * 4); uend.reserve((size_t)d1 * 4);
-            for (int blk = 0; blk < nb; ++blk)
-                for (i64 u = 0; u < d1; ++u) {
-                    const i64 lo = bpos[(size_t)u * (nb + 1) + blk];
-                    const i64 hi = blk + 1 == nb ? X.h_row_ptr[u + 1] : bpos[(size_t)u * (nb + 1) + blk + 1];
-                    for (i64 bb = lo; bb < hi; bb += ROWSUM_CHUNK) {
-                        useg.push_back((int32_t)u); ustart.push_back(bb); uend.push_back(std::min<i64>(bb + ROWSUM_CHUNK, hi));
-                        supt[u + 1] += 1;
-                    }
-                }
-            X.n_units = (i64)useg.size();
-            for (i64 u = 0; u < d1; ++u) supt[u + 1] += supt[u];
-            uidx.resize(useg.size());
-            std::vector<i64> fill(supt.begin(), supt.end() - 1);
-            for (size_t q = 0; q < useg.size(); ++q) uidx[fill[useg[q]]++] = (int32_t)q;
-            X.un_seg = upload_vec(useg); X.un_start = upload_vec(ustart); X.un_end = upload_vec(uend);
-            X.seg_unit_ptr = upload_vec(supt); X.seg_unit_idx = upload_vec(uidx);
-            sync();
-        } else {
+        {
             std::vector<int32_t> useg; std::vector<i64> ustart, supt;
             make_units(X.h_row_ptr, useg, ustart, supt);
             X.n_units = (i64)useg.size();
@@ -451,6 +409,7 @@ struct Engine {
         // of <= ~40 MB, so while the persistent grid walks the unit list the gathered rows stay L2-resident
         // (users ascend inside a column, so a column's entries of one block are contiguous).
         {
+            const double blk_bytes = getenv("PRIMALCR_UBLOCK_MB") ? atof(getenv("PRIMALCR_UBLOCK_MB")) * 1e6 : 24e6;
             const double u_bytes = (double)d1 * ld * 8.0;
             int nb = (int)std::ceil(u_bytes / blk_bytes);
             // ... but never so many blocks that an (item, user block) unit averages fewer than ~32 ratings: with many
@@ -500,7 +459,7 @@ struct Engine {
         meta.ub = pool.alloc<int32_t>((size_t)nnz); meta.lb = pool.alloc<int32_t>((size_t)nnz);
         meta.cnt_lo = pool.alloc<int32_t>((size_t)nnz); meta.cnt_hi = pool.alloc<int32_t>((size_t)nnz);
         meta.nnz = nnz;
-        if (use_tiles && getenv("PRIMALCR_NO_LM") == nullptr) {     // level-major copy for the tile users
+        if (use_tiles) {     // level-major copy for the tile users
             meta.lm_s = pool.alloc<double>((size_t)nnz);
             meta.lm_w0 = pool.alloc<unsigned long long>((size_t)nnz); meta.lm_w1 = pool.alloc<unsigned long long>((size_t)nnz);
             if (T > 5) meta.lm_w2 = pool.alloc<unsigned long long>((size_t)nnz);
@@ -539,7 +498,7 @@ struct Engine {
         has_train = true;
     }
 
-    void alloc_heavy_legacy() {
+    void alloc_heavy_cta_scratch() {
         if (h_v != nullptr || X.heavy_total <= 0) return;
         const size_t htot = (size_t)X.heavy_total;
         h_v = pool.alloc<double>(htot); h_p1 = pool.alloc<double>(htot);
@@ -550,7 +509,7 @@ struct Engine {
     // chunk-parallel path is on (the sweeps use the level-major ranks)
     void ensure_heavy_windows() {
         if (!heavy_chunked || heavy_windows_valid || X.n_cls[2] == 0) return;
-        alloc_heavy_legacy();
+        alloc_heavy_cta_scratch();
         k_windows(ctx, 2, X.cls_users[2], X.n_cls[2], nullptr, X.row_ptr, meta, T, X.heavy_off, h_cnt);
         heavy_windows_valid = true;
     }
@@ -642,14 +601,12 @@ struct Engine {
     // out[e] = P[user(e)] . Q[item(e)] over the training set
     void train_dots(const double *P, const double *Q, double *out, const uint8_t *active) {
         const double bytes = active ? 0.0 : pass_bytes(X.nnz, d1);
-        if (!k_dots_units(ctx, X.un_seg, X.un_start, X.un_end, X.n_units, P, Q, X.item, ld, k, active, out, bytes))
-            k_dots(ctx, P, X.user, Q, X.item, X.nnz, ld, k, active, out, bytes);
+        k_dots_units(ctx, X.un_seg, X.un_start, nullptr, X.n_units, P, Q, X.item, ld, k, active, out, bytes);
     }
     // get_sorted_mm + window pointers for every (active) user
     void prepare(const double *sc, const uint8_t *active) {
-        const bool par = heavy_on_aux();
-        Ctx &hc = par ? ctx_aux : ctx;
-        if (par) fork_aux();
+        Ctx &hc = heavy_chunked ? ctx_aux : ctx;
+        if (heavy_chunked) fork_aux();
         if (X.n_cls[2] > 0) {
             k_heavy_sort(hc, hsort, sc, meta.s, meta.pos);
             k_gather_level(hc, X.cls_users[2], X.n_cls[2], nullptr, X.row_ptr, X.level, meta);
@@ -662,27 +619,25 @@ struct Engine {
             if (q == 2 && heavy_chunked) continue;
             k_windows(ctx, q, X.cls_users[q], X.n_cls[q], q == 2 ? nullptr : active, X.row_ptr, meta, T, X.heavy_off, h_cnt);
         }
-        if (par) join_aux();
+        if (heavy_chunked) join_aux();
         heavy_windows_valid = false;
         meta_valid = true;
     }
     void sweep_coeff(int mode, const uint8_t *active, const double *bsrc) {
-        const bool par = heavy_on_aux();
-        if (par) { fork_aux(); k_heavy_sweep(ctx_aux, mode, hv, active, meta, bsrc, cbuf, nullptr, T); }
+        if (heavy_chunked) { fork_aux(); k_heavy_sweep(ctx_aux, mode, hv, active, meta, bsrc, cbuf, nullptr, T); }
         for (int gq = 0; gq < 3; ++gq) k_tile_sweep(ctx, mode, X, gq, active, meta, bsrc, cbuf, nullptr, T);
-        if (par) join_aux();
+        if (heavy_chunked) join_aux();
         for (int q = 0; q < 3; ++q) {
-            if (q == 2 && heavy_chunked) { if (!par) k_heavy_sweep(ctx, mode, hv, active, meta, bsrc, cbuf, nullptr, T); continue; }
+            if (q == 2 && heavy_chunked) continue;
             k_sweep_coeff(ctx, q, mode, X.cls_users[q], X.n_cls[q], active, X.row_ptr, meta, bsrc, cbuf, T, X.heavy_off, h_v, h_p1, h_acc);
         }
     }
     void sweep_obj(const uint8_t *active) {
-        const bool par = heavy_on_aux();
-        if (par) { fork_aux(); k_heavy_sweep(ctx_aux, 2, hv, active, meta, nullptr, nullptr, us.loss, T); }
+        if (heavy_chunked) { fork_aux(); k_heavy_sweep(ctx_aux, 2, hv, active, meta, nullptr, nullptr, us.loss, T); }
         for (int gq = 0; gq < 3; ++gq) k_tile_sweep(ctx, 2, X, gq, active, meta, nullptr, nullptr, us.loss, T);
-        if (par) join_aux();
+        if (heavy_chunked) join_aux();
         for (int q = 0; q < 3; ++q) {
-            if (q == 2 && heavy_chunked) { if (!par) k_heavy_sweep(ctx, 2, hv, active, meta, nullptr, nullptr, us.loss, T); continue; }
+            if (q == 2 && heavy_chunked) continue;
             k_sweep_obj(ctx, q, X.cls_users[q], X.n_cls[q], active, X.row_ptr, meta, us.loss, T, X.heavy_off, h_p1, h_p2, h_acc);
         }
     }
@@ -740,7 +695,7 @@ struct Engine {
     }
     // out[i] = lambda*x[i] + sum over user i of cbuf[e] * V[item(e)]   (U-side gradient / Hessian-vector product)
     void rowsum_users(const double *x, double *out, const uint8_t *active, int zero_if_empty) {
-        k_rowsum(ctx, X.un_seg, X.un_start, X.un_end, X.n_units, X.seg_unit_ptr, X.seg_unit_idx, d1, X.item, nullptr, cbuf, V, ld,
+        k_rowsum(ctx, X.un_seg, X.un_start, nullptr, X.n_units, X.seg_unit_ptr, nullptr, d1, X.item, nullptr, cbuf, V, ld,
                  active, partial, cfg.lambda, x, out, zero_if_empty, active ? 0.0 : pass_bytes(X.nnz, d1), k);
     }
 
@@ -877,7 +832,7 @@ struct Engine {
         if (cfg.solver == 2 && !meta_valid) prepare(m, nullptr);
         // m holds scores(U, V) for every user (not the scores of a rejected V trial): then what the line search leaves
         // behind is valid for the next update_V (see there)
-        const bool m_covers_all_users = scores_valid && cfg.solver == 2 && getenv("PRIMALCR_NO_REUSE") == nullptr;
+        const bool m_covers_all_users = scores_valid && cfg.solver == 2;
         // gradient coefficients from m (stale m included, as precompute_ui / obtain_g_u do)
         coeffs(0, nullptr);
         // prev_obj: Primal-CR++ takes it from the same sorted state (objective_u_new :785); Primal-CR recomputes
@@ -899,12 +854,9 @@ struct Engine {
             coeffs(1, us.cg_active);
             zero_counters();
             // unit partials of V_i^T c, then finalize (Hs = lambda s + sum) fused with the user's CG recurrences
-            k_rowsum(ctx, X.un_seg, X.un_start, X.un_end, X.n_units, X.seg_unit_ptr, X.seg_unit_idx, /*n_seg=*/0, X.item, nullptr, cbuf, V, ld,
+            k_rowsum(ctx, X.un_seg, X.un_start, nullptr, X.n_units, X.seg_unit_ptr, nullptr, /*n_seg=*/0, X.item, nullptr, cbuf, V, ld,
                      us.cg_active, partial, cfg.lambda, us.p, us.Hp, 0, 0.0, k);
-            if (!k_u_finalize_cg(ctx, X.seg_unit_ptr, X.seg_unit_idx, partial, us, d1, ld, k, cfg.lambda)) {
-                rowsum_users(us.p, us.Hp, us.cg_active, 0);
-                k_u_cg_step(ctx, us, d1, ld);
-            }
+            k_u_finalize_cg(ctx, X.seg_unit_ptr, partial, us, d1, ld, k, cfg.lambda);
             n_active = read_counter(0);
         }
         // ---- line search: <= 20 halvings per user; the last trial is kept even if it never decreased (:814)
@@ -960,8 +912,7 @@ struct Engine {
     // pair errors from the sorted state (O(len * T)) are possible for the training set of Primal-CR++ whenever the
     // sorted state of the CURRENT scores exists and the ratings are integers (levels == exact ratings), T <= 8
     bool eval_sorted_ok(int which) const {
-        return which == 0 && cfg.solver == 2 && scores_valid && meta_valid && ratings_integer && T <= 8 &&
-               getenv("PRIMALCR_EVAL_ALL_PAIRS") == nullptr;
+        return which == 0 && cfg.solver == 2 && scores_valid && meta_valid && ratings_integer && T <= 8;
     }
     // method: -1 automatic, 0 all-pairs kernel (the reference's O(len^2) loop util.cpp:467-479), 1 sorted-state count
     void eval(int which, double *err, double *ndcg, int method = -1, i64 *err_user_host = nullptr) {

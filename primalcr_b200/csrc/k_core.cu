@@ -185,21 +185,20 @@ static void launch_dots_units(Ctx &c, const int32_t *un_seg, const i64 *un_start
            nch, ld, active, out);
 }
 
-// returns false when no specialisation fits (caller falls back to k_dots)
-bool k_dots_units(Ctx &c, const int32_t *un_seg, const i64 *un_start, const i64 *un_end, i64 n_units, const double *P, const double *Q,
+void k_dots_units(Ctx &c, const int32_t *un_seg, const i64 *un_start, const i64 *un_end, i64 n_units, const double *P, const double *Q,
                   const int32_t *qrow, int ld, int kk, const uint8_t *active, double *out, double bytes) {
-    if (n_units <= 0) return true;
+    if (n_units <= 0) return;
     const int nch = (kk + 1) / 2;
-#define DU(G, NC) launch_dots_units<G, NC>(c, un_seg, un_start, un_end, n_units, P, Q, qrow, nch, ld, active, out, bytes); return true;
+    PCR_REQUIRE(nch <= 128, "rank too large for dots kernel (k <= 256)");
+#define DU(G, NC) launch_dots_units<G, NC>(c, un_seg, un_start, un_end, n_units, P, Q, qrow, nch, ld, active, out, bytes); return;
     if (nch <= 56) {
         switch ((nch + 7) / 8) { case 1: DU(8, 1) case 2: DU(8, 2) case 3: DU(8, 3) case 4: DU(8, 4) case 5: DU(8, 5) case 6: DU(8, 6) default: DU(8, 7) }
     } else if (nch <= 112) {
         switch ((nch + 15) / 16) { case 4: DU(16, 4) case 5: DU(16, 5) case 6: DU(16, 6) default: DU(16, 7) }
-    } else if (nch <= 224) {
-        switch ((nch + 31) / 32) { case 4: DU(32, 4) case 5: DU(32, 5) case 6: DU(32, 6) default: DU(32, 7) }
+    } else {
+        DU(32, 4)
     }
 #undef DU
-    return false;
 }
 
 // ------------------------------------------------------------------ K4: segmented weighted row sums
@@ -333,11 +332,10 @@ void k_rowsum(Ctx &c, const int32_t *un_seg, const i64 *un_start, const i64 *un_
     const char *rs_name = widx ? "rowsum_items" : (active ? "rowsum_users_active" : "rowsum_users");
     if (n_units > 0) {
         PCR_CUDA(cudaMemsetAsync(c.ticket, 0, sizeof(unsigned long long), c.stream));
-        // measured -2.3 % per item-major launch (profiles/experiments/README.md r02_rowsum_l2hint); PRIMALCR_ROWSUM_L2HINT=0 disables
-        static const bool l2hint = getenv("PRIMALCR_ROWSUM_L2HINT") == nullptr || atoi(getenv("PRIMALCR_ROWSUM_L2HINT")) != 0;
+        // L2 hints on the item-major pass only: measured -2.3 % per launch (profiles/experiments/README.md r02_rowsum_l2hint)
 #define RSL(N, H) { const unsigned grid = resident_grid(rowsum_kernel<N, H>, 256, 0, c.sms, (n_units + 7) / 8); \
                   LAUNCH(c, rs_name, bytes, (rowsum_kernel<N, H>), grid, 256, 0, un_seg, un_start, un_end, n_units, c.ticket, ridx, widx, w, M, ld, nch, active, partial); }
-#define RS(N) { if (l2hint && widx) RSL(N, true) else RSL(N, false) }
+#define RS(N) { if (widx) RSL(N, true) else RSL(N, false) }
         switch (NCH) { case 1: RS(1) break; case 2: RS(2) break; case 3: RS(3) break; default: RS(4) break; }
 #undef RS
 #undef RSL
@@ -710,9 +708,6 @@ void k_sweep_obj(Ctx &c, int cls, const int32_t *users, int n_users, const uint8
 __global__ void fill_kernel(double *x, i64 n, double v) {
     for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) x[i] = v;
 }
-__global__ void fill_u8_kernel(uint8_t *x, i64 n, uint8_t v) {
-    for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) x[i] = v;
-}
 // out may alias x or y (in-place CG updates): no __restrict__ here
 __global__ void axpby_kernel(double *out, double a, const double *x, double b, const double *y, i64 n) {
     for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x)
@@ -721,16 +716,15 @@ __global__ void axpby_kernel(double *out, double a, const double *x, double b, c
 
 static const int RED_BLOCKS = 592;   // 4 x 148
 
-// MODE 0: x.y   1: sum x   2: sum x[i] where mask[i]
+// MODE 0: x.y   1: sum x
 template <int MODE>
-__global__ void __launch_bounds__(256) reduce_kernel(const double *__restrict__ x, const double *__restrict__ y,
-                                                     const uint8_t *__restrict__ mask, i64 n, double *__restrict__ partials) {
+__global__ void __launch_bounds__(256) reduce_kernel(const double *__restrict__ x, const double *__restrict__ y, i64 n,
+                                                     double *__restrict__ partials) {
     __shared__ double wsum[8];
     double acc = 0.0;
     for (i64 i = (i64)blockIdx.x * 256 + threadIdx.x; i < n; i += (i64)gridDim.x * 256) {
         if (MODE == 0) acc = fma(x[i], y[i], acc);
-        else if (MODE == 1) acc += x[i];
-        else if (mask[i]) acc += x[i];
+        else acc += x[i];
     }
     const double t = block_sum<256>(acc, wsum);
     if (threadIdx.x == 0) partials[blockIdx.x] = t;
@@ -802,24 +796,16 @@ void k_fill(Ctx &c, double *x, i64 n, double v) {
     if (n <= 0) return;
     LAUNCH(c, "fill", 0.0, fill_kernel, grid_for(n, 1024, c.sms * 8), 256, 0, x, n, v);
 }
-void k_fill_u8(Ctx &c, uint8_t *x, i64 n, uint8_t v) {
-    if (n <= 0) return;
-    LAUNCH(c, "fill_u8", 0.0, fill_u8_kernel, grid_for(n, 1024, c.sms * 8), 256, 0, x, n, v);
-}
 void k_axpby(Ctx &c, double *out, double a, const double *x, double b, const double *y, i64 n) {
     if (n <= 0) return;
     LAUNCH(c, "axpby", 24.0 * n, axpby_kernel, grid_for(n, 1024, c.sms * 8), 256, 0, out, a, x, b, y, n);
 }
 void k_dot(Ctx &c, const double *x, const double *y, i64 n, double *partials, double *slot) {
-    LAUNCH(c, "dot", 16.0 * n, reduce_kernel<0>, RED_BLOCKS, 256, 0, x, y, (const uint8_t *)nullptr, n, partials);
+    LAUNCH(c, "dot", 16.0 * n, reduce_kernel<0>, RED_BLOCKS, 256, 0, x, y, n, partials);
     LAUNCH(c, "reduce_final", 0.0, reduce_final_kernel, 1, 256, 0, partials, RED_BLOCKS, slot);
 }
 void k_sum(Ctx &c, const double *x, i64 n, double *partials, double *slot) {
-    LAUNCH(c, "sum", 8.0 * n, reduce_kernel<1>, RED_BLOCKS, 256, 0, x, (const double *)nullptr, (const uint8_t *)nullptr, n, partials);
-    LAUNCH(c, "reduce_final", 0.0, reduce_final_kernel, 1, 256, 0, partials, RED_BLOCKS, slot);
-}
-void k_sum_active(Ctx &c, const double *x, const uint8_t *mask, i64 n, double *partials, double *slot) {
-    LAUNCH(c, "sum_active", 9.0 * n, reduce_kernel<2>, RED_BLOCKS, 256, 0, x, (const double *)nullptr, mask, n, partials);
+    LAUNCH(c, "sum", 8.0 * n, reduce_kernel<1>, RED_BLOCKS, 256, 0, x, (const double *)nullptr, n, partials);
     LAUNCH(c, "reduce_final", 0.0, reduce_final_kernel, 1, 256, 0, partials, RED_BLOCKS, slot);
 }
 
@@ -830,20 +816,9 @@ __global__ void pad_copy_kernel(const double *__restrict__ src, i64 rows, int k,
         dst[i] = cidx < k ? src[r * k + cidx] : 0.0;
     }
 }
-__global__ void unpad_copy_kernel(const double *__restrict__ src, i64 rows, int k, int ld, double *__restrict__ dst) {
-    const i64 total = rows * k;
-    for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (i64)gridDim.x * blockDim.x) {
-        const i64 r = i / k; const int cidx = (int)(i - r * k);
-        dst[i] = src[r * ld + cidx];
-    }
-}
 void k_pad_copy(Ctx &c, const double *src, i64 rows, int k, int ld, double *dst) {
     if (rows <= 0) return;
     LAUNCH(c, "pad_copy", 0.0, pad_copy_kernel, grid_for(rows * ld, 1024, c.sms * 8), 256, 0, src, rows, k, ld, dst);
-}
-void k_unpad_copy(Ctx &c, const double *src, i64 rows, int k, int ld, double *dst) {
-    if (rows <= 0) return;
-    LAUNCH(c, "unpad_copy", 0.0, unpad_copy_kernel, grid_for(rows * k, 1024, c.sms * 8), 256, 0, src, rows, k, ld, dst);
 }
 
 // ------------------------------------------------------------------ K6: batched per-user Newton-CG bookkeeping
@@ -856,69 +831,9 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
-// after g (d1 x ld) and loss (d1) are known: prev_obj, skip test, CG initial state
-__global__ void __launch_bounds__(256) u_init_kernel(UState s, const double *__restrict__ U, const i64 *__restrict__ row_ptr,
-                                                     const uint8_t *__restrict__ has_pairs, i64 d1, int ld, double lambda) {
-    const int lane = threadIdx.x & 31;
-    const i64 i = ((i64)blockIdx.x * 256 + threadIdx.x) >> 5;
-    if (i >= d1) return;
-    const size_t o = (size_t)i * ld;
-    double gg = 0.0, uu = 0.0;
-    for (int cidx = lane; cidx < ld; cidx += 32) { const double g = s.g[o + cidx], u = U[o + cidx]; gg = fma(g, g, gg); uu = fma(u, u, uu); }
-    gg = warp_sum(gg); uu = warp_sum(uu);
-    const double prev = lambda / 2.0 * uu + s.loss[i];
-    const bool skip = (gg < 0.0001) || (has_pairs != nullptr && !has_pairs[i]);
-    for (int cidx = lane; cidx < ld; cidx += 32) {
-        const double g = s.g[o + cidx];
-        s.delta[o + cidx] = 0.0; s.rr[o + cidx] = -g; s.p[o + cidx] = g;
-        s.Unew[o + cidx] = U[o + cidx];
-    }
-    if (lane == 0) {
-        s.prev_obj[i] = prev; s.obj_new[i] = prev;
-        s.err[i] = sqrt(gg) * 0.01;
-        s.skipped[i] = skip ? 1 : 0; s.cg_active[i] = skip ? 0 : 1; s.ls_active[i] = 0;
-        s.cg_its[i] = 0; s.ls_trials[i] = 0;
-        if (!skip) atomicAdd(&s.counters[0], 1);
-    }
-}
-
-// one CG iteration's scalar/vector updates for users with cg_active (Hp already holds H p)
-__global__ void __launch_bounds__(256) u_cg_step_kernel(UState s, i64 d1, int ld) {
-    const int lane = threadIdx.x & 31;
-    const i64 i = ((i64)blockIdx.x * 256 + threadIdx.x) >> 5;
-    if (i >= d1) return;
-    if (!s.cg_active[i]) return;
-    const size_t o = (size_t)i * ld;
-    double pHp = 0.0, rp = 0.0;
-    for (int cidx = lane; cidx < ld; cidx += 32) {
-        const double p = s.p[o + cidx];
-        pHp = fma(p, s.Hp[o + cidx], pHp); rp = fma(s.rr[o + cidx], p, rp);
-    }
-    pHp = warp_sum(pHp); rp = warp_sum(rp);
-    const double alpha = -1.0 * rp / pHp;
-    double nr = 0.0, rHp = 0.0;
-    for (int cidx = lane; cidx < ld; cidx += 32) {
-        const double p = s.p[o + cidx], hp = s.Hp[o + cidx];
-        s.delta[o + cidx] = s.delta[o + cidx] + p * alpha;
-        const double r = s.rr[o + cidx] + hp * alpha;
-        s.rr[o + cidx] = r;
-        nr = fma(r, r, nr); rHp = fma(r, hp, rHp);
-    }
-    nr = warp_sum(nr); rHp = warp_sum(rHp);
-    const int its = s.cg_its[i] + 1;
-    const bool done = (sqrt(nr) < s.err[i]) || (its >= 10);
-    if (!done) {
-        const double beta = rHp / pHp;
-        for (int cidx = lane; cidx < ld; cidx += 32) s.p[o + cidx] = -s.rr[o + cidx] + s.p[o + cidx] * beta;
-    }
-    if (lane == 0) {
-        s.cg_its[i] = its;
-        if (done) s.cg_active[i] = 0; else atomicAdd(&s.counters[0], 1);
-    }
-}
-
-// Register-resident variants of the two kernels above for ld <= 64 * NV doubles: every lane owns NV 16-byte chunks of
-// the user's k-vectors, each array is read once (all loads issued up front) and written once.
+// after g (d1 x ld) and loss (d1) are known: prev_obj, skip test, CG initial state.  Register-resident for ld <= 64 * NV
+// doubles: every lane owns NV 16-byte chunks of the user's k-vectors, each array is read once (all loads issued up front)
+// and written once.
 template <int NV>
 __global__ void __launch_bounds__(256) u_init_vec_kernel(UState s, const double *__restrict__ U, const i64 *__restrict__ row_ptr,
                                                          const uint8_t *__restrict__ has_pairs, i64 d1, int ld, double lambda) {
@@ -957,63 +872,11 @@ __global__ void __launch_bounds__(256) u_init_vec_kernel(UState s, const double 
     }
 }
 
+// rowsum_finalize (user side) + one CG iteration's updates in one pass: the warp that adds up a user's partial rows into
+// Hp = lambda p + V_i^T c keeps the row in registers and runs the user's CG recurrences on it right away -- Hp is never
+// written or re-read.  Same additions in the same order as rowsum_finalize_kernel.
 template <int NV>
-__global__ void __launch_bounds__(256) u_cg_step_vec_kernel(UState s, i64 d1, int ld) {
-    const int lane = threadIdx.x & 31;
-    const i64 i = ((i64)blockIdx.x * 256 + threadIdx.x) >> 5;
-    if (i >= d1) return;
-    if (!s.cg_active[i]) return;
-    const size_t o = (size_t)i * ld;
-    const int n2 = ld >> 1;
-    double2 *p2 = reinterpret_cast<double2 *>(s.p + o), *r2 = reinterpret_cast<double2 *>(s.rr + o);
-    double2 *d2p = reinterpret_cast<double2 *>(s.delta + o);
-    const double2 *h2 = reinterpret_cast<const double2 *>(s.Hp + o);
-    double2 p[NV], hp[NV], rr[NV], dl[NV];
-#pragma unroll
-    for (int q = 0; q < NV; ++q) {
-        const int c = lane + 32 * q;
-        const double2 z = make_double2(0.0, 0.0);
-        p[q] = c < n2 ? p2[c] : z; hp[q] = c < n2 ? h2[c] : z; rr[q] = c < n2 ? r2[c] : z; dl[q] = c < n2 ? d2p[c] : z;
-    }
-    double pHp = 0.0, rp = 0.0;
-#pragma unroll
-    for (int q = 0; q < NV; ++q) {
-        pHp = fma(p[q].x, hp[q].x, pHp); pHp = fma(p[q].y, hp[q].y, pHp);
-        rp = fma(rr[q].x, p[q].x, rp); rp = fma(rr[q].y, p[q].y, rp);
-    }
-    pHp = warp_sum(pHp); rp = warp_sum(rp);
-    const double alpha = -1.0 * rp / pHp;
-    double nr = 0.0, rHp = 0.0;
-#pragma unroll
-    for (int q = 0; q < NV; ++q) {
-        dl[q].x = dl[q].x + p[q].x * alpha; dl[q].y = dl[q].y + p[q].y * alpha;
-        rr[q].x = rr[q].x + hp[q].x * alpha; rr[q].y = rr[q].y + hp[q].y * alpha;
-        nr = fma(rr[q].x, rr[q].x, nr); nr = fma(rr[q].y, rr[q].y, nr);
-        rHp = fma(rr[q].x, hp[q].x, rHp); rHp = fma(rr[q].y, hp[q].y, rHp);
-    }
-    nr = warp_sum(nr); rHp = warp_sum(rHp);
-    const int its = s.cg_its[i] + 1;
-    const bool done = (sqrt(nr) < s.err[i]) || (its >= 10);
-    const double beta = rHp / pHp;
-#pragma unroll
-    for (int q = 0; q < NV; ++q) {
-        const int c = lane + 32 * q;
-        if (c < n2) {
-            d2p[c] = dl[q]; r2[c] = rr[q];
-            if (!done) p2[c] = make_double2(-rr[q].x + p[q].x * beta, -rr[q].y + p[q].y * beta);
-        }
-    }
-    if (lane == 0) {
-        s.cg_its[i] = its;
-        if (done) s.cg_active[i] = 0; else atomicAdd(&s.counters[0], 1);
-    }
-}
-
-// rowsum_finalize (user side) + u_cg_step in one pass: the warp that adds up a user's partial rows into Hp = lambda p + V_i^T c
-// keeps the row in registers and runs the user's CG recurrences on it right away -- Hp is never written or re-read and one
-// launch per CG round goes away.  Same additions in the same order as the two separate kernels (bit-identical state).
-template <int NV>
-__global__ void __launch_bounds__(256) u_finalize_cg_kernel(const i64 *__restrict__ seg_unit_ptr, const int32_t *__restrict__ seg_unit_idx,
+__global__ void __launch_bounds__(256) u_finalize_cg_kernel(const i64 *__restrict__ seg_unit_ptr,
                                                             const double *__restrict__ partial, UState s, i64 d1, int ld, int kp,
                                                             double lambda) {
     const int lane = threadIdx.x & 31;
@@ -1033,7 +896,7 @@ __global__ void __launch_bounds__(256) u_finalize_cg_kernel(const i64 *__restric
         hp[q] = c < nch ? make_double2(lambda * p[q].x, lambda * p[q].y) : z;        // rowsum_finalize: v = lambda * x ...
     }
     for (i64 u = seg_unit_ptr[i]; u < seg_unit_ptr[i + 1]; ++u) {                    // ... + the unit partials, in list order
-        const double2 *prow = reinterpret_cast<const double2 *>(partial + (size_t)(seg_unit_idx ? seg_unit_idx[u] : u) * ld);
+        const double2 *prow = reinterpret_cast<const double2 *>(partial + (size_t)u * ld);
 #pragma unroll
         for (int q = 0; q < NV; ++q) {
             const int c = lane + 32 * q;
@@ -1074,17 +937,14 @@ __global__ void __launch_bounds__(256) u_finalize_cg_kernel(const i64 *__restric
     }
 }
 
-// returns false when ld is too large for the register-resident form (caller runs finalize + k_u_cg_step instead)
-bool k_u_finalize_cg(Ctx &c, const i64 *seg_unit_ptr, const int32_t *seg_unit_idx, const double *partial, UState &s, i64 d1, int ld,
-                     int kk, double lambda) {
-    if (d1 <= 0) return true;
-    if (ld > 256) return false;
+void k_u_finalize_cg(Ctx &c, const i64 *seg_unit_ptr, const double *partial, UState &s, i64 d1, int ld, int kk, double lambda) {
+    if (d1 <= 0) return;
+    PCR_REQUIRE(ld <= 256, "rank too large for the per-user CG kernels (k <= 256)");
     const unsigned grid = (unsigned)((d1 + 7) / 8);
     const int kp = 2 * ((kk + 1) / 2);
-    if (ld <= 64) LAUNCH(c, "u_finalize_cg", 0.0, u_finalize_cg_kernel<1>, grid, 256, 0, seg_unit_ptr, seg_unit_idx, partial, s, d1, ld, kp, lambda);
-    else if (ld <= 128) LAUNCH(c, "u_finalize_cg", 0.0, u_finalize_cg_kernel<2>, grid, 256, 0, seg_unit_ptr, seg_unit_idx, partial, s, d1, ld, kp, lambda);
-    else LAUNCH(c, "u_finalize_cg", 0.0, u_finalize_cg_kernel<4>, grid, 256, 0, seg_unit_ptr, seg_unit_idx, partial, s, d1, ld, kp, lambda);
-    return true;
+    if (ld <= 64) LAUNCH(c, "u_finalize_cg", 0.0, u_finalize_cg_kernel<1>, grid, 256, 0, seg_unit_ptr, partial, s, d1, ld, kp, lambda);
+    else if (ld <= 128) LAUNCH(c, "u_finalize_cg", 0.0, u_finalize_cg_kernel<2>, grid, 256, 0, seg_unit_ptr, partial, s, d1, ld, kp, lambda);
+    else LAUNCH(c, "u_finalize_cg", 0.0, u_finalize_cg_kernel<4>, grid, 256, 0, seg_unit_ptr, partial, s, d1, ld, kp, lambda);
 }
 
 __global__ void __launch_bounds__(256) u_ls_begin_kernel(UState s, i64 d1, double stepsize0) {
@@ -1158,21 +1018,11 @@ __global__ void __launch_bounds__(256) u_stats_kernel(UState s, const i64 *__res
 
 void k_u_init(Ctx &c, UState &s, const double *U, const i64 *row_ptr, const uint8_t *has_pairs, i64 d1, int ld, double lambda) {
     if (d1 <= 0) return;
-    static const bool scalar = getenv("PRIMALCR_U_SCALAR") != nullptr;     // A/B: the first, 8-byte-per-lane kernels
+    PCR_REQUIRE(ld <= 256, "rank too large for the per-user CG kernels (k <= 256)");
     const unsigned grid = (unsigned)((d1 + 7) / 8);
-    if (!scalar && ld <= 64) LAUNCH(c, "u_init", 0.0, u_init_vec_kernel<1>, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
-    else if (!scalar && ld <= 128) LAUNCH(c, "u_init", 0.0, u_init_vec_kernel<2>, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
-    else if (!scalar && ld <= 256) LAUNCH(c, "u_init", 0.0, u_init_vec_kernel<4>, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
-    else LAUNCH(c, "u_init", 0.0, u_init_kernel, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
-}
-void k_u_cg_step(Ctx &c, UState &s, i64 d1, int ld) {
-    if (d1 <= 0) return;
-    static const bool scalar = getenv("PRIMALCR_U_SCALAR") != nullptr;
-    const unsigned grid = (unsigned)((d1 + 7) / 8);
-    if (!scalar && ld <= 64) LAUNCH(c, "u_cg_step", 0.0, u_cg_step_vec_kernel<1>, grid, 256, 0, s, d1, ld);
-    else if (!scalar && ld <= 128) LAUNCH(c, "u_cg_step", 0.0, u_cg_step_vec_kernel<2>, grid, 256, 0, s, d1, ld);
-    else if (!scalar && ld <= 256) LAUNCH(c, "u_cg_step", 0.0, u_cg_step_vec_kernel<4>, grid, 256, 0, s, d1, ld);
-    else LAUNCH(c, "u_cg_step", 0.0, u_cg_step_kernel, grid, 256, 0, s, d1, ld);
+    if (ld <= 64) LAUNCH(c, "u_init", 0.0, u_init_vec_kernel<1>, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
+    else if (ld <= 128) LAUNCH(c, "u_init", 0.0, u_init_vec_kernel<2>, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
+    else LAUNCH(c, "u_init", 0.0, u_init_vec_kernel<4>, grid, 256, 0, s, U, row_ptr, has_pairs, d1, ld, lambda);
 }
 void k_u_ls_trial(Ctx &c, UState &s, const double *U, i64 d1, int ld, double stepsize0, int first) {
     if (d1 <= 0) return;

@@ -6,7 +6,7 @@
 //
 //   tile_prepare  K2+K3  get_sorted_mm pcrpp.cpp:52-83 as one bitonic sort over (user, score, index) keys, then the
 //                        window pointers and integer level counters of the sweep pcrpp.cpp:214-229
-//   tile_sweep    K3     c_j of obtain_g_new :230-238 / compute_Ha_new :310-318 / obtain_g_u_new :527-535 /
+//   tile_lm_sweep K3     c_j of obtain_g_new :230-238 / compute_Ha_new :310-318 / obtain_g_u_new :527-535 /
 //                        obtain_Hs_new :613-621 and the objective :392-407 / :556-571
 //
 // Per-level exclusive prefix sums S_t(x) = sum_{q<x, l_q=t} v_q of one user are produced by a SEGMENTED blocked scan
@@ -370,49 +370,45 @@ __global__ void __launch_bounds__(TH, TH == 256 ? PCR_PREP_MINB : (TH == 512 ? 2
         ub_out[e0 + i] = ub; lb_out[e0 + i] = lb; lo_out[e0 + i] = clo; hi_out[e0 + i] = chi;
         // level-major copy: rank of this rating in (level, score) order inside its user, and for every OTHER level t the
         // rank where its window ends: B_t + C_t(ub) above, B_t + C_t(lb) below  (B_t = first rank of level t)
-        if (lm.lm_s != nullptr) {
-            int run = 0, r = 0;
-            uint16_t other[TT];
+        int run = 0, r = 0;
+        uint16_t other[TT];
 #pragma unroll
-            for (int t = 0; t < TT; ++t) {
-                other[t] = 0;
-                if (t < T) {
-                    const int *Ct = C + t * SLOTS + base;
-                    if (t == l) r = run + Ct[x];
-                    else other[t] = (uint16_t)(run + (t > l ? Ct[ub] : Ct[lb]));
-                    run += Ct[n];
-                }
+        for (int t = 0; t < TT; ++t) {
+            other[t] = 0;
+            if (t < T) {
+                const int *Ct = C + t * SLOTS + base;
+                if (t == l) r = run + Ct[x];
+                else other[t] = (uint16_t)(run + (t > l ? Ct[ub] : Ct[lb]));
+                run += Ct[n];
             }
-            const i64 gi = e0 + u0 + r;
-            unsigned long long w1 = 0ull, w2 = 0ull;
-#pragma unroll
-            for (int t = 0; t < TT; ++t) {
-                if (t < T && t != l) {
-                    const int slot = t < l ? t : t - 1;
-                    if (slot < 4) w1 |= (unsigned long long)other[t] << (13 * slot);
-                    else          w2 |= (unsigned long long)other[t] << (13 * (slot - 4));
-                }
-            }
-            lm.lm_s[gi] = sj;
-            lm.lm_w0[gi] = (unsigned long long)(tag[i] & 0xFFFFu) | ((unsigned long long)clo << 13) | ((unsigned long long)chi << 26) |
-                           ((unsigned long long)l << 39) | ((unsigned long long)u << 42);
-            lm.lm_w1[gi] = w1;
-            if (TT > 5) lm.lm_w2[gi] = w2;
         }
+        const i64 gi = e0 + u0 + r;
+        unsigned long long w1 = 0ull, w2 = 0ull;
+#pragma unroll
+        for (int t = 0; t < TT; ++t) {
+            if (t < T && t != l) {
+                const int slot = t < l ? t : t - 1;
+                if (slot < 4) w1 |= (unsigned long long)other[t] << (13 * slot);
+                else          w2 |= (unsigned long long)other[t] << (13 * (slot - 4));
+            }
+        }
+        lm.lm_s[gi] = sj;
+        lm.lm_w0[gi] = (unsigned long long)(tag[i] & 0xFFFFu) | ((unsigned long long)clo << 13) | ((unsigned long long)chi << 26) |
+                       ((unsigned long long)l << 39) | ((unsigned long long)u << 42);
+        lm.lm_w1[gi] = w1;
+        if (TT > 5) lm.lm_w2[gi] = w2;
     }
-    if (lm.ulev != nullptr) {
-        for (int w = tid; w < n_users * T; w += TH) {
-            const int u = w / T, t = w - u * T;
-            const int n = ts.ustart[u + 1] - ts.ustart[u];
-            if (ts.uact[u]) lm.ulev[(i64)(first_user + u) * 8 + t] = (uint16_t)(n > 0 ? C[t * SLOTS + ts.ustart[u] + u + n] : 0);
-        }
+    for (int w = tid; w < n_users * T; w += TH) {
+        const int u = w / T, t = w - u * T;
+        const int n = ts.ustart[u + 1] - ts.ustart[u];
+        if (ts.uact[u]) lm.ulev[(i64)(first_user + u) * 8 + t] = (uint16_t)(n > 0 ? C[t * SLOTS + ts.ustart[u] + u + n] : 0);
     }
 }
 
 // ---------------------------------------------------------------- tile_lm_sweep: the sweeps on the level-major copy
 // In (user, level, score) order the ratings of one level form a block, so every per-level prefix S_t(x) is a difference
 // of ONE running prefix G over the user: S_t(x) = G[B_t + C_t(x)] - G[B_t].  A scalar segmented scan replaces the
-// T-vector scan of tile_sweep_kernel, and the look-up positions B_t + C_t(ub|lb) were stored by tile_prepare:
+// T-vector scan, and the look-up positions B_t + C_t(ub|lb) were stored by tile_prepare:
 //   acc_j = sum_{t>l} (G[idx_t] - G[B_t]) + sum_{t<l} (G[B_{t+1}] - G[idx_t]) = K_u[l] + sum_{t>l} G[idx_t] - sum_{t<l} G[idx_t]
 #ifndef PCR_LM_MINB
 #define PCR_LM_MINB 5      // measured with the packed records: 4 -> 21.2, 5 -> 18.5, 6 -> 19.8 ms per iteration (Hv sweeps)
@@ -555,139 +551,7 @@ __global__ void __launch_bounds__(TH, TH == 256 ? PCR_LM_MINB : (TH == 512 ? 2 :
     }
 }
 
-// ---------------------------------------------------------------- tile_sweep
-// MODE 0: gradient coefficient (stream s)   c_j = 2 [ lo (s_j-1) + hi (s_j+1) - acc_j ]
-// MODE 1: Hv coefficient (stream b[pos])    c_j = 2 [ (lo+hi) b_j - acc_j ]
-//         acc_j = sum_{t<l_j} (S_t(n) - S_t(lb_j)) + sum_{t>l_j} S_t(ub_j)
-// MODE 2: per-user loss  sum_j [ hi s_j^2 - 2 s_j sum_{t>l_j} S1_t(ub_j) + sum_{t>l_j} S2_t(ub_j) ],
-//         S1 / S2 = per-level prefixes of (s-1) / (s-1)^2
-template <int MODE, int TT, int TH>
-__global__ void __launch_bounds__(TH) tile_sweep_kernel(const int32_t *__restrict__ tile_first,
-                                                        const int32_t *__restrict__ tile_nusers,
-                                                        const i64 *__restrict__ tile_e0, const int32_t *__restrict__ tile_ne,
-                                                        const uint8_t *__restrict__ active,
-                                                        const i64 *__restrict__ row_ptr, const int32_t *__restrict__ user_of,
-                                                        const double *__restrict__ s_g, const int32_t *__restrict__ pos_g,
-                                                        const uint8_t *__restrict__ lev_g, const int32_t *__restrict__ ub_g,
-                                                        const int32_t *__restrict__ lb_g, const int32_t *__restrict__ lo_g,
-                                                        const int32_t *__restrict__ hi_g, const double *__restrict__ b_g,
-                                                        double *__restrict__ c_out, double *__restrict__ obj_user, int T) {
-    constexpr int CAP = TH * TE, SLOTS = CAP + TILE_MAX_USERS;
-    extern __shared__ __align__(16) unsigned char smraw[];
-    __shared__ TileShared<CAP> ts;
-    __shared__ double wagg[TH / 32 * TT];
-    __shared__ int wflag[TH / 32];
-    // dynamic layout: S[T][SLOTS] f64 | val[CAP] f64 | lev[CAP] u8
-    double *S = reinterpret_cast<double *>(smraw);
-    double *sval = S + T * SLOTS;
-    uint8_t *slev = reinterpret_cast<uint8_t *>(sval + CAP);
-    const int tid = threadIdx.x;
-    const int first_user = tile_first[blockIdx.x], n_users = tile_nusers[blockIdx.x];
-    const i64 e0 = tile_e0[blockIdx.x];
-    const int ne = tile_ne[blockIdx.x];
-    bool users_done = false;
-    if (active) {
-        if (!tile_users<TH>(ts, first_user, n_users, e0, row_ptr, active)) return;
-        users_done = true;
-    }
-    // every global read of the tile is issued up front (striped ownership i = tid + q*TH), the scan and the
-    // look-ups below then run from registers / shared memory only
-    int r_pos[TE], r_ub[TE], r_lb[TE], r_lo[TE], r_hi[TE], r_u[TE];
-    uint8_t r_l[TE];
-    double r_v[TE];
-#pragma unroll
-    for (int q = 0; q < TE; ++q) {
-        const int i = tid + q * TH;
-        r_pos[q] = 0; r_ub[q] = 0; r_lb[q] = 0; r_lo[q] = 0; r_hi[q] = 0; r_u[q] = 0; r_l[q] = 0; r_v[q] = 0.0;
-        if (i < ne) {
-            r_u[q] = user_of[e0 + i] - first_user;
-            r_l[q] = lev_g[e0 + i];
-            r_ub[q] = ub_g[e0 + i];
-            r_hi[q] = hi_g[e0 + i];
-            if (MODE != 2) { r_pos[q] = pos_g[e0 + i]; r_lb[q] = lb_g[e0 + i]; r_lo[q] = lo_g[e0 + i]; }
-            if (MODE != 1) r_v[q] = s_g[e0 + i];
-        }
-    }
-    if (MODE == 1) {
-#pragma unroll
-        for (int q = 0; q < TE; ++q) { const int i = tid + q * TH; if (i < ne) r_v[q] = b_g[r_pos[q]]; }
-    }
-    if (!users_done) tile_users<TH>(ts, first_user, n_users, e0, row_ptr, active);
-#pragma unroll
-    for (int q = 0; q < TE; ++q) {
-        const int i = tid + q * TH;
-        if (i < ne) { ts.ul[i] = (uint8_t)r_u[q]; slev[i] = r_l[q]; sval[i] = MODE == 2 ? r_v[q] - 1.0 : r_v[q]; }
-    }
-    __syncthreads();
-    if (MODE != 2) {
-        tile_level_scan<double, TT, TH>(ts, ne, T, S, wagg, wflag, [&](int i) { return sval[i]; }, [&](int i) { return (int)slev[i]; });
-#pragma unroll
-        for (int q = 0; q < TE; ++q) {
-            const int i = tid + q * TH;
-            if (i >= ne) continue;
-            const int u = r_u[q];
-            if (!ts.uact[u]) continue;
-            const int u0 = ts.ustart[u], n = ts.ustart[u + 1] - u0;
-            const int base = u0 + u, l = r_l[q];
-            double acc = 0.0;
-            for (int t = 0; t < T; ++t) {
-                const double *St = S + t * SLOTS + base;
-                if (t > l) acc += St[r_ub[q]];
-                else if (t < l) acc += St[n] - St[r_lb[q]];
-            }
-            const double lo = (double)r_lo[q], hi = (double)r_hi[q];
-            const double v = r_v[q];
-            const double cc = MODE == 0 ? lo * (v - 1.0) + hi * (v + 1.0) - acc : (lo + hi) * v - acc;
-            c_out[r_pos[q]] = 2.0 * cc;
-        }
-    } else {
-        // pass A: S1 -> acc1, pass B: S2 -> obj_j, pass C: per-user sums
-        double acc1[TE];
-        tile_level_scan<double, TT, TH>(ts, ne, T, S, wagg, wflag, [&](int i) { return sval[i]; }, [&](int i) { return (int)slev[i]; });
-#pragma unroll
-        for (int q = 0; q < TE; ++q) {
-            const int i = tid + q * TH;
-            double a = 0.0;
-            if (i < ne) {
-                const int u = r_u[q];
-                const int base = ts.ustart[u] + u;
-                for (int t = r_l[q] + 1; t < T; ++t) a += S[t * SLOTS + base + r_ub[q]];
-            }
-            acc1[q] = a;
-        }
-        __syncthreads();
-        tile_level_scan<double, TT, TH>(ts, ne, T, S, wagg, wflag, [&](int i) { const double d = sval[i]; return d * d; },
-                                        [&](int i) { return (int)slev[i]; });
-        double objj[TE];
-#pragma unroll
-        for (int q = 0; q < TE; ++q) {
-            const int i = tid + q * TH;
-            double o = 0.0;
-            if (i < ne) {
-                const int u = r_u[q];
-                const int base = ts.ustart[u] + u;
-                double a2 = 0.0;
-                for (int t = r_l[q] + 1; t < T; ++t) a2 += S[t * SLOTS + base + r_ub[q]];
-                const double sj = r_v[q];
-                o = (double)r_hi[q] * (sj * sj) - 2.0 * sj * acc1[q] + a2;
-            }
-            objj[q] = o;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int q = 0; q < TE; ++q) { const int i = tid + q * TH; if (i < ne) sval[i] = objj[q]; }
-        __syncthreads();
-        // per-user totals: one more segmented scan with every element on level 0 (T = 1)
-        tile_level_scan<double, 1, TH>(ts, ne, 1, S, wagg, wflag, [&](int i) { return sval[i]; }, [](int) { return 0; });
-        for (int u = tid; u < n_users; u += TH) {
-            const int n = ts.ustart[u + 1] - ts.ustart[u];
-            if (n > 0 && ts.uact[u]) obj_user[first_user + u] = S[ts.ustart[u] + u + n];
-        }
-    }
-}
-
 static size_t prepare_smem(int T, int cap) { return (size_t)cap * 16 + (size_t)T * (cap + TILE_MAX_USERS) * 4 + (size_t)cap * 4 + 2 * (size_t)cap; }
-static size_t sweep_smem(int T, int cap) { return (size_t)T * (cap + TILE_MAX_USERS) * 8 + (size_t)cap * 8 + cap; }
 
 template <typename K>
 static void set_smem(K kernel, size_t bytes) {
@@ -720,35 +584,19 @@ void k_tile_sweep(Ctx &c, int mode, const DevCsr &X, int geo, const uint8_t *act
     const double per = mode == 2 ? (16 + 8) : (16 + 8 + 8);
     const double bytes = (double)L.nnz * per;
     const unsigned grid = (unsigned)L.n;
-    if (meta.lm_s != nullptr) {          // level-major fast path (scalar segmented scan)
 #define LM_ARGS L.first, L.nusers, L.e0, L.ne, active, X.row_ptr, X.user, meta, b, c_out, obj_user, T
 #define LM_LAUNCH(MODE, TT, TH, NAME) { const size_t sm = ((size_t)(TH * TE + TILE_MAX_USERS) * (MODE == 2 ? 2 : 1) + TH * TE * (MODE == 2 ? 1 : 2)) * 8; \
-        set_smem(tile_lm_sweep_kernel<MODE, TT, TH>, sm); LAUNCH(c, NAME, bytes, (tile_lm_sweep_kernel<MODE, TT, TH>), grid, TH, sm, LM_ARGS); }
+    set_smem(tile_lm_sweep_kernel<MODE, TT, TH>, sm); LAUNCH(c, NAME, bytes, (tile_lm_sweep_kernel<MODE, TT, TH>), grid, TH, sm, LM_ARGS); }
 #define LM_MODE(MODE, NAME)                                                                                         \
-        if (geo == 0)      { if (T <= 5) { LM_LAUNCH(MODE, 5, 256, NAME) } else { LM_LAUNCH(MODE, 8, 256, NAME) } }   \
-        else if (geo == 1) { LM_LAUNCH(MODE, 5, 512, NAME "_M") }                                                    \
-        else               { LM_LAUNCH(MODE, 5, 1024, NAME "_L") }
-        if (mode == 0) { LM_MODE(0, "lm_sweep_grad") }
-        else if (mode == 1) { LM_MODE(1, "lm_sweep_hv") }
-        else { LM_MODE(2, "lm_sweep_obj") }
+    if (geo == 0)      { if (T <= 5) { LM_LAUNCH(MODE, 5, 256, NAME) } else { LM_LAUNCH(MODE, 8, 256, NAME) } }   \
+    else if (geo == 1) { LM_LAUNCH(MODE, 5, 512, NAME "_M") }                                                    \
+    else               { LM_LAUNCH(MODE, 5, 1024, NAME "_L") }
+    if (mode == 0) { LM_MODE(0, "lm_sweep_grad") }
+    else if (mode == 1) { LM_MODE(1, "lm_sweep_hv") }
+    else { LM_MODE(2, "lm_sweep_obj") }
 #undef LM_MODE
 #undef LM_LAUNCH
 #undef LM_ARGS
-        return;
-    }
-#define SW_ARGS L.first, L.nusers, L.e0, L.ne, active, X.row_ptr, X.user, meta.s, meta.pos, meta.lev, meta.ub, meta.lb, meta.cnt_lo, meta.cnt_hi, b, c_out, obj_user, T
-#define SW_LAUNCH(MODE, TT, TH, NAME) { const size_t sm = sweep_smem(T, TH * TE); set_smem(tile_sweep_kernel<MODE, TT, TH>, sm); \
-        LAUNCH(c, NAME, bytes, (tile_sweep_kernel<MODE, TT, TH>), grid, TH, sm, SW_ARGS); }
-#define SW_MODE(MODE, NAME)                                                                                         \
-    if (geo == 0)      { if (T <= 5) SW_LAUNCH(MODE, 5, 256, NAME) else SW_LAUNCH(MODE, 8, 256, NAME) }              \
-    else if (geo == 1) { SW_LAUNCH(MODE, 5, 512, NAME "_M") }                                                        \
-    else               { SW_LAUNCH(MODE, 5, 1024, NAME "_L") }
-    if (mode == 0) { SW_MODE(0, "tile_sweep_grad") }
-    else if (mode == 1) { SW_MODE(1, "tile_sweep_hv") }
-    else { SW_MODE(2, "tile_sweep_obj") }
-#undef SW_MODE
-#undef SW_LAUNCH
-#undef SW_ARGS
 }
 
 }  // namespace pcr

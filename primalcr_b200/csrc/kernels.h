@@ -31,8 +31,8 @@ void k_heavy_sort(Ctx &c, const HeavySortPlan &h, const double *m, double *s_sor
 // out[e] = P[prow[e]] . Q[qrow[e]]  (rows are ld-strided, ld % 4 == 0); skipped when active[prow[e]] == 0
 void k_dots(Ctx &c, const double *P, const int32_t *prow, const double *Q, const int32_t *qrow, i64 n, int ld, int kk,
             const uint8_t *active, double *out, double bytes);
-// same as k_dots for the training set, user-major over row-sum units (P row in registers); false => use k_dots
-bool k_dots_units(Ctx &c, const int32_t *un_seg, const i64 *un_start, const i64 *un_end, i64 n_units, const double *P, const double *Q,
+// same as k_dots for the training set, user-major over row-sum units (P row in registers)
+void k_dots_units(Ctx &c, const int32_t *un_seg, const i64 *un_start, const i64 *un_end, i64 n_units, const double *P, const double *Q,
                   const int32_t *qrow, int ld, int kk, const uint8_t *active, double *out, double bytes);
 // out[seg] = lambda*x[seg] + sum_{e in seg} w[widx ? widx[e] : e] * M[ridx[e]]   (deterministic two-phase)
 // un_end == nullptr: unit u covers [un_start[u], un_start[u+1]); seg_unit_idx == nullptr: a segment's units are contiguous
@@ -60,7 +60,6 @@ void k_sweep_obj(Ctx &c, int cls, const int32_t *users, int n_users, const uint8
                  double *g_acc);
 // dense vector helpers (length n, deterministic reductions into slot[0..])
 void k_fill(Ctx &c, double *x, i64 n, double v);
-void k_fill_u8(Ctx &c, uint8_t *x, i64 n, uint8_t v);
 void k_axpby(Ctx &c, double *out, double a, const double *x, double b, const double *y, i64 n);  // out = a*x + b*y
 void k_dot(Ctx &c, const double *x, const double *y, i64 n, double *partials, double *slot);      // slot = x.y
 void k_sum(Ctx &c, const double *x, i64 n, double *partials, double *slot);
@@ -70,9 +69,7 @@ void k_sum(Ctx &c, const double *x, i64 n, double *partials, double *slot);
 void k_cg_dots2(Ctx &c, const double *p, const double *Hp, const double *rr, i64 n, double *partials, double *slot2);
 void k_cg_update(Ctx &c, double *delta, double *rr, const double *p, const double *Hp, i64 n, const double *slot_in, double *partials,
                  double *slot2_out);
-void k_sum_active(Ctx &c, const double *x, const uint8_t *mask, i64 n, double *partials, double *slot);
 void k_pad_copy(Ctx &c, const double *src, i64 rows, int k, int ld, double *dst);    // compact [rows x k] -> padded
-void k_unpad_copy(Ctx &c, const double *src, i64 rows, int k, int ld, double *dst);  // padded -> compact
 // batched per-user Newton-CG state (one warp per user)
 struct UState {
     double *g, *delta, *rr, *p, *Hp, *Unew;      // [d1 x ld]
@@ -83,10 +80,9 @@ struct UState {
 };
 void k_u_init(Ctx &c, UState &s, const double *U, const i64 *row_ptr, const uint8_t *has_pairs, i64 d1, int ld,
               double lambda);
-void k_u_cg_step(Ctx &c, UState &s, i64 d1, int ld);
-// the user-side rowsum_finalize (Hp = lambda p + unit partials) and k_u_cg_step in one pass; false: ld too large, not launched
-bool k_u_finalize_cg(Ctx &c, const i64 *seg_unit_ptr, const int32_t *seg_unit_idx, const double *partial, UState &s, i64 d1, int ld,
-                     int kk, double lambda);
+// the user-side rowsum_finalize (Hp = lambda p + unit partials, a user's units contiguous) and one CG iteration's
+// scalar / vector updates of every user with cg_active, in one pass
+void k_u_finalize_cg(Ctx &c, const i64 *seg_unit_ptr, const double *partial, UState &s, i64 d1, int ld, int kk, double lambda);
 void k_u_ls_trial(Ctx &c, UState &s, const double *U, i64 d1, int ld, double stepsize0, int first);
 void k_u_ls_check(Ctx &c, UState &s, i64 d1, int ld, double lambda, int last);
 void k_u_commit(Ctx &c, UState &s, double *U, i64 d1, int ld);

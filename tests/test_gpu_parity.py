@@ -541,10 +541,9 @@ def test_bad_inputs_are_rejected():
 
 @pytest.mark.parametrize("name,k", [("tiny", 7), ("ragged", 10)])
 def test_l2_block_ordered_work_lists(name, k, monkeypatch):
-    """With a (artificially tiny) L2 block size both work lists switch to their blocked order -- CSC units user-block-major,
-    user units item-block-major (the Yahoo / power-law shapes take this path at full size): results must not change."""
+    """With a (artificially tiny) L2 block size the CSC work units switch to their user-block-major order (the Yahoo /
+    power-law shapes take this path at full size): results must not change."""
     monkeypatch.setenv("PRIMALCR_UBLOCK_MB", "0.002")
-    monkeypatch.setenv("PRIMALCR_ITEM_BLOCKS", "1")
     ds = dataset(name)
     lam = 25.0
     e, U, V = make_engine(ds, k, lam, test=False)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """A/B measurement helper (never a bench number): one engine on the named shape, `--warmup` untimed outer iterations,
 then `--iters` iterations timed with CUDA events on the engine's stream and the per-kernel CUDA-event table.  The variant
-is whatever the environment selects (PRIMALCR_* switches, PRIMALCR_LIB); `--tag` labels the JSON line."""
+is the library PRIMALCR_LIB names (default: the in-tree build); `--tag` labels the JSON line."""
 import argparse
 import json
 import os
