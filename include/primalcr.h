@@ -151,6 +151,26 @@ int64_t primalcr_device_bytes(primalcr_engine *e);                /* device memo
 int primalcr_predict(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int32_t *user,
                      const int32_t *item, int64_t n, double *out, int device);
 
+/* ---- top-N recommendation: for each requested user, the topn items of highest U[u] . V[i] over all d2 items, skipping
+   the items of that user's row in an optional exclusion CSR (normally the training set). U is d1 x k, V is d2 x k,
+   row-major host arrays, as for primalcr_predict.
+   - Order: sorted by score, highest first; ties go to the smaller item id.  Scores compare as doubles (+0.0 == -0.0);
+     NaN ranks below -inf and NaN scores tie with each other, so the item id decides among them.
+   - A returned item is never in the user's exclusion row and never repeats.  A user with fewer than topn eligible items
+     gets the tail of its row padded with item -1 and score NaN.
+   - A user's row is bit-identical from call to call and does not depend on which other users are in the batch or on
+     n_users: each score is one fixed-order fp64 reduction over k.
+   - 1 <= topn <= 256, 1 <= k <= 256.
+   - Ids out of range, an exclusion row whose items do not ascend (repeats are allowed), excl_row_ptr without excl_item or
+     any other bad argument returns PRIMALCR_EARG before any kernel runs; without a device the call returns PRIMALCR_ECUDA.
+   - The library owns the stream and device memory of the call and releases them before returning. */
+int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2, int k,
+                       const int64_t *excl_row_ptr, const int32_t *excl_item,  /* d1+1 / row_ptr[d1]; both NULL: exclude nothing */
+                       const int32_t *users, int64_t n_users,                  /* 0-based ids, any order, repeats allowed;
+                                                                                  NULL: 0..d1-1, and n_users must be d1 */
+                       int topn, int32_t *items_out, double *scores_out,       /* [n_users x topn] row-major; scores_out may be NULL */
+                       int device);
+
 /* ---- fast host loader for the reference's data directory (meta + ratings files): replaces load() util.cpp:6-25,
    smat_t::load_from_iterator util.h:201-271 and testset_t::load util.h:360-371 (no GPU needed) ------------------ */
 typedef struct primalcr_dataset primalcr_dataset;

@@ -53,7 +53,7 @@ SYMBOLS = [
     "primalcr_grad_U", "primalcr_hv_U", "primalcr_stream", "primalcr_launch_count", "primalcr_profile_enable",
     "primalcr_profile_reset", "primalcr_profile_count", "primalcr_profile_get", "primalcr_device_bytes",
     "primalcr_reference_init", "primalcr_write_text_matrix", "primalcr_predict", "primalcr_load_dir", "primalcr_dataset_info",
-    "primalcr_dataset_csr", "primalcr_dataset_free",
+    "primalcr_dataset_csr", "primalcr_dataset_free", "primalcr_recommend",
 ]
 
 _lib = None
@@ -117,6 +117,8 @@ def lib():
     L.primalcr_reference_init.argtypes = [f64p, C.c_int64, C.c_int64]; L.primalcr_reference_init.restype = None
     L.primalcr_write_text_matrix.argtypes = [C.c_char_p, f64p, C.c_int64, C.c_int]
     L.primalcr_predict.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i32p, i32p, C.c_int64, f64p, C.c_int]
+    L.primalcr_recommend.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i64p, i32p, i32p, C.c_int64, C.c_int, i32p,
+                                     f64p, C.c_int]
     L.primalcr_load_dir.argtypes = [C.c_char_p, C.c_int, C.POINTER(vp)]
     L.primalcr_dataset_info.argtypes = [vp] + [C.POINTER(C.c_int64)] * 4
     L.primalcr_dataset_csr.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
@@ -196,6 +198,35 @@ def predict(U, V, users, items, device: int = 0) -> np.ndarray:
     if rc != 0:
         raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
     return out
+
+
+def recommend(U, V, n: int, exclude: Ratings | None = None, users=None, device: int = 0):
+    """Top-n items of every requested user by U[u] . V[i] over all items, skipping the user's items in `exclude`
+    (normally the training set) -> (items int32 (n_users, n), scores float64 (n_users, n)).
+
+    Rows are sorted best first, ties to the smaller item id, NaN scores last; a user with fewer than n eligible items is
+    padded with item -1 / score NaN.  users: 0-based ids in any order, repeats allowed (default: every user)."""
+    U = np.ascontiguousarray(U, np.float64); V = np.ascontiguousarray(V, np.float64)
+    if U.ndim != 2 or V.ndim != 2 or U.shape[1] != V.shape[1]:
+        raise PrimalCRError("U and V must be 2-D with the same number of columns, got %s and %s" % (U.shape, V.shape))
+    d1, d2, k = U.shape[0], V.shape[0], U.shape[1]
+    rp = it = None
+    if exclude is not None:
+        if exclude.d1 != d1 or exclude.d2 != d2:
+            raise PrimalCRError("exclude is %d x %d, the factors are %d x %d" % (exclude.d1, exclude.d2, d1, d2))
+        rp = np.ascontiguousarray(exclude.row_ptr, np.int64); it = np.ascontiguousarray(exclude.item, np.int32)
+        if len(rp) != d1 + 1 or len(it) < rp[-1]:
+            raise PrimalCRError("exclude: row_ptr needs d1+1 entries and item row_ptr[d1]")
+    if users is not None:
+        users = np.ascontiguousarray(users, np.int32).reshape(-1)
+    n_users = d1 if users is None else len(users)
+    items = np.empty((n_users, max(int(n), 0)), np.int32)
+    scores = np.empty((n_users, max(int(n), 0)), np.float64)
+    rc = lib().primalcr_recommend(U.ctypes.data, d1, V.ctypes.data, d2, k, _ptr(rp), _ptr(it), _ptr(users), n_users,
+                                  int(n), items.ctypes.data, scores.ctypes.data, device)
+    if rc != 0:
+        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    return items, scores
 
 
 @dataclass

@@ -1354,6 +1354,76 @@ int primalcr_predict(const double *U, int64_t d1, const double *V, int64_t d2, i
     API_END
 }
 
+// ---- top-N recommendation ---------------------------------------------------------------------------------------
+int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
+                       const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn, int32_t *items_out,
+                       double *scores_out, int device) {
+    API_BEGIN
+    PCR_REQUIRE(k >= 1 && k <= 256, "rank k out of range [1, 256]");
+    PCR_REQUIRE(topn >= 1 && topn <= 256, "topn out of range [1, 256]");
+    PCR_REQUIRE(d1 >= 0 && d2 >= 0 && d1 <= INT32_MAX && d2 <= INT32_MAX, "d1 / d2 out of range");
+    PCR_REQUIRE((U || d1 == 0) && (V || d2 == 0), "null factor matrix");
+    PCR_REQUIRE(n_users >= 0 && (users || n_users == d1), "users == NULL requires n_users == d1");
+    PCR_REQUIRE(n_users == 0 || items_out, "null items_out");
+    PCR_REQUIRE((excl_row_ptr == nullptr) == (excl_item == nullptr), "excl_row_ptr and excl_item must both be given or both be NULL");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        throw pcr::Error(PRIMALCR_ECUDA, "no CUDA device available: libprimalcr_b200 has no CPU fallback");
+    PCR_REQUIRE(device >= 0 && device < ndev, "bad device ordinal");
+    // every id the kernel reads through is checked here, before anything runs
+    bool bad_user = false;
+    if (users) {
+#pragma omp parallel for reduction(|| : bad_user) schedule(static)
+        for (int64_t t = 0; t < n_users; ++t) bad_user = bad_user || users[t] < 0 || users[t] >= d1;
+    }
+    PCR_REQUIRE(!bad_user, "user id out of range");
+    int64_t ex_nnz = 0;
+    if (excl_row_ptr) {
+        PCR_REQUIRE(excl_row_ptr[0] == 0, "excl_row_ptr[0] must be 0");
+        bool bad_ptr = false, bad_item = false, descending = false;
+#pragma omp parallel for reduction(|| : bad_ptr, bad_item, descending) schedule(dynamic, 4096)
+        for (int64_t u = 0; u < d1; ++u) {
+            const int64_t a = excl_row_ptr[u], b = excl_row_ptr[u + 1];
+            if (b < a) { bad_ptr = true; continue; }
+            for (int64_t e = a; e < b; ++e) {
+                if (excl_item[e] < 0 || excl_item[e] >= d2) { bad_item = true; break; }
+                if (e > a && excl_item[e] < excl_item[e - 1]) { descending = true; break; }
+            }
+        }
+        PCR_REQUIRE(!bad_ptr, "excl_row_ptr decreases");
+        PCR_REQUIRE(!bad_item, "exclusion item id out of range");
+        PCR_REQUIRE(!descending, "exclusion row items must ascend");
+        ex_nnz = excl_row_ptr[d1];
+    }
+    if (n_users == 0) return PRIMALCR_OK;
+    PCR_CUDA(cudaSetDevice(device));
+    pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
+    // declared after the pool, so on every exit the stream is drained and destroyed before the buffers are freed
+    struct StreamGuard { cudaStream_t s = nullptr; ~StreamGuard() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } } } sg;
+    PCR_CUDA(cudaStreamCreateWithFlags(&sg.s, cudaStreamNonBlocking));
+    cudaStream_t st = sg.s;
+    cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
+    ctx.stream = st; ctx.prof = &prof; ctx.sms = prop.multiProcessorCount; ctx.ticket = nullptr;
+    double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = pool.alloc<double>((size_t)d2 * k);
+    int32_t *ud = pool.alloc<int32_t>((size_t)n_users), *itd = pool.alloc<int32_t>((size_t)n_users * topn);
+    double *scd = scores_out ? pool.alloc<double>((size_t)n_users * topn) : nullptr;
+    int64_t *exp_d = nullptr; int32_t *exi_d = nullptr;
+    if (d1) PCR_CUDA(cudaMemcpyAsync(Ud, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
+    if (d2) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
+    if (users) PCR_CUDA(cudaMemcpyAsync(ud, users, sizeof(int32_t) * (size_t)n_users, cudaMemcpyHostToDevice, st));
+    else pcr::k_iota32(ctx, ud, n_users);
+    if (excl_row_ptr) {
+        exp_d = pool.alloc<int64_t>((size_t)d1 + 1); exi_d = pool.alloc<int32_t>((size_t)ex_nnz);
+        PCR_CUDA(cudaMemcpyAsync(exp_d, excl_row_ptr, sizeof(int64_t) * ((size_t)d1 + 1), cudaMemcpyHostToDevice, st));
+        if (ex_nnz) PCR_CUDA(cudaMemcpyAsync(exi_d, excl_item, sizeof(int32_t) * (size_t)ex_nnz, cudaMemcpyHostToDevice, st));
+    }
+    pcr::k_topn(ctx, Ud, Vd, d2, k, (const pcr::i64 *)exp_d, exi_d, ud, n_users, topn, itd, scd);
+    PCR_CUDA(cudaMemcpyAsync(items_out, itd, sizeof(int32_t) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
+    if (scores_out) PCR_CUDA(cudaMemcpyAsync(scores_out, scd, sizeof(double) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
+    PCR_CUDA(cudaStreamSynchronize(st));
+    API_END
+}
+
 // ---- host loader ------------------------------------------------------------------------------------------
 struct primalcr_dataset { pcrhost::DataDir d; };
 

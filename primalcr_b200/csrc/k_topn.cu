@@ -1,0 +1,307 @@
+// k_topn.cu -- top-N recommendation: every requested user scored against every item (fp64 DFMA register tiles) with the
+// per-user selection fused in, so the d1 x d2 score matrix is never written anywhere.
+//
+// A CTA owns BU users and streams V through shared memory in tiles of BI consecutive items, ascending.  Each tile is
+// computed as a small GEMM, k sliced in chunks of KC double-buffered with cp.async, 8 users x 8 items per thread.
+// Scores stay in registers while they are filtered against each user's threshold (the current N-th best entry); the
+// survivors go to a per-user candidate buffer in shared memory, and a buffer that fills (or the end of the item
+// stream) merges the candidates into the user's sorted top-N and raises the threshold.  Excluded items (the user's
+// ascending exclusion row) are masked per tile with a cursor per user, so the cost is O(nnz of the block + tiles).
+//
+// Order: (score descending, item ascending) on a 64-bit key of the score that equates +0.0 / -0.0 and ranks every NaN
+// below -inf (NaNs tie, so the item decides).  Every score is the fma chain acc = fma(U[u][j], V[i][j], acc), j = 0..k-1,
+// from +0.0 -- the same for every class and batch -- and the top-N under a total order is unique, so a user's row does not
+// depend on the batch it is computed in.
+#include "kernels.h"
+
+namespace pcr {
+
+#ifndef FULL
+#define FULL 0xffffffffu
+#endif
+
+typedef unsigned long long u64;
+
+// 1 for NaN, order-preserving above it; 0 is below every key (the "no threshold yet" value)
+__device__ __forceinline__ u64 score_key(double s) {
+    if (s != s) return 1ull;
+    if (s == 0.0) s = 0.0;                       // -0.0 -> +0.0: the two compare equal
+    const u64 b = (u64)__double_as_longlong(s);
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double key_score(u64 key) {
+    if (key == 1ull) return __longlong_as_double(0x7ff8000000000000ll);
+    return __longlong_as_double((long long)((key >> 63) ? (key & 0x7fffffffffffffffull) : ~key));
+}
+// a ranks before b
+__device__ __forceinline__ bool better(u64 ka, int ia, u64 kb, int ib) { return ka > kb || (ka == kb && ia < ib); }
+
+__device__ __forceinline__ void cp_async8(void *smem, const void *gmem, bool valid) {
+    const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;\n" ::"r"(s), "l"(gmem), "r"(valid ? 8 : 0));
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
+template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
+
+// NMAX: largest topn of the class; UG: groups of 8 users (BU = 8 UG users, BI = 2048 / UG items per tile); CAP: candidates
+// buffered per user between merges.  256 threads: thread (ug, ig) computes users ug*8..+7 x items ig + IG*c, c = 0..7.
+template <int NMAX, int UG, int CAP>
+struct TopnCfg {
+    static constexpr int THREADS = 256, WARPS = THREADS / 32;
+    static constexpr int IG = THREADS / UG, BU = 8 * UG, BI = 8 * IG, KC = UG;   // KC * BI = 2048 doubles per V chunk
+    static constexpr int PAD = 32 / KC;          // row padding: the transposing cp.async stores of a warp hit distinct banks
+    static constexpr int VS = KC * (BI + PAD), US = KC * (BU + PAD), MW = BI / 32, SCR = NMAX > CAP ? NMAX : CAP;
+    // 8-byte arrays first, then 4-byte ones
+    static constexpr size_t o_vs = 0, o_us = o_vs + 2 * VS, o_lkey = o_us + 2 * US, o_ckey = o_lkey + BU * NMAX,
+                            o_skey = o_ckey + BU * CAP, o_thr = o_skey + WARPS * SCR, o_cur = o_thr + BU, o_end = o_cur + BU,
+                            n8 = o_end + BU;
+    static constexpr size_t o_litem = 0, o_citem = o_litem + BU * NMAX, o_sitem = o_citem + BU * CAP,
+                            o_thri = o_sitem + WARPS * SCR, o_lcnt = o_thri + BU, o_ccnt = o_lcnt + BU, o_uid = o_ccnt + BU,
+                            o_mask = o_uid + BU, n4 = o_mask + BU * MW;
+    static constexpr size_t smem = n8 * 8 + n4 * 4;
+    static_assert(KC * BI == 2048 && BU * KC <= 2 * THREADS && IG >= 32, "tile shape");
+};
+
+template <int NMAX, int UG, int CAP>
+__global__ void __launch_bounds__(256, 1)
+topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, int k, const i64 *__restrict__ ex_ptr,
+            const int32_t *__restrict__ ex_item, const int32_t *__restrict__ users, i64 n_users, int topn,
+            int32_t *__restrict__ items_out, double *__restrict__ scores_out) {
+    typedef TopnCfg<NMAX, UG, CAP> C;
+    constexpr int BU = C::BU, BI = C::BI, KC = C::KC, IG = C::IG, PAD = C::PAD, MW = C::MW, SCR = C::SCR;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    double *Vs = reinterpret_cast<double *>(smem_raw) + C::o_vs;
+    double *Us = reinterpret_cast<double *>(smem_raw) + C::o_us;
+    u64 *lkey = reinterpret_cast<u64 *>(smem_raw) + C::o_lkey;
+    u64 *ckey = reinterpret_cast<u64 *>(smem_raw) + C::o_ckey;
+    u64 *skey_all = reinterpret_cast<u64 *>(smem_raw) + C::o_skey;
+    u64 *thr_key = reinterpret_cast<u64 *>(smem_raw) + C::o_thr;
+    i64 *cur = reinterpret_cast<i64 *>(smem_raw) + C::o_cur;
+    i64 *cend = reinterpret_cast<i64 *>(smem_raw) + C::o_end;
+    int *i4 = reinterpret_cast<int *>(smem_raw + C::n8 * 8);
+    int *litem = i4 + C::o_litem, *citem = i4 + C::o_citem, *sitem_all = i4 + C::o_sitem, *thr_item = i4 + C::o_thri;
+    int *lcnt = i4 + C::o_lcnt, *ccnt = i4 + C::o_ccnt, *uid = i4 + C::o_uid;
+    unsigned *mask = reinterpret_cast<unsigned *>(i4 + C::o_mask);
+
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int ug = tid / IG, ig = tid % IG;
+    const i64 row0 = (i64)blockIdx.x * BU;
+    const int nrows = (int)(n_users - row0 < BU ? n_users - row0 : BU);
+    u64 *skey = skey_all + warp * SCR;
+    int *sitem = sitem_all + warp * SCR;
+
+    for (int r = tid; r < BU; r += C::THREADS) {
+        const int u = r < nrows ? users[row0 + r] : 0;
+        uid[r] = u; lcnt[r] = 0; ccnt[r] = 0; thr_key[r] = 0ull; thr_item[r] = 0;
+        cur[r] = (ex_ptr && r < nrows) ? ex_ptr[u] : 0;
+        cend[r] = (ex_ptr && r < nrows) ? ex_ptr[u + 1] : 0;
+    }
+    __syncthreads();
+
+    const int nkc = (k + KC - 1) / KC;
+    const int ntiles = (int)((d2 + BI - 1) / BI);
+
+    // chunk kc of item tile t into buffer buf
+    auto load_step = [&](int t, int kc, int buf) {
+        const int k0 = kc * KC;
+        const i64 base = (i64)t * BI;
+        double *vs = Vs + buf * C::VS;
+#pragma unroll
+        for (int j = 0; j < 2048 / C::THREADS; ++j) {
+            const int e = tid + j * C::THREADS, il = e / KC, kk = e % KC;
+            const i64 item = base + il;
+            const bool ok = item < d2 && k0 + kk < k;
+            cp_async8(vs + kk * (BI + PAD) + il, ok ? V + item * k + k0 + kk : V, ok);
+        }
+        double *us = Us + buf * C::US;
+        for (int e = tid; e < BU * KC; e += C::THREADS) {
+            const int r = e / KC, kk = e % KC;
+            const bool ok = r < nrows && k0 + kk < k;
+            cp_async8(us + kk * (BU + PAD) + r, ok ? U + (i64)uid[r] * k + k0 + kk : U, ok);
+        }
+        cp_async_commit();
+    };
+
+    // merge every user's candidates into its sorted top-N (warp per user); caller synchronises before and after
+    auto merge_all = [&]() {
+        for (int r = warp; r < BU; r += C::WARPS) {
+            const int m = min(ccnt[r], CAP);
+            if (m == 0) continue;
+            const u64 *ck = ckey + r * CAP; const int *ci = citem + r * CAP;
+            u64 *lk = lkey + r * NMAX; int *li = litem + r * NMAX;
+            const int nl = lcnt[r];
+            for (int i = lane; i < m; i += 32) {          // candidates sorted by rank counting into the scratch
+                const u64 ka = ck[i]; const int ia = ci[i];
+                int rank = 0;
+                for (int j = 0; j < m; ++j) rank += better(ck[j], ci[j], ka, ia);
+                skey[rank] = ka; sitem[rank] = ia;
+            }
+            __syncwarp();
+            for (int i = lane; i < m; i += 32) { ckey[r * CAP + i] = skey[i]; citem[r * CAP + i] = sitem[i]; }
+            __syncwarp();
+            // merge path: an element's place = its index + the number of entries of the other list that rank before it
+            for (int i = lane; i < nl; i += 32) {
+                const u64 ka = lk[i]; const int ia = li[i];
+                int lo = 0, hi = m;
+                while (lo < hi) { const int mid = (lo + hi) >> 1; if (better(ck[mid], ci[mid], ka, ia)) lo = mid + 1; else hi = mid; }
+                if (i + lo < topn) { skey[i + lo] = ka; sitem[i + lo] = ia; }
+            }
+            for (int j = lane; j < m; j += 32) {
+                const u64 ka = ck[j]; const int ia = ci[j];
+                int lo = 0, hi = nl;
+                while (lo < hi) { const int mid = (lo + hi) >> 1; if (better(lk[mid], li[mid], ka, ia)) lo = mid + 1; else hi = mid; }
+                if (j + lo < topn) { skey[j + lo] = ka; sitem[j + lo] = ia; }
+            }
+            __syncwarp();
+            const int nn = min(nl + m, topn);
+            for (int i = lane; i < nn; i += 32) { lk[i] = skey[i]; li[i] = sitem[i]; }
+            if (lane == 0) {
+                lcnt[r] = nn; ccnt[r] = 0;
+                if (nn == topn) { thr_key[r] = skey[nn - 1]; thr_item[r] = sitem[nn - 1]; }
+            }
+            __syncwarp();
+        }
+    };
+
+    double acc[8][8];
+    int buf = 0;
+    if (ntiles > 0) load_step(0, 0, 0);
+    for (int t = 0; t < ntiles; ++t) {
+        const i64 base = (i64)t * BI;
+        {
+#pragma unroll
+            for (int r = 0; r < 8; ++r)
+#pragma unroll
+                for (int c = 0; c < 8; ++c) acc[r][c] = 0.0;
+            if (ex_ptr) {                                   // exclusion bitmask of this tile
+                for (int e = tid; e < BU * MW; e += C::THREADS) mask[e] = 0u;
+                __syncthreads();
+                const i64 lim = base + BI;
+                for (int r = warp; r < nrows; r += C::WARPS) {
+                    i64 p = cur[r];
+                    const i64 pe = cend[r];
+                    while (true) {
+                        const i64 q = p + lane;
+                        const i64 it = q < pe ? (i64)ex_item[q] : lim;
+                        const bool in = it < lim;
+                        if (in) atomicOr(&mask[r * MW + (int)((it - base) >> 5)], 1u << ((it - base) & 31));
+                        const int n = __popc(__ballot_sync(FULL, in));
+                        p += n;
+                        if (n < 32) break;
+                    }
+                    if (lane == 0) cur[r] = p;
+                }
+            }
+        }
+        for (int kc = 0; kc < nkc; ++kc, buf ^= 1) {
+            // prefetch the next chunk (of this tile, or the first of the next) while this one is computed
+            if (kc + 1 < nkc) { load_step(t, kc + 1, buf ^ 1); cp_async_wait<1>(); }
+            else if (t + 1 < ntiles) { load_step(t + 1, 0, buf ^ 1); cp_async_wait<1>(); }
+            else cp_async_wait<0>();
+            __syncthreads();
+            const double *vs = Vs + buf * C::VS + ig;
+            const double *us = Us + buf * C::US + ug * 8;
+#pragma unroll
+            for (int kk = 0; kk < KC; ++kk) {
+                double a[8], b[8];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const double2 v2 = *reinterpret_cast<const double2 *>(us + kk * (BU + PAD) + 2 * q);
+                    a[2 * q] = v2.x; a[2 * q + 1] = v2.y;
+                }
+#pragma unroll
+                for (int c = 0; c < 8; ++c) b[c] = vs[kk * (BI + PAD) + IG * c];
+#pragma unroll
+                for (int r = 0; r < 8; ++r)
+#pragma unroll
+                    for (int c = 0; c < 8; ++c) acc[r][c] = fma(a[r], b[c], acc[r][c]);
+            }
+            __syncthreads();
+        }
+
+        // ---- selection of this tile's scores
+        u64 pend = ~0ull;
+        auto filter = [&]() {        // keeps the pending scores that are eligible and beat their user's threshold
+            u64 keep = 0ull;
+#pragma unroll
+            for (int r = 0; r < 8; ++r) {
+                const int row = ug * 8 + r;
+                if (row >= nrows) continue;
+                const u64 tk = thr_key[row]; const int ti = thr_item[row];
+#pragma unroll
+                for (int c = 0; c < 8; ++c) {
+                    const int il = ig + IG * c;
+                    const u64 bit = 1ull << (r * 8 + c);
+                    if (!(pend & bit) || base + il >= d2) continue;
+                    if (ex_ptr && ((mask[row * MW + (il >> 5)] >> (il & 31)) & 1u)) continue;
+                    if (better(score_key(acc[r][c]), (int)(base + il), tk, ti)) keep |= bit;
+                }
+            }
+            pend = keep;
+        };
+        filter();
+        while (true) {
+#pragma unroll
+            for (int r = 0; r < 8; ++r)
+#pragma unroll
+                for (int c = 0; c < 8; ++c) {
+                    const u64 bit = 1ull << (r * 8 + c);
+                    if (pend & bit) {
+                        const int row = ug * 8 + r;
+                        const int pos = atomicAdd(&ccnt[row], 1);
+                        if (pos < CAP) {
+                            ckey[row * CAP + pos] = score_key(acc[r][c]);
+                            citem[row * CAP + pos] = (int)(base + ig + IG * c);
+                            pend &= ~bit;
+                        }
+                    }
+                }
+            if (!__syncthreads_or(pend != 0ull)) break;
+            merge_all();             // some buffer is full: merge, raise the thresholds, retry what did not fit
+            __syncthreads();
+            filter();
+        }
+    }
+    __syncthreads();
+    merge_all();
+    __syncthreads();
+    for (int r = warp; r < nrows; r += C::WARPS) {
+        const i64 o = (row0 + r) * topn;
+        const int n = lcnt[r];
+        for (int j = lane; j < topn; j += 32) {
+            const bool have = j < n;
+            items_out[o + j] = have ? litem[r * NMAX + j] : -1;
+            if (scores_out) scores_out[o + j] = have ? key_score(lkey[r * NMAX + j]) : key_score(1ull);
+        }
+    }
+}
+
+template <int NMAX, int UG, int CAP>
+static void launch_topn(Ctx &c, const char *name, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr,
+                        const int32_t *ex_item, const int32_t *users, i64 n_users, int topn, int32_t *items_out,
+                        double *scores_out) {
+    typedef TopnCfg<NMAX, UG, CAP> C;
+    auto kern = topn_kernel<NMAX, UG, CAP>;
+    PCR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
+    const i64 grid = (n_users + C::BU - 1) / C::BU;
+    const double bytes = (double)grid * d2 * k * 8.0 + (double)n_users * (k * 8.0 + topn * 12.0);
+    c.prof->begin(name, c.stream, bytes);
+    kern<<<(unsigned)grid, C::THREADS, C::smem, c.stream>>>(U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out,
+                                                             scores_out);
+    c.prof->end(c.stream);
+    PCR_CUDA(cudaGetLastError());
+}
+
+void k_topn(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr, const int32_t *ex_item,
+            const int32_t *users, i64 n_users, int topn, int32_t *items_out, double *scores_out) {
+    PCR_REQUIRE(topn >= 1 && topn <= 256 && k >= 1 && k <= 256, "topn / k out of range [1, 256]");
+    if (n_users <= 0) return;
+    if (topn <= 32)
+        launch_topn<32, 8, 64>(c, "pcr::topn_kernel<32,8,64>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+    else if (topn <= 128)
+        launch_topn<128, 8, 64>(c, "pcr::topn_kernel<128,8,64>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+    else
+        launch_topn<256, 4, 128>(c, "pcr::topn_kernel<256,4,128>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+}
+
+}  // namespace pcr

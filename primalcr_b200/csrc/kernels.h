@@ -119,4 +119,11 @@ void k_eval_item_to_user(Ctx &c, const DevCsr &X, const i64 *err_item, i64 *err_
 void k_eval_users(Ctx &c, const DevCsr &X, const double *score, const i64 *err_item, int err_per_user, int ndcg_k,
                   double *err_ratio_user, double *ndcg_user, double *has_pair_user, double *has_any_user);
 
+// ---------------------------------------------------------------- k_topn.cu (top-N recommendation)
+// for each of n_users rows users[q]: the topn items of highest U[u] . V[i] (compact rows of k doubles), skipping the items
+// of the user's ascending exclusion row (ex_ptr == nullptr: none); sorted best first, ties to the smaller item, NaN last;
+// rows with fewer eligible items are padded with item -1 / score NaN.  scores_out may be nullptr.  1 <= topn, k <= 256.
+void k_topn(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr, const int32_t *ex_item,
+            const int32_t *users, i64 n_users, int topn, int32_t *items_out, double *scores_out);
+
 }  // namespace pcr
