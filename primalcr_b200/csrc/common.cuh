@@ -148,7 +148,7 @@ struct DevCsr {
     int n_cls[3] = {0, 0, 0};
     i64 *heavy_off = nullptr;    // [d1] offset into the heavy scratch arrays, -1 if not heavy
     i64 heavy_total = 0;         // sum over heavy users of (len + 1)
-    i64 *heavy_begin = nullptr, *heavy_end = nullptr;  // [n_cls[2]] absolute segment bounds (CUB segmented sort)
+    i64 *heavy_begin = nullptr, *heavy_end = nullptr;  // [n_cls[2]] absolute segment bounds (heavy-user sort, k_hsort.cu)
     i64 max_len = 0;
     // tiles of consecutive users: [0] small (<= TILE_CAP ratings in total), [1] medium (users with TILE_CAP < len <= TILE_CAP_M),
     // [2] large (TILE_CAP_M < len <= TILE_CAP_L)

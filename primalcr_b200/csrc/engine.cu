@@ -63,7 +63,7 @@ static std::mutex g_comm_mutex;
 static thread_local std::string g_last_error;
 
 // leading dimension of every factor-shaped array: rows start on 128-byte lines (a 128-byte row chunk never straddles two)
-static int ceil4(int k) { return (k + 15) & ~15; }
+static int ceil16(int k) { return (k + 15) & ~15; }
 
 struct Engine {
     primalcr_config cfg;
@@ -146,7 +146,7 @@ struct Engine {
         }
         PCR_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
         PCR_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
-        k = cfg.k; ld = ceil4(k);
+        k = cfg.k; ld = ceil16(k);
         PCR_CUDA(cudaMallocHost(&h_slots, sizeof(double) * 32));
         PCR_CUDA(cudaMallocHost(&h_counters, sizeof(int) * 4));
         PCR_CUDA(cudaMallocHost(&h_stats, sizeof(i64) * 8));
@@ -1334,7 +1334,7 @@ int primalcr_predict(const double *U, int64_t d1, const double *V, int64_t d2, i
     for (int64_t t = 0; t < n; ++t)
         PCR_REQUIRE(user[t] >= 0 && user[t] < d1 && item[t] >= 0 && item[t] < d2, "user/item id out of range");
     PCR_CUDA(cudaSetDevice(device));
-    const int ld = pcr::ceil4(k);
+    const int ld = pcr::ceil16(k);
     pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
     cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
     cudaStream_t st; PCR_CUDA(cudaStreamCreate(&st));

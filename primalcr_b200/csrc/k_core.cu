@@ -400,7 +400,7 @@ void k_sort_users(Ctx &c, int cls, const int32_t *users, int n_users, const uint
         LAUNCH(c, "sort_users_L", 0.0, (sort_users_kernel<1024, L_CAP>), n_users, 1024, 0, users, n_users, active, row_ptr, m, level, meta.s, meta.pos, meta.lev);
 }
 
-// heavy users: CUB wrote s and pos; fetch the levels
+// heavy users: k_hsort.cu wrote s and pos; fetch the levels
 __global__ void __launch_bounds__(256) gather_level_kernel(const int32_t *__restrict__ users, int n_users,
                                                            const uint8_t *__restrict__ active,
                                                            const i64 *__restrict__ row_ptr,

@@ -12,7 +12,7 @@
 //   idx_t(j) = B_t + #{q in level t : s_q <= fl(s_j + 1.0)}   for t > l_j     (left window, pcrpp.cpp:218)
 //   idx_t(j) = B_t + #{q in level t : s_q <  fl(s_j - 1.0)}   for t < l_j     (right window, pcrpp.cpp:224)
 //
-//   prepare:  CUB segmented sort by score (k_setup.cu) -> level histogram per chunk -> bases -> stable scatter into
+//   prepare:  segmented sort by score (k_hsort.cu) -> level histogram per chunk -> bases -> stable scatter into
 //             (level, score) order -> per-level binary searches for idx_t / cnt_lo / cnt_hi
 //   sweep:    chunk sums of the stream -> per-chunk exclusive scan + base = G -> look-ups -> c_j / objective
 // All sums have a fixed association order (deterministic, independent of the grid schedule).

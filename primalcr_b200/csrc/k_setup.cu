@@ -1,7 +1,7 @@
 // k_setup.cu -- one-time preprocessing on the device (replaces convert() util.cpp:219-274 and the CSR->CSC
-// transpose of smat_t::load_from_iterator util.h:259-270) plus the heavy-user segmented sort.
-// CUB (shipped with the CUDA toolkit) is used here only for set-up sorts/scans and for users whose rating
-// count exceeds the shared-memory sort classes; the per-iteration hot kernels are in k_core.cu.
+// transpose of smat_t::load_from_iterator util.h:259-270).
+// CUB (shipped with the CUDA toolkit) is used here only for the scan and the radix sort of the CSC build; the heavy
+// users are sorted by k_hsort.cu, the per-iteration hot kernels are in k_core.cu.
 #include "kernels.h"
 #include <cub/cub.cuh>
 

@@ -43,6 +43,40 @@ def test_scores(name, k):
     e.close()
 
 
+def check_sorted_state(R, m, out, cl, cr, levels):
+    """The engine's sorted state (sort_segments() -> out, level_counts() -> cl, cr) of every user of R under the scores m
+    against the oracle's, bit for bit.  levels: the engine's global level table."""
+    rp = R.row_ptr
+    for u in range(R.d1):
+        a, b = int(rp[u]), int(rp[u + 1])
+        if a == b:
+            continue
+        o = ob.level_counts(m[a:b], R.rating[a:b])
+        assert np.array_equal(out["sorted"][a:b].view(np.int64), o["s"].view(np.int64)), u   # bit pattern, -0.0 != +0.0
+        # permutation: valid, and equal to the oracle's wherever the key is unique
+        perm = out["perm"][a:b]
+        assert np.array_equal(np.sort(perm), np.arange(b - a))
+        assert np.array_equal(m[a:b][perm], o["s"])
+        assert np.array_equal(perm, o["perm"]), u          # both break ties by index
+        # levels: oracle's are user-local ranks, ours global ranks
+        lv_user = np.unique(np.rint(R.rating[a:b]).astype(np.int64))
+        glob = np.searchsorted(levels, lv_user)
+        assert np.array_equal(out["level"][a:b], glob[o["level"]])
+        # window pointers and per-level counters (loop locals of pcrpp.cpp:206-229)
+        assert np.array_equal(out["ub"][a:b], o["cntL"].sum(1)), u
+        assert np.array_equal((b - a) - out["lb"][a:b], o["cntR"].sum(1)), u
+        assert np.array_equal(cl[a:b][:, glob], o["cntL"]), u
+        assert np.array_equal(cr[a:b][:, glob], o["cntR"]), u
+        other = np.setdiff1d(np.arange(len(levels)), glob)
+        assert not cl[a:b][:, other].any() and not cr[a:b][:, other].any()
+        lev = o["level"]
+        col = np.arange(o["cntL"].shape[1])[None, :]
+        hi = np.where(col > lev[:, None], o["cntL"], 0).sum(1)
+        lo = np.where(col < lev[:, None], o["cntR"], 0).sum(1)
+        assert np.array_equal(out["cnt_hi"][a:b], hi), u
+        assert np.array_equal(out["cnt_lo"][a:b], lo), u
+
+
 @pytest.mark.parametrize("name", ["tiny", "ragged", "ragged_real"])
 def test_sort_and_counts_bitexact(name):
     """Identical scores in -> identical sorted order, window pointers and per-level counters out."""
@@ -61,34 +95,7 @@ def test_sort_and_counts_bitexact(name):
     e.set_scores(m)
     out = e.sort_segments()
     cl, cr = e.level_counts()
-    levels = np.unique(np.rint(ds.train.rating).astype(np.int64))
-    for u in range(ds.d1):
-        a, b = int(rp[u]), int(rp[u + 1])
-        if a == b:
-            continue
-        o = ob.level_counts(m[a:b], ds.train.rating[a:b])
-        assert np.array_equal(out["sorted"][a:b].view(np.int64), o["s"].view(np.int64)), u   # bit pattern, -0.0 != +0.0
-        # permutation: valid, and equal to the oracle's wherever the key is unique
-        perm = out["perm"][a:b]
-        assert np.array_equal(np.sort(perm), np.arange(b - a))
-        assert np.array_equal(m[a:b][perm], o["s"])
-        assert np.array_equal(perm, o["perm"]), u          # both break ties by index
-        # levels: oracle's are user-local ranks, ours global ranks
-        lv_user = np.unique(np.rint(ds.train.rating[a:b]).astype(np.int64))
-        glob = np.searchsorted(levels, lv_user)
-        assert np.array_equal(out["level"][a:b], glob[o["level"]])
-        # window pointers and per-level counters (loop locals of pcrpp.cpp:206-229)
-        assert np.array_equal(out["ub"][a:b], o["cntL"].sum(1)), u
-        assert np.array_equal((b - a) - out["lb"][a:b], o["cntR"].sum(1)), u
-        assert np.array_equal(cl[a:b][:, glob], o["cntL"]), u
-        assert np.array_equal(cr[a:b][:, glob], o["cntR"]), u
-        other = np.setdiff1d(np.arange(len(levels)), glob)
-        assert not cl[a:b][:, other].any() and not cr[a:b][:, other].any()
-        lev = o["level"]
-        hi = np.array([o["cntL"][j, lev[j] + 1:].sum() for j in range(b - a)])
-        lo = np.array([o["cntR"][j, :lev[j]].sum() for j in range(b - a)])
-        assert np.array_equal(out["cnt_hi"][a:b], hi), u
-        assert np.array_equal(out["cnt_lo"][a:b], lo), u
+    check_sorted_state(ds.train, m, out, cl, cr, np.unique(np.rint(ds.train.rating).astype(np.int64)))
     e.close()
 
 
