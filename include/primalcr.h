@@ -171,6 +171,55 @@ int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2,
                        int topn, int32_t *items_out, double *scores_out,       /* [n_users x topn] row-major; scores_out may be NULL */
                        int device);
 
+/* ---- held-out ranking evaluation: the exact catalog rank of every held-out entry (normally the test set), scored and
+   ordered as primalcr_recommend scores and orders, with every user's items of an optional exclusion CSR (normally the
+   training set) removed from its candidates.  U, V, k and the exclusion CSR are as for primalcr_recommend.
+   - Candidates of user u: the items not in u's exclusion row.  "Better" is primalcr_recommend's order: score descending,
+     ties to the smaller item id, +0.0 == -0.0, NaN below -inf.
+   - rank_out[e] for held-out entry e = (u, i): 1 + the number of u's candidates better than (score(u,i), i).  u's other
+     held-out items are candidates too; an item never beats itself.  An entry whose item is in u's exclusion row gets 0
+     (not a candidate, not ranked).
+   - Held-out rows may be in any order and may repeat an item; every occurrence gets the same rank.
+   - score_out[e] (may be NULL) is the score of entry e, the fma chain acc = fma(U[u][j], V[i][j], acc), j = 0..k-1, from
+     +0.0, returned as primalcr_recommend returns scores (-0.0 as +0.0, every NaN as the default quiet NaN).  Hence, for
+     every ranked entry with rank r <= N, primalcr_recommend(..., topn = N) returns item i at position r-1 of u's row with
+     a bit-identical score, and for r > N item i is not in that row.
+   - Ranks are bit-identical from call to call and do not depend on which other users have held-out entries.
+   - 1 <= k <= 256, d1, d2 <= INT32_MAX.  The kernel scores the catalog once per user and run of 64 held-out entries.
+   - Ids out of range, a decreasing ho_row_ptr or ho_row_ptr[0] != 0, the exclusion-row errors of primalcr_recommend, a
+     NULL ho_row_ptr, or a NULL ho_item / rank_out when there are entries return PRIMALCR_EARG before any kernel runs;
+     without a device the call returns PRIMALCR_ECUDA.
+   - The library owns the stream and device memory of the call and releases them before returning.
+   Several GPUs: split the users over devices (empty held-out rows cost nothing), one call per device. */
+int primalcr_rank_heldout(const double *U, int64_t d1, const double *V, int64_t d2, int k,
+                          const int64_t *excl_row_ptr, const int32_t *excl_item,  /* as primalcr_recommend; both NULL: none */
+                          const int64_t *ho_row_ptr, const int32_t *ho_item,      /* held-out CSR: d1+1 / ho_row_ptr[d1] */
+                          int32_t *rank_out, double *score_out,                   /* [ho_row_ptr[d1]], CSR order; score may be NULL */
+                          int device);
+
+/* ---- top-N metrics from held-out ranks (host only, no GPU).  rank[e] is primalcr_rank_heldout's rank of held-out entry e
+   and ho_rating[e] its rating; the exclusion CSR is the one the ranks were computed with.  Per user u:
+   - H_u: the distinct held-out items of u with rank > 0; an item's rating is the largest, its rank the smallest, among its
+     entries with rank > 0.  R_u = {i in H_u : rating >= min_rating} are the relevant items (min_rating = -inf: all).
+   - C_u = d2 - (number of distinct items in u's exclusion row); N_u = C_u - |R_u| non-relevant candidates.
+   - Only users with |R_u| >= 1 are evaluated; *n_users is their number.
+   - hits(N) = |{i in R_u : rank_i <= N}|;  recall@N = hits / |R_u|;  precision@N = hits / N.
+   - NDCG@N with binary gains: DCG = sum_{i in R_u, rank_i <= N} 1 / log2(rank_i + 1), IDCG = sum_{p=1}^{min(N,|R_u|)}
+     1 / log2(p + 1).  (2^r - 1 gains break on real-valued and negative ratings; min_rating carries the grading.)
+   - MRR = 1 / min_{i in R_u} rank_i.
+   - AUC_u = sum_{i in R_u} (N_u - (rank_i - 1 - pos_i)) / (|R_u| N_u), pos_i = the number of relevant items with a smaller
+     rank; users with N_u = 0 are left out of the AUC mean.
+   - Every metric is the plain mean over its users, summed in ascending user order in fp64 (deterministic); NaN when no
+     user is evaluated.
+   recall / precision / ndcg have n_cutoffs entries; any output may be NULL.  A rank outside [0, d2], a cutoff < 1, a
+   malformed CSR (the exclusion rows must ascend as for primalcr_recommend) or a NULL array that is needed returns
+   PRIMALCR_EARG. */
+int primalcr_rank_metrics(int64_t d1, int64_t d2, const int64_t *excl_row_ptr, const int32_t *excl_item,
+                          const int64_t *ho_row_ptr, const int32_t *ho_item, const double *ho_rating,
+                          const int32_t *rank, double min_rating, const int32_t *cutoffs, int n_cutoffs,
+                          double *recall, double *precision, double *ndcg,       /* [n_cutoffs] each; any may be NULL */
+                          double *mrr, double *auc, int64_t *n_users);           /* any may be NULL */
+
 /* ---- fast host loader for the reference's data directory (meta + ratings files): replaces load() util.cpp:6-25,
    smat_t::load_from_iterator util.h:201-271 and testset_t::load util.h:360-371 (no GPU needed) ------------------ */
 typedef struct primalcr_dataset primalcr_dataset;

@@ -53,7 +53,7 @@ SYMBOLS = [
     "primalcr_grad_U", "primalcr_hv_U", "primalcr_stream", "primalcr_launch_count", "primalcr_profile_enable",
     "primalcr_profile_reset", "primalcr_profile_count", "primalcr_profile_get", "primalcr_device_bytes",
     "primalcr_reference_init", "primalcr_write_text_matrix", "primalcr_predict", "primalcr_load_dir", "primalcr_dataset_info",
-    "primalcr_dataset_csr", "primalcr_dataset_free", "primalcr_recommend",
+    "primalcr_dataset_csr", "primalcr_dataset_free", "primalcr_recommend", "primalcr_rank_heldout", "primalcr_rank_metrics",
 ]
 
 _lib = None
@@ -119,6 +119,10 @@ def lib():
     L.primalcr_predict.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i32p, i32p, C.c_int64, f64p, C.c_int]
     L.primalcr_recommend.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i64p, i32p, i32p, C.c_int64, C.c_int, i32p,
                                      f64p, C.c_int]
+    L.primalcr_rank_heldout.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i64p, i32p, i64p, i32p, i32p, f64p, C.c_int]
+    L.primalcr_rank_metrics.argtypes = [C.c_int64, C.c_int64, i64p, i32p, i64p, i32p, f64p, i32p, C.c_double, i32p, C.c_int,
+                                        f64p, f64p, f64p, C.POINTER(C.c_double), C.POINTER(C.c_double),
+                                        C.POINTER(C.c_int64)]
     L.primalcr_load_dir.argtypes = [C.c_char_p, C.c_int, C.POINTER(vp)]
     L.primalcr_dataset_info.argtypes = [vp] + [C.POINTER(C.c_int64)] * 4
     L.primalcr_dataset_csr.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
@@ -227,6 +231,70 @@ def recommend(U, V, n: int, exclude: Ratings | None = None, users=None, device: 
     if rc != 0:
         raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
     return items, scores
+
+
+def _csr_arrays(R: Ratings, d1: int, d2: int, name: str):
+    """(row_ptr int64, item int32) of a d1 x d2 Ratings, checked for the lengths the C ABI reads."""
+    if R.d1 != d1 or R.d2 != d2:
+        raise PrimalCRError("%s is %d x %d, expected %d x %d" % (name, R.d1, R.d2, d1, d2))
+    rp = np.ascontiguousarray(R.row_ptr, np.int64); it = np.ascontiguousarray(R.item, np.int32)
+    if len(rp) != d1 + 1 or len(it) < rp[-1]:
+        raise PrimalCRError("%s: row_ptr needs d1+1 entries and item row_ptr[d1]" % name)
+    return rp, it
+
+
+def heldout_ranks(U, V, heldout: Ratings, exclude: Ratings | None = None, device: int = 0):
+    """The catalog rank of every held-out entry -> (ranks int32 [nnz], scores float64 [nnz]), in heldout's CSR order.
+
+    rank = 1 + the number of the user's items outside `exclude` (normally the training set) that api.recommend would put
+    before the entry's item; 0 when the item itself is excluded.  So an entry of rank r <= n is at position r-1 of
+    api.recommend(U, V, n, exclude)'s row for that user, with the same score bit for bit."""
+    U = np.ascontiguousarray(U, np.float64); V = np.ascontiguousarray(V, np.float64)
+    if U.ndim != 2 or V.ndim != 2 or U.shape[1] != V.shape[1]:
+        raise PrimalCRError("U and V must be 2-D with the same number of columns, got %s and %s" % (U.shape, V.shape))
+    d1, d2, k = U.shape[0], V.shape[0], U.shape[1]
+    hp, hi = _csr_arrays(heldout, d1, d2, "heldout")
+    rp = it = None
+    if exclude is not None:
+        rp, it = _csr_arrays(exclude, d1, d2, "exclude")
+    nnz = int(hp[-1])
+    ranks = np.empty(max(nnz, 0), np.int32); scores = np.empty(max(nnz, 0), np.float64)
+    rc = lib().primalcr_rank_heldout(U.ctypes.data, d1, V.ctypes.data, d2, k, _ptr(rp), _ptr(it), hp.ctypes.data,
+                                     hi.ctypes.data, ranks.ctypes.data, scores.ctypes.data, device)
+    if rc != 0:
+        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    return ranks, scores
+
+
+def ranking_metrics(ranks, heldout: Ratings, exclude: Ratings | None = None, cutoffs=(10,), min_rating=None) -> dict:
+    """recall@N, precision@N, ndcg@N for every N in cutoffs, mrr, auc and n_users from heldout_ranks' ranks (host only).
+
+    A held-out item is relevant when its rating is >= min_rating (None: every item); the definitions are those of
+    primalcr_rank_metrics in include/primalcr.h.  `exclude` must be the one the ranks were computed with."""
+    d1, d2 = heldout.d1, heldout.d2
+    hp, hi = _csr_arrays(heldout, d1, d2, "heldout")
+    hr = np.ascontiguousarray(heldout.rating, np.float64)
+    ranks = np.ascontiguousarray(ranks, np.int32).reshape(-1)
+    if len(ranks) < hp[-1] or len(hr) < hp[-1]:
+        raise PrimalCRError("ranks and heldout.rating need heldout.row_ptr[d1] entries")
+    rp = it = None
+    if exclude is not None:
+        rp, it = _csr_arrays(exclude, d1, d2, "exclude")
+    cuts = np.ascontiguousarray(cutoffs, np.int32).reshape(-1)
+    nc = len(cuts)
+    rec, prec, ndcg = np.empty(nc), np.empty(nc), np.empty(nc)
+    mrr, auc, n_users = C.c_double(), C.c_double(), C.c_int64()
+    rc = lib().primalcr_rank_metrics(d1, d2, _ptr(rp), _ptr(it), hp.ctypes.data, hi.ctypes.data, hr.ctypes.data,
+                                     ranks.ctypes.data, -np.inf if min_rating is None else float(min_rating),
+                                     cuts.ctypes.data, nc, rec.ctypes.data, prec.ctypes.data, ndcg.ctypes.data,
+                                     C.byref(mrr), C.byref(auc), C.byref(n_users))
+    if rc != 0:
+        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    out = {}
+    for j, n in enumerate(cuts):
+        out["recall@%d" % n] = float(rec[j]); out["precision@%d" % n] = float(prec[j]); out["ndcg@%d" % n] = float(ndcg[j])
+    out.update(mrr=mrr.value, auc=auc.value, n_users=int(n_users.value))
+    return out
 
 
 @dataclass

@@ -3,16 +3,11 @@
 // prints one "%lf" per test line: U[i-1] . V[j-1].  The dot products are evaluated on the GPU in one batch through
 // the C ABI (primalcr_predict); the model layout is the reference's (load_mat_t util.cpp:56-79).
 #include "../host/loader.hpp"
+#include "../host/model.hpp"
 #include "primalcr.h"
 
 #include <cstdio>
 #include <vector>
-
-static bool read_matrix(FILE *fp, std::vector<double> &M, long &rows, long &k) {
-    if (fread(&rows, sizeof(long), 1, fp) != 1 || fread(&k, sizeof(long), 1, fp) != 1) return false;
-    M.resize((size_t)rows * k);
-    return fread(M.data(), sizeof(double), (size_t)rows * k, fp) == (size_t)rows * k;
-}
 
 int main(int argc, char **argv) {
     if (argc != 4) { printf("Usage: primalcr-predict test_file model output_file\n"); return 1; }
@@ -22,7 +17,7 @@ int main(int argc, char **argv) {
     if (!out) { fprintf(stderr, "can't open output file %s\n", argv[3]); return 1; }
     std::vector<double> W, H;
     long d1 = 0, k = 0, d2 = 0, k2 = 0;
-    if (!read_matrix(model_fp, W, d1, k) || !read_matrix(model_fp, H, d2, k2) || k != k2) { fprintf(stderr, "bad model file %s\n", argv[2]); return 1; }
+    if (!pcrhost::read_matrix(model_fp, W, d1, k) || !pcrhost::read_matrix(model_fp, H, d2, k2) || k != k2) { fprintf(stderr, "bad model file %s\n", argv[2]); return 1; }
     fclose(model_fp);
     pcrhost::Triples t;
     try { t = pcrhost::parse_file(argv[1], -1); }

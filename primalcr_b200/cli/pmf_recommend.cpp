@@ -5,6 +5,7 @@
 // Writes one "user item score" line per recommendation: 1-based ids, "%.17g" scores (the doubles round-trip), users in
 // request order, best first; padding entries (fewer eligible items than topN) are not written.
 #include "../host/loader.hpp"
+#include "../host/model.hpp"
 #include "primalcr.h"
 
 #include <cstdio>
@@ -12,13 +13,6 @@
 #include <cstring>
 #include <string>
 #include <vector>
-
-static bool read_matrix(FILE *fp, std::vector<double> &M, long &rows, long &k) {
-    if (fread(&rows, sizeof(long), 1, fp) != 1 || fread(&k, sizeof(long), 1, fp) != 1) return false;
-    if (rows < 0 || k < 1) return false;
-    M.resize((size_t)rows * k);
-    return fread(M.data(), sizeof(double), (size_t)rows * k, fp) == (size_t)rows * k;
-}
 
 static void usage() {
     printf("Usage: primalcr-recommend [-n topN (default 10)] [-e data_dir] [-u users_file] [-d device] model output_file\n");
@@ -41,13 +35,9 @@ int main(int argc, char **argv) {
     if (argc - i != 2) { usage(); return 1; }
     const char *model_path = argv[i], *out_path = argv[i + 1];
 
-    FILE *model_fp = fopen(model_path, "rb");
-    if (!model_fp) { fprintf(stderr, "can't open model file %s\n", model_path); return 1; }
     std::vector<double> W, H;
-    long d1 = 0, k = 0, d2 = 0, k2 = 0;
-    const bool ok = read_matrix(model_fp, W, d1, k) && read_matrix(model_fp, H, d2, k2) && k == k2;
-    fclose(model_fp);
-    if (!ok) { fprintf(stderr, "bad model file %s\n", model_path); return 1; }
+    long d1 = 0, k = 0, d2 = 0;
+    if (!pcrhost::read_model(model_path, W, d1, H, d2, k)) { fprintf(stderr, "can't read model file %s\n", model_path); return 1; }
 
     pcrhost::DataDir data;
     if (data_dir) {

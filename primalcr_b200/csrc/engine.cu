@@ -9,6 +9,7 @@
 #include "kernels.h"
 #include "../../include/primalcr.h"
 #include "../host/loader.hpp"
+#include "../host/rankmetrics.hpp"
 #include "../host/textio.hpp"
 
 #include <algorithm>
@@ -1355,6 +1356,24 @@ int primalcr_predict(const double *U, int64_t d1, const double *V, int64_t d2, i
 }
 
 // ---- top-N recommendation ---------------------------------------------------------------------------------------
+// the exclusion CSR of primalcr_recommend / primalcr_rank_heldout: both pointers or neither, ascending rows -> its nnz
+static int64_t check_exclusion(int64_t d1, int64_t d2, const int64_t *excl_row_ptr, const int32_t *excl_item) {
+    if (!excl_row_ptr) return 0;
+    const std::string err = pcrhost::csr_error("exclusion", d1, d2, excl_row_ptr, excl_item, true);
+    PCR_REQUIRE(err.empty(), err);
+    return excl_row_ptr[d1];
+}
+
+// exclusion CSR to the device (both nullptr when there is none)
+static void upload_exclusion(pcr::DevPool &pool, cudaStream_t st, int64_t d1, const int64_t *excl_row_ptr,
+                             const int32_t *excl_item, int64_t ex_nnz, int64_t *&exp_d, int32_t *&exi_d) {
+    exp_d = nullptr; exi_d = nullptr;
+    if (!excl_row_ptr) return;
+    exp_d = pool.alloc<int64_t>((size_t)d1 + 1); exi_d = pool.alloc<int32_t>((size_t)ex_nnz);
+    PCR_CUDA(cudaMemcpyAsync(exp_d, excl_row_ptr, sizeof(int64_t) * ((size_t)d1 + 1), cudaMemcpyHostToDevice, st));
+    if (ex_nnz) PCR_CUDA(cudaMemcpyAsync(exi_d, excl_item, sizeof(int32_t) * (size_t)ex_nnz, cudaMemcpyHostToDevice, st));
+}
+
 int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
                        const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn, int32_t *items_out,
                        double *scores_out, int device) {
@@ -1377,24 +1396,7 @@ int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2,
         for (int64_t t = 0; t < n_users; ++t) bad_user = bad_user || users[t] < 0 || users[t] >= d1;
     }
     PCR_REQUIRE(!bad_user, "user id out of range");
-    int64_t ex_nnz = 0;
-    if (excl_row_ptr) {
-        PCR_REQUIRE(excl_row_ptr[0] == 0, "excl_row_ptr[0] must be 0");
-        bool bad_ptr = false, bad_item = false, descending = false;
-#pragma omp parallel for reduction(|| : bad_ptr, bad_item, descending) schedule(dynamic, 4096)
-        for (int64_t u = 0; u < d1; ++u) {
-            const int64_t a = excl_row_ptr[u], b = excl_row_ptr[u + 1];
-            if (b < a) { bad_ptr = true; continue; }
-            for (int64_t e = a; e < b; ++e) {
-                if (excl_item[e] < 0 || excl_item[e] >= d2) { bad_item = true; break; }
-                if (e > a && excl_item[e] < excl_item[e - 1]) { descending = true; break; }
-            }
-        }
-        PCR_REQUIRE(!bad_ptr, "excl_row_ptr decreases");
-        PCR_REQUIRE(!bad_item, "exclusion item id out of range");
-        PCR_REQUIRE(!descending, "exclusion row items must ascend");
-        ex_nnz = excl_row_ptr[d1];
-    }
+    const int64_t ex_nnz = check_exclusion(d1, d2, excl_row_ptr, excl_item);
     if (n_users == 0) return PRIMALCR_OK;
     PCR_CUDA(cudaSetDevice(device));
     pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
@@ -1407,20 +1409,91 @@ int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2,
     double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = pool.alloc<double>((size_t)d2 * k);
     int32_t *ud = pool.alloc<int32_t>((size_t)n_users), *itd = pool.alloc<int32_t>((size_t)n_users * topn);
     double *scd = scores_out ? pool.alloc<double>((size_t)n_users * topn) : nullptr;
-    int64_t *exp_d = nullptr; int32_t *exi_d = nullptr;
+    int64_t *exp_d; int32_t *exi_d;
     if (d1) PCR_CUDA(cudaMemcpyAsync(Ud, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
     if (d2) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
     if (users) PCR_CUDA(cudaMemcpyAsync(ud, users, sizeof(int32_t) * (size_t)n_users, cudaMemcpyHostToDevice, st));
     else pcr::k_iota32(ctx, ud, n_users);
-    if (excl_row_ptr) {
-        exp_d = pool.alloc<int64_t>((size_t)d1 + 1); exi_d = pool.alloc<int32_t>((size_t)ex_nnz);
-        PCR_CUDA(cudaMemcpyAsync(exp_d, excl_row_ptr, sizeof(int64_t) * ((size_t)d1 + 1), cudaMemcpyHostToDevice, st));
-        if (ex_nnz) PCR_CUDA(cudaMemcpyAsync(exi_d, excl_item, sizeof(int32_t) * (size_t)ex_nnz, cudaMemcpyHostToDevice, st));
-    }
+    upload_exclusion(pool, st, d1, excl_row_ptr, excl_item, ex_nnz, exp_d, exi_d);
     pcr::k_topn(ctx, Ud, Vd, d2, k, (const pcr::i64 *)exp_d, exi_d, ud, n_users, topn, itd, scd);
     PCR_CUDA(cudaMemcpyAsync(items_out, itd, sizeof(int32_t) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
     if (scores_out) PCR_CUDA(cudaMemcpyAsync(scores_out, scd, sizeof(double) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
     PCR_CUDA(cudaStreamSynchronize(st));
+    API_END
+}
+
+// ---- held-out ranking evaluation --------------------------------------------------------------------------------
+int primalcr_rank_heldout(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
+                          const int32_t *excl_item, const int64_t *ho_row_ptr, const int32_t *ho_item, int32_t *rank_out,
+                          double *score_out, int device) {
+    API_BEGIN
+    PCR_REQUIRE(k >= 1 && k <= 256, "rank k out of range [1, 256]");
+    PCR_REQUIRE(d1 >= 0 && d2 >= 0 && d1 <= INT32_MAX && d2 <= INT32_MAX, "d1 / d2 out of range");
+    PCR_REQUIRE((U || d1 == 0) && (V || d2 == 0), "null factor matrix");
+    PCR_REQUIRE(ho_row_ptr, "null ho_row_ptr");
+    PCR_REQUIRE((excl_row_ptr == nullptr) == (excl_item == nullptr), "excl_row_ptr and excl_item must both be given or both be NULL");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        throw pcr::Error(PRIMALCR_ECUDA, "no CUDA device available: libprimalcr_b200 has no CPU fallback");
+    PCR_REQUIRE(device >= 0 && device < ndev, "bad device ordinal");
+    // every id the kernel reads through is checked here, before anything runs
+    const int64_t nnz = ho_row_ptr[d1];
+    PCR_REQUIRE(nnz == 0 || (ho_item && rank_out), "null ho_item or rank_out");
+    const std::string err = pcrhost::csr_error("held-out", d1, d2, ho_row_ptr, ho_item, false);
+    PCR_REQUIRE(err.empty(), err);
+    const int64_t ex_nnz = check_exclusion(d1, d2, excl_row_ptr, excl_item);
+    if (nnz == 0) return PRIMALCR_OK;
+    // units: a user and at most RANK_UNIT consecutive entries of its row; they tile [0, nnz) in order
+    std::vector<int32_t> unit_user;
+    std::vector<int64_t> unit_beg;
+    for (int64_t u = 0; u < d1; ++u)
+        for (int64_t e = ho_row_ptr[u]; e < ho_row_ptr[u + 1]; e += pcr::RANK_UNIT) { unit_user.push_back((int32_t)u); unit_beg.push_back(e); }
+    unit_beg.push_back(nnz);
+    const int64_t n_units = (int64_t)unit_user.size();
+    PCR_CUDA(cudaSetDevice(device));
+    pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
+    // declared after the pool, so on every exit the stream is drained and destroyed before the buffers are freed
+    struct StreamGuard { cudaStream_t s = nullptr; ~StreamGuard() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } } } sg;
+    PCR_CUDA(cudaStreamCreateWithFlags(&sg.s, cudaStreamNonBlocking));
+    cudaStream_t st = sg.s;
+    cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
+    ctx.stream = st; ctx.prof = &prof; ctx.sms = prop.multiProcessorCount; ctx.ticket = nullptr;
+    double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = pool.alloc<double>((size_t)d2 * k);
+    int32_t *hid = pool.alloc<int32_t>((size_t)nnz), *rkd = pool.alloc<int32_t>((size_t)nnz);
+    int32_t *uud = pool.alloc<int32_t>((size_t)n_units);
+    int64_t *ubd = pool.alloc<int64_t>((size_t)n_units + 1);
+    double *scd = score_out ? pool.alloc<double>((size_t)nnz) : nullptr;
+    int64_t *exp_d; int32_t *exi_d;
+    if (d1) PCR_CUDA(cudaMemcpyAsync(Ud, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
+    if (d2) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
+    PCR_CUDA(cudaMemcpyAsync(hid, ho_item, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
+    PCR_CUDA(cudaMemcpyAsync(uud, unit_user.data(), sizeof(int32_t) * (size_t)n_units, cudaMemcpyHostToDevice, st));
+    PCR_CUDA(cudaMemcpyAsync(ubd, unit_beg.data(), sizeof(int64_t) * ((size_t)n_units + 1), cudaMemcpyHostToDevice, st));
+    upload_exclusion(pool, st, d1, excl_row_ptr, excl_item, ex_nnz, exp_d, exi_d);
+    pcr::k_rank_heldout(ctx, Ud, Vd, d2, k, (const pcr::i64 *)exp_d, exi_d, hid, uud, (const pcr::i64 *)ubd, n_units, rkd, scd);
+    PCR_CUDA(cudaMemcpyAsync(rank_out, rkd, sizeof(int32_t) * (size_t)nnz, cudaMemcpyDeviceToHost, st));
+    if (score_out) PCR_CUDA(cudaMemcpyAsync(score_out, scd, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToHost, st));
+    PCR_CUDA(cudaStreamSynchronize(st));
+    API_END
+}
+
+int primalcr_rank_metrics(int64_t d1, int64_t d2, const int64_t *excl_row_ptr, const int32_t *excl_item,
+                          const int64_t *ho_row_ptr, const int32_t *ho_item, const double *ho_rating, const int32_t *rank,
+                          double min_rating, const int32_t *cutoffs, int n_cutoffs, double *recall, double *precision,
+                          double *ndcg, double *mrr, double *auc, int64_t *n_users) {
+    API_BEGIN
+    pcrhost::RankMetrics m;
+    const std::string err = pcrhost::rank_metrics(d1, d2, excl_row_ptr, excl_item, ho_row_ptr, ho_item, ho_rating, rank,
+                                                  min_rating, cutoffs, n_cutoffs, m);
+    PCR_REQUIRE(err.empty(), err);
+    for (int c = 0; c < n_cutoffs; ++c) {
+        if (recall) recall[c] = m.recall[(size_t)c];
+        if (precision) precision[c] = m.precision[(size_t)c];
+        if (ndcg) ndcg[c] = m.ndcg[(size_t)c];
+    }
+    if (mrr) *mrr = m.mrr;
+    if (auc) *auc = m.auc;
+    if (n_users) *n_users = m.n_users;
     API_END
 }
 

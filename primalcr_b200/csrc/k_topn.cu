@@ -43,23 +43,123 @@ __device__ __forceinline__ void cp_async8(void *smem, const void *gmem, bool val
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
-// NMAX: largest topn of the class; UG: groups of 8 users (BU = 8 UG users, BI = 2048 / UG items per tile); CAP: candidates
-// buffered per user between merges.  256 threads: thread (ug, ig) computes users ug*8..+7 x items ig + IG*c, c = 0..7.
-template <int NMAX, int UG, int CAP>
-struct TopnCfg {
+// The scoring tile shared by topn_kernel and rank_kernel.  UG: groups of 8 rows (BU = 8 UG rows, BI = 2048 / UG items per
+// tile).  256 threads: thread (ug, ig) computes rows ug*8..+7 x items ig + IG*c, c = 0..7.
+template <int UG>
+struct TileCfg {
     static constexpr int THREADS = 256, WARPS = THREADS / 32;
     static constexpr int IG = THREADS / UG, BU = 8 * UG, BI = 8 * IG, KC = UG;   // KC * BI = 2048 doubles per V chunk
     static constexpr int PAD = 32 / KC;          // row padding: the transposing cp.async stores of a warp hit distinct banks
-    static constexpr int VS = KC * (BI + PAD), US = KC * (BU + PAD), MW = BI / 32, SCR = NMAX > CAP ? NMAX : CAP;
+    static constexpr int VS = KC * (BI + PAD), US = KC * (BU + PAD), MW = BI / 32;
+    static_assert(KC * BI == 2048 && BU * KC <= 2 * THREADS && IG >= 32, "tile shape");
+};
+
+// chunk kc of item tile t into buffer buf: V rows of the tile and U rows uid[0..nrows-1], k slice kc*KC..+KC-1
+template <int UG>
+__device__ __forceinline__ void tile_load(double *Vs, double *Us, const double *__restrict__ U, const double *__restrict__ V,
+                                          i64 d2, int k, const int *uid, int nrows, int t, int kc, int buf) {
+    typedef TileCfg<UG> C;
+    constexpr int BU = C::BU, BI = C::BI, KC = C::KC, PAD = C::PAD;
+    const int tid = threadIdx.x;
+    const int k0 = kc * KC;
+    const i64 base = (i64)t * BI;
+    double *vs = Vs + buf * C::VS;
+#pragma unroll
+    for (int j = 0; j < 2048 / C::THREADS; ++j) {
+        const int e = tid + j * C::THREADS, il = e / KC, kk = e % KC;
+        const i64 item = base + il;
+        const bool ok = item < d2 && k0 + kk < k;
+        cp_async8(vs + kk * (BI + PAD) + il, ok ? V + item * k + k0 + kk : V, ok);
+    }
+    double *us = Us + buf * C::US;
+    for (int e = tid; e < BU * KC; e += C::THREADS) {
+        const int r = e / KC, kk = e % KC;
+        const bool ok = r < nrows && k0 + kk < k;
+        cp_async8(us + kk * (BU + PAD) + r, ok ? U + (i64)uid[r] * k + k0 + kk : U, ok);
+    }
+    cp_async_commit();
+}
+
+// Scores of item tile t into acc: acc[r][c] = U[uid[ug*8+r]] . V[t*BI + ig + IG*c], the fma chain over k from +0.0.  With
+// `masked`, first the tile's rows x items exclusion bitmask, from each row's cursor cur[r] into its ascending exclusion row
+// (ending at cend[r]); the cursors advance past the tile.  Chunk 0 of tile t must have been loaded into buffer buf; the
+// first chunk of tile t+1 is prefetched.  Ends synchronised, with buf the buffer of that prefetch.
+template <int UG>
+__device__ __forceinline__ void score_tile(double (&acc)[8][8], double *Vs, double *Us, unsigned *mask, i64 *cur,
+                                           const i64 *cend, const double *__restrict__ U, const double *__restrict__ V,
+                                           i64 d2, int k, bool masked, const int32_t *__restrict__ ex_item, const int *uid,
+                                           int nrows, int t, int ntiles, int nkc, int &buf) {
+    typedef TileCfg<UG> C;
+    constexpr int BU = C::BU, BI = C::BI, KC = C::KC, IG = C::IG, PAD = C::PAD, MW = C::MW;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int ug = tid / IG, ig = tid % IG;
+    const i64 base = (i64)t * BI;
+    {
+#pragma unroll
+        for (int r = 0; r < 8; ++r)
+#pragma unroll
+            for (int c = 0; c < 8; ++c) acc[r][c] = 0.0;
+        if (masked) {                                   // exclusion bitmask of this tile
+            for (int e = tid; e < BU * MW; e += C::THREADS) mask[e] = 0u;
+            __syncthreads();
+            const i64 lim = base + BI;
+            for (int r = warp; r < nrows; r += C::WARPS) {
+                i64 p = cur[r];
+                const i64 pe = cend[r];
+                while (true) {
+                    const i64 q = p + lane;
+                    const i64 it = q < pe ? (i64)ex_item[q] : lim;
+                    const bool in = it < lim;
+                    if (in) atomicOr(&mask[r * MW + (int)((it - base) >> 5)], 1u << ((it - base) & 31));
+                    const int n = __popc(__ballot_sync(FULL, in));
+                    p += n;
+                    if (n < 32) break;
+                }
+                if (lane == 0) cur[r] = p;
+            }
+        }
+    }
+    for (int kc = 0; kc < nkc; ++kc, buf ^= 1) {
+        // prefetch the next chunk (of this tile, or the first of the next) while this one is computed
+        if (kc + 1 < nkc) { tile_load<UG>(Vs, Us, U, V, d2, k, uid, nrows, t, kc + 1, buf ^ 1); cp_async_wait<1>(); }
+        else if (t + 1 < ntiles) { tile_load<UG>(Vs, Us, U, V, d2, k, uid, nrows, t + 1, 0, buf ^ 1); cp_async_wait<1>(); }
+        else cp_async_wait<0>();
+        __syncthreads();
+        const double *vs = Vs + buf * C::VS + ig;
+        const double *us = Us + buf * C::US + ug * 8;
+#pragma unroll
+        for (int kk = 0; kk < KC; ++kk) {
+            double a[8], b[8];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const double2 v2 = *reinterpret_cast<const double2 *>(us + kk * (BU + PAD) + 2 * q);
+                a[2 * q] = v2.x; a[2 * q + 1] = v2.y;
+            }
+#pragma unroll
+            for (int c = 0; c < 8; ++c) b[c] = vs[kk * (BI + PAD) + IG * c];
+#pragma unroll
+            for (int r = 0; r < 8; ++r)
+#pragma unroll
+                for (int c = 0; c < 8; ++c) acc[r][c] = fma(a[r], b[c], acc[r][c]);
+        }
+        __syncthreads();
+    }
+}
+
+// NMAX: largest topn of the class; UG: the tile (BU = 8 UG users); CAP: candidates buffered per user between merges.
+template <int NMAX, int UG, int CAP>
+struct TopnCfg : TileCfg<UG> {
+    typedef TileCfg<UG> T;
+    static constexpr int SCR = NMAX > CAP ? NMAX : CAP;
+    static constexpr int BU = T::BU, WARPS = T::WARPS, MW = T::MW;
     // 8-byte arrays first, then 4-byte ones
-    static constexpr size_t o_vs = 0, o_us = o_vs + 2 * VS, o_lkey = o_us + 2 * US, o_ckey = o_lkey + BU * NMAX,
+    static constexpr size_t o_vs = 0, o_us = o_vs + 2 * T::VS, o_lkey = o_us + 2 * T::US, o_ckey = o_lkey + BU * NMAX,
                             o_skey = o_ckey + BU * CAP, o_thr = o_skey + WARPS * SCR, o_cur = o_thr + BU, o_end = o_cur + BU,
                             n8 = o_end + BU;
     static constexpr size_t o_litem = 0, o_citem = o_litem + BU * NMAX, o_sitem = o_citem + BU * CAP,
                             o_thri = o_sitem + WARPS * SCR, o_lcnt = o_thri + BU, o_ccnt = o_lcnt + BU, o_uid = o_ccnt + BU,
                             o_mask = o_uid + BU, n4 = o_mask + BU * MW;
     static constexpr size_t smem = n8 * 8 + n4 * 4;
-    static_assert(KC * BI == 2048 && BU * KC <= 2 * THREADS && IG >= 32, "tile shape");
 };
 
 template <int NMAX, int UG, int CAP>
@@ -68,7 +168,7 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
             const int32_t *__restrict__ ex_item, const int32_t *__restrict__ users, i64 n_users, int topn,
             int32_t *__restrict__ items_out, double *__restrict__ scores_out) {
     typedef TopnCfg<NMAX, UG, CAP> C;
-    constexpr int BU = C::BU, BI = C::BI, KC = C::KC, IG = C::IG, PAD = C::PAD, MW = C::MW, SCR = C::SCR;
+    constexpr int BU = C::BU, BI = C::BI, KC = C::KC, IG = C::IG, MW = C::MW, SCR = C::SCR;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double *Vs = reinterpret_cast<double *>(smem_raw) + C::o_vs;
     double *Us = reinterpret_cast<double *>(smem_raw) + C::o_us;
@@ -100,27 +200,6 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
 
     const int nkc = (k + KC - 1) / KC;
     const int ntiles = (int)((d2 + BI - 1) / BI);
-
-    // chunk kc of item tile t into buffer buf
-    auto load_step = [&](int t, int kc, int buf) {
-        const int k0 = kc * KC;
-        const i64 base = (i64)t * BI;
-        double *vs = Vs + buf * C::VS;
-#pragma unroll
-        for (int j = 0; j < 2048 / C::THREADS; ++j) {
-            const int e = tid + j * C::THREADS, il = e / KC, kk = e % KC;
-            const i64 item = base + il;
-            const bool ok = item < d2 && k0 + kk < k;
-            cp_async8(vs + kk * (BI + PAD) + il, ok ? V + item * k + k0 + kk : V, ok);
-        }
-        double *us = Us + buf * C::US;
-        for (int e = tid; e < BU * KC; e += C::THREADS) {
-            const int r = e / KC, kk = e % KC;
-            const bool ok = r < nrows && k0 + kk < k;
-            cp_async8(us + kk * (BU + PAD) + r, ok ? U + (i64)uid[r] * k + k0 + kk : U, ok);
-        }
-        cp_async_commit();
-    };
 
     // merge every user's candidates into its sorted top-N (warp per user); caller synchronises before and after
     auto merge_all = [&]() {
@@ -165,59 +244,10 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
 
     double acc[8][8];
     int buf = 0;
-    if (ntiles > 0) load_step(0, 0, 0);
+    if (ntiles > 0) tile_load<UG>(Vs, Us, U, V, d2, k, uid, nrows, 0, 0, 0);
     for (int t = 0; t < ntiles; ++t) {
         const i64 base = (i64)t * BI;
-        {
-#pragma unroll
-            for (int r = 0; r < 8; ++r)
-#pragma unroll
-                for (int c = 0; c < 8; ++c) acc[r][c] = 0.0;
-            if (ex_ptr) {                                   // exclusion bitmask of this tile
-                for (int e = tid; e < BU * MW; e += C::THREADS) mask[e] = 0u;
-                __syncthreads();
-                const i64 lim = base + BI;
-                for (int r = warp; r < nrows; r += C::WARPS) {
-                    i64 p = cur[r];
-                    const i64 pe = cend[r];
-                    while (true) {
-                        const i64 q = p + lane;
-                        const i64 it = q < pe ? (i64)ex_item[q] : lim;
-                        const bool in = it < lim;
-                        if (in) atomicOr(&mask[r * MW + (int)((it - base) >> 5)], 1u << ((it - base) & 31));
-                        const int n = __popc(__ballot_sync(FULL, in));
-                        p += n;
-                        if (n < 32) break;
-                    }
-                    if (lane == 0) cur[r] = p;
-                }
-            }
-        }
-        for (int kc = 0; kc < nkc; ++kc, buf ^= 1) {
-            // prefetch the next chunk (of this tile, or the first of the next) while this one is computed
-            if (kc + 1 < nkc) { load_step(t, kc + 1, buf ^ 1); cp_async_wait<1>(); }
-            else if (t + 1 < ntiles) { load_step(t + 1, 0, buf ^ 1); cp_async_wait<1>(); }
-            else cp_async_wait<0>();
-            __syncthreads();
-            const double *vs = Vs + buf * C::VS + ig;
-            const double *us = Us + buf * C::US + ug * 8;
-#pragma unroll
-            for (int kk = 0; kk < KC; ++kk) {
-                double a[8], b[8];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const double2 v2 = *reinterpret_cast<const double2 *>(us + kk * (BU + PAD) + 2 * q);
-                    a[2 * q] = v2.x; a[2 * q + 1] = v2.y;
-                }
-#pragma unroll
-                for (int c = 0; c < 8; ++c) b[c] = vs[kk * (BI + PAD) + IG * c];
-#pragma unroll
-                for (int r = 0; r < 8; ++r)
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) acc[r][c] = fma(a[r], b[c], acc[r][c]);
-            }
-            __syncthreads();
-        }
+        score_tile<UG>(acc, Vs, Us, mask, cur, cend, U, V, d2, k, ex_ptr != nullptr, ex_item, uid, nrows, t, ntiles, nkc, buf);
 
         // ---- selection of this tile's scores
         u64 pend = ~0ull;
@@ -302,6 +332,180 @@ void k_topn(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *
         launch_topn<128, 8, 64>(c, "pcr::topn_kernel<128,8,64>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
     else
         launch_topn<256, 4, 128>(c, "pcr::topn_kernel<256,4,128>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+}
+
+// ---- held-out ranks: the exact catalog rank of every held-out entry, under the same scores and order as topn_kernel
+// A CTA owns BU units; a unit is one user and a run of at most H consecutive entries of its held-out row (rows longer
+// than H become several units, each of which streams the whole catalog).  The prologue scores the unit's entries, drops
+// the ones in the exclusion row (rank 0) and rank-sorts the rest best first.  Per tile, an eligible candidate that beats
+// the unit's worst entry is binary-searched for the first sorted entry p it beats and counted in hist[p]; the rank of
+// sorted entry q is then 1 + sum_{p <= q} hist[p].  An entry never beats itself (the order is strict and both scores are
+// the same fma chain), so a held-out item is one of the candidates of its user's other entries and not of its own.
+template <int UG, int H>
+struct RankCfg : TileCfg<UG> {
+    typedef TileCfg<UG> T;
+    static constexpr int BU = T::BU, MW = T::MW;
+    static constexpr size_t o_vs = 0, o_us = o_vs + 2 * T::VS, o_hkey = o_us + 2 * T::US, o_wkey = o_hkey + BU * H,
+                            o_cur = o_wkey + BU, o_end = o_cur + BU, n8 = o_end + BU;
+    static constexpr size_t o_hitem = 0, o_hoff = o_hitem + BU * H, o_hist = o_hoff + BU * H, o_witem = o_hist + BU * H,
+                            o_nv = o_witem + BU, o_uid = o_nv + BU, o_mask = o_uid + BU, n4 = o_mask + BU * MW;
+    static constexpr size_t smem = n8 * 8 + n4 * 4;
+    static_assert(2 * T::VS >= BU * H, "the prologue's unsorted keys live in the V buffers");
+    static_assert(H % 32 == 0, "H is a multiple of the warp");
+};
+
+template <int UG, int H>
+__global__ void __launch_bounds__(256, 1)
+rank_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, int k, const i64 *__restrict__ ex_ptr,
+            const int32_t *__restrict__ ex_item, const int32_t *__restrict__ ho_item,
+            const int32_t *__restrict__ unit_user, const i64 *__restrict__ unit_beg, i64 n_units,
+            int32_t *__restrict__ rank_out, double *__restrict__ score_out) {
+    typedef RankCfg<UG, H> C;
+    constexpr int BU = C::BU, BI = C::BI, KC = C::KC, IG = C::IG, MW = C::MW;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    double *Vs = reinterpret_cast<double *>(smem_raw) + C::o_vs;
+    double *Us = reinterpret_cast<double *>(smem_raw) + C::o_us;
+    u64 *hkey = reinterpret_cast<u64 *>(smem_raw) + C::o_hkey;     // sorted entries of row r: [r*H, r*H + nv[r])
+    u64 *wkey = reinterpret_cast<u64 *>(smem_raw) + C::o_wkey;     // the worst sorted entry of each row
+    i64 *cur = reinterpret_cast<i64 *>(smem_raw) + C::o_cur;
+    i64 *cend = reinterpret_cast<i64 *>(smem_raw) + C::o_end;
+    int *i4 = reinterpret_cast<int *>(smem_raw + C::n8 * 8);
+    int *hitem = i4 + C::o_hitem, *hoff = i4 + C::o_hoff, *hist = i4 + C::o_hist, *witem = i4 + C::o_witem;
+    int *nv = i4 + C::o_nv, *uid = i4 + C::o_uid;
+    unsigned *mask = reinterpret_cast<unsigned *>(i4 + C::o_mask);
+    u64 *tkey = reinterpret_cast<u64 *>(Vs);       // prologue scratch: unsorted keys (V buffers) and items (hist)
+    int *titem = hist;
+
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int ug = tid / IG, ig = tid % IG;
+    const i64 row0 = (i64)blockIdx.x * BU;
+    const int nrows = (int)(n_units - row0 < BU ? n_units - row0 : BU);
+
+    for (int r = tid; r < BU; r += C::THREADS) {
+        const int u = r < nrows ? unit_user[row0 + r] : 0;
+        uid[r] = u; nv[r] = 0;
+        cur[r] = (ex_ptr && r < nrows) ? ex_ptr[u] : 0;
+        cend[r] = (ex_ptr && r < nrows) ? ex_ptr[u + 1] : 0;
+    }
+    __syncthreads();
+
+    // ---- prologue: score the entries (the tile's fma chain), look them up in the exclusion row, sort best first
+    for (int e = tid; e < BU * H; e += C::THREADS) {
+        const int r = e / H, j = e % H;
+        titem[e] = -1;
+        if (r >= nrows) continue;
+        const i64 g = unit_beg[row0 + r] + j;
+        if (g >= unit_beg[row0 + r + 1]) continue;
+        const int item = ho_item[g];
+        const double *ur = U + (i64)uid[r] * k, *vr = V + (i64)item * k;
+        double acc = 0.0;
+        for (int jj = 0; jj < k; ++jj) acc = fma(ur[jj], vr[jj], acc);
+        const u64 key = score_key(acc);
+        if (score_out) score_out[g] = key_score(key);       // as topn_kernel returns it: -0.0 as +0.0, one NaN
+        i64 lo = cur[r], hi = cend[r];
+        while (lo < hi) { const i64 mid = (lo + hi) >> 1; if (ex_item[mid] < item) lo = mid + 1; else hi = mid; }
+        if (lo < cend[r] && ex_item[lo] == item) { rank_out[g] = 0; continue; }
+        tkey[e] = key; titem[e] = item;
+        atomicAdd(&nv[r], 1);
+    }
+    __syncthreads();
+    for (int e = tid; e < BU * H; e += C::THREADS) {
+        const int r = e / H, j = e % H;
+        const u64 ka = tkey[e]; const int ia = titem[e];
+        if (ia < 0) continue;
+        int pos = 0;                  // entries before it: better ones, and equal ones (a repeated item) at smaller j
+        for (int q = 0; q < H; ++q) {
+            const int iq = titem[r * H + q];
+            if (iq < 0) continue;
+            const u64 kq = tkey[r * H + q];
+            pos += better(kq, iq, ka, ia) || (kq == ka && iq == ia && q < j);
+        }
+        hkey[r * H + pos] = ka; hitem[r * H + pos] = ia; hoff[r * H + pos] = j;
+    }
+    __syncthreads();
+    for (int e = tid; e < BU * H; e += C::THREADS) hist[e] = 0;
+    for (int r = tid; r < BU; r += C::THREADS) {
+        const int n = nv[r];
+        wkey[r] = n ? hkey[r * H + n - 1] : ~0ull;          // ~0 / -1: nothing beats it
+        witem[r] = n ? hitem[r * H + n - 1] : -1;
+    }
+    __syncthreads();
+
+    // ---- main loop: every eligible candidate of every tile against the unit's sorted entries
+    const int nkc = (k + KC - 1) / KC;
+    const int ntiles = (int)((d2 + BI - 1) / BI);
+    double acc[8][8];
+    int buf = 0;
+    if (ntiles > 0) tile_load<UG>(Vs, Us, U, V, d2, k, uid, nrows, 0, 0, 0);
+    for (int t = 0; t < ntiles; ++t) {
+        const i64 base = (i64)t * BI;
+        score_tile<UG>(acc, Vs, Us, mask, cur, cend, U, V, d2, k, ex_ptr != nullptr, ex_item, uid, nrows, t, ntiles, nkc, buf);
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {
+            const int row = ug * 8 + r;
+            if (row >= nrows) continue;
+            const u64 wk = wkey[row]; const int wi = witem[row];
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                const int il = ig + IG * c;
+                const int item = (int)(base + il);
+                if (base + il >= d2) continue;
+                if (ex_ptr && ((mask[row * MW + (il >> 5)] >> (il & 31)) & 1u)) continue;
+                const u64 ck = score_key(acc[r][c]);
+                if (!better(ck, item, wk, wi)) continue;       // the common case: beats no entry of the unit
+                const u64 *sk = hkey + row * H; const int *si = hitem + row * H;
+                int lo = 0, hi = nv[row] - 1;                  // the worst entry is beaten: the answer is in [0, nv-1]
+                while (lo < hi) { const int mid = (lo + hi) >> 1; if (better(ck, item, sk[mid], si[mid])) hi = mid; else lo = mid + 1; }
+                atomicAdd(&hist[row * H + lo], 1);
+            }
+        }
+        __syncthreads();                                      // the mask is rebuilt by the next tile
+    }
+
+    // ---- ranks: prefix sums of the histograms in sorted order, written to the entries' CSR positions
+    constexpr int PER = H / 32;
+    for (int r = warp; r < nrows; r += C::WARPS) {
+        const int n = nv[r];
+        const i64 g0 = unit_beg[row0 + r];
+        int h[PER], s = 0;
+#pragma unroll
+        for (int q = 0; q < PER; ++q) { h[q] = hist[r * H + lane * PER + q]; s += h[q]; }
+        int incl = s;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
+        int run = incl - s;
+#pragma unroll
+        for (int q = 0; q < PER; ++q) {
+            const int p = lane * PER + q;
+            run += h[q];
+            if (p < n) rank_out[g0 + hoff[r * H + p]] = 1 + run;
+        }
+    }
+}
+
+template <int UG, int H>
+static void launch_rank(Ctx &c, const char *name, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr,
+                        const int32_t *ex_item, const int32_t *ho_item, const int32_t *unit_user, const i64 *unit_beg,
+                        i64 n_units, int32_t *rank_out, double *score_out) {
+    typedef RankCfg<UG, H> C;
+    auto kern = rank_kernel<UG, H>;
+    PCR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
+    const i64 grid = (n_units + C::BU - 1) / C::BU;
+    const double bytes = (double)grid * d2 * k * 8.0 + (double)n_units * (k * 8.0 + H * 12.0);
+    c.prof->begin(name, c.stream, bytes);
+    kern<<<(unsigned)grid, C::THREADS, C::smem, c.stream>>>(U, V, d2, k, ex_ptr, ex_item, ho_item, unit_user, unit_beg,
+                                                             n_units, rank_out, score_out);
+    c.prof->end(c.stream);
+    PCR_CUDA(cudaGetLastError());
+}
+
+void k_rank_heldout(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr, const int32_t *ex_item,
+                    const int32_t *ho_item, const int32_t *unit_user, const i64 *unit_beg, i64 n_units, int32_t *rank_out,
+                    double *score_out) {
+    PCR_REQUIRE(k >= 1 && k <= 256, "k out of range [1, 256]");
+    if (n_units <= 0) return;
+    launch_rank<8, RANK_UNIT>(c, "pcr::rank_kernel<8,64>", U, V, d2, k, ex_ptr, ex_item, ho_item, unit_user, unit_beg,
+                              n_units, rank_out, score_out);
 }
 
 }  // namespace pcr

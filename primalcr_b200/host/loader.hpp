@@ -37,6 +37,29 @@ struct Csr {
 
 struct Triples { std::vector<int32_t> u, i; std::vector<double> r; };
 
+// Checks a caller's d1-row CSR over items [0, d2) (row_ptr: d1+1 entries; ascending: the items of a row must not
+// decrease, repeats allowed).  item == NULL checks the row pointers only.  Returns "" when it is well formed, else what is
+// wrong, prefixed with `what`.
+inline std::string csr_error(const char *what, int64_t d1, int64_t d2, const int64_t *row_ptr, const int32_t *item,
+                             bool ascending) {
+    if (row_ptr[0] != 0) return std::string(what) + ": row_ptr[0] must be 0";
+    bool bad_ptr = false, bad_item = false, descending = false;
+#pragma omp parallel for reduction(|| : bad_ptr, bad_item, descending) schedule(dynamic, 4096)
+    for (int64_t u = 0; u < d1; ++u) {
+        const int64_t a = row_ptr[u], b = row_ptr[u + 1];
+        if (b < a) { bad_ptr = true; continue; }
+        if (!item) continue;
+        for (int64_t e = a; e < b; ++e) {
+            if (item[e] < 0 || item[e] >= d2) { bad_item = true; break; }
+            if (ascending && e > a && item[e] < item[e - 1]) { descending = true; break; }
+        }
+    }
+    if (bad_ptr) return std::string(what) + ": row_ptr decreases";
+    if (bad_item) return std::string(what) + ": item id out of range";
+    if (descending) return std::string(what) + ": row items must ascend";
+    return "";
+}
+
 inline void parse_chunk(const char *p, const char *end, Triples &out) {
     while (p < end) {
         while (p < end && (*p == ' ' || *p == '\t' || *p == '\r' || *p == '\n')) ++p;
