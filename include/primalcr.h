@@ -101,12 +101,14 @@ int primalcr_update_U(primalcr_engine *e, double *now_obj);       /* update_U_ne
 int primalcr_outer_iteration(primalcr_engine *e, double *now_obj);/* update_V then update_U                     */
 /* compute_pairwise_error_ndcg util.cpp:434-542; which = 0 training set, 1 test set */
 int primalcr_eval(primalcr_engine *e, int which, double *pairwise_error, double *ndcg);
-/* the same evaluation with the integer pair-error count of every user written to err_per_user[d1] (any pointer may be NULL).
+/* the same evaluation with the integer pair-error count of every user written to err_per_user[d1] and every user's NDCG@k
+   to ndcg_per_user[d1] (any pointer may be NULL).  A user's NDCG is 0 for an empty row, otherwise dcg / idcg of that user,
+   which is NaN when idcg is 0 (every rating of the row is 0); the mean NDCG averages it over the non-empty rows.
    method 0: the reference's all-pairs count (util.cpp:467-479), O(len^2); method 1: the identical integer obtained from the
    Primal-CR++ sorted state in O(len * levels) (training set, integer ratings, <= 8 levels; PRIMALCR_EARG otherwise).
-   primalcr_eval picks method 1 whenever it applies. */
-int primalcr_eval_error_counts(primalcr_engine *e, int which, int method, int64_t *err_per_user, double *pairwise_error,
-                               double *ndcg);
+   primalcr_eval picks method 1 whenever it applies.  Both methods give bit-identical per-user NDCG. */
+int primalcr_eval_error_counts(primalcr_engine *e, int which, int method, int64_t *err_per_user, double *ndcg_per_user,
+                               double *pairwise_error, double *ndcg);
 /* whole driver with the reference's stdout lines (one callback per line, without the newline) */
 int primalcr_run(primalcr_engine *e, primalcr_log_fn log, void *ctx);
 int primalcr_get_counters(primalcr_engine *e, primalcr_counters *out);
@@ -114,7 +116,8 @@ int primalcr_get_counters(primalcr_engine *e, primalcr_counters *out);
 /* ---- per-stage entry points (parity tests call these through the same library) ----------------- */
 /* comp_m_new pcrpp.cpp:17 : scores of every training rating, CSR order */
 int primalcr_scores(primalcr_engine *e, double *m_out);
-/* load externally supplied scores (so sort / counts can be compared bit-exactly on identical inputs) */
+/* load externally supplied scores (so sort / counts can be compared bit-exactly on identical inputs); training-set
+   evaluation (which = 0) then evaluates the loaded scores until the factors or the scores change */
 int primalcr_set_scores(primalcr_engine *e, const double *m);
 /* get_sorted_mm pcrpp.cpp:52 + the window pointers of the sweep pcrpp.cpp:214-229, for all users:
    per rating, in (user, ascending score) order: sorted score, local index of that score inside its user,

@@ -68,7 +68,10 @@ class _Lib:
         f = g("compute_Ha_new"); f.restype = None; f.argtypes = csr + [_f64, _f64, _f64, _i, _d, _f64]
         f = g("objective_new"); f.restype = _d; f.argtypes = csr + [_f64, _f64, _f64, _i, _d]
         f = g("eval"); f.restype = None
-        f.argtypes = csr + [_f64, _f64, _i, _i, _f64] + ([C.c_void_p, C.c_void_p] if prefix == "orc_" else [])
+        f.argtypes = csr + [_f64, _f64, _i, _i, _f64] + ([C.c_void_p, C.c_void_p, C.c_void_p] if prefix == "orc_" else [])
+        if prefix == "orc_":
+            f = g("eval_scores"); f.restype = None
+            f.argtypes = [_l, _i64, _f64, _f64, _i, _f64, _i64, _i64, _f64]
         f = g("pcr_obtain_g"); f.restype = None
         f = g("pcr_compute_Ha"); f.restype = None
         f = g("pcr_objective"); f.restype = _d
@@ -151,16 +154,32 @@ class _Lib:
             self.lib.ref_user_stage(n, _padl(rows), _pad(vals), _pad(m), V, V.shape[0], r, lam, ui, s, g, obj, Hs)
         return g, float(obj[0]), Hs
 
-    def eval(self, X, U, V, ndcg_k=10, want_counts=False):
+    def eval(self, X, U, V, ndcg_k=10, want_counts=False, per_user=False):
+        """[pairwise error, ndcg]; want_counts: (that, the 4 totals, per-user error counts); per_user: the same plus the
+        per-user NDCG (NaN where the ideal DCG is 0, 0 for an empty row)."""
         out = np.zeros(2)
         if self.prefix == "orc_":
-            counts = np.zeros(4, np.int64); per_user = np.zeros(max(X.d1, 1), np.int64)
-            self.lib.orc_eval(*X.args(), U, V, U.shape[1], ndcg_k, out, _opt(counts), _opt(per_user))
+            counts = np.zeros(4, np.int64); err = np.zeros(max(X.d1, 1), np.int64); nd = np.zeros(max(X.d1, 1))
+            self.lib.orc_eval(*X.args(), U, V, U.shape[1], ndcg_k, out, _opt(counts), _opt(err), _opt(nd))
+            if per_user:
+                return out, counts, err[:X.d1], nd[:X.d1]
             if want_counts:
-                return out, counts, per_user[:X.d1]
+                return out, counts, err[:X.d1]
         else:
+            assert not (want_counts or per_user), "the reference harness returns the two means only"
             self.lib.ref_eval(*X.args(), U, V, U.shape[1], ndcg_k, out)
         return out
+
+    def eval_scores(self, X, m, ndcg_k=10):
+        """eval() from given scores m (one per rating of X, CSR order): (means, 4 totals, per-user error counts,
+        per-user NDCG)."""
+        assert self.prefix == "orc_"
+        m = np.ascontiguousarray(m, np.float64)
+        assert len(m) == X.nnz
+        out = np.zeros(2); counts = np.zeros(4, np.int64)
+        err = np.zeros(max(X.d1, 1), np.int64); nd = np.zeros(max(X.d1, 1))
+        self.lib.orc_eval_scores(X.d1, X.index, X.vals, _pad(m), ndcg_k, out, counts, err, nd)
+        return out, counts, err[:X.d1], nd[:X.d1]
 
     def train(self, solver, X, XT, U, V, lam, maxiter, do_predict=1, ndcg_k=10, stepsize=1.0, threads=1):
         """Runs `maxiter` outer iterations; returns dict(obj, evals, U, V[, counters])."""

@@ -505,20 +505,21 @@ static int desc_cmp(const void *a, const void *b) {
     return (x->idx > y->idx) - (x->idx < y->idx);
 }
 
-/* compute_pairwise_error_ndcg util.cpp:434-542.  out[0] = pairwise error, out[1] = ndcg.
+/* compute_pairwise_error_ndcg util.cpp:434-542 from given scores (score[e] of rating e, CSR order).
+   out[0] = pairwise error, out[1] = ndcg.
    counts (optional, 4 longs): total error_comps, total num_comps, users with >=1 pair, users with >=1 rating.
-   per_user_err (optional, d1 longs) = error_comps_i */
-void orc_eval(long d1, long d2, long nnz, const long *index, const long *rows, const double *vals,
-              const double *U, const double *V, int r, int ndcg_k, double *out, long *counts, long *per_user_err) {
-    (void)d2; (void)nnz;
+   per_user_err (optional, d1 longs) = error_comps_i.
+   per_user_ndcg (optional, d1 doubles) = dcg / dcg_max of the user (NaN when dcg_max is 0), 0 for an empty row */
+void orc_eval_scores(long d1, const long *index, const double *vals, const double *scores, int ndcg_k, double *out,
+                     long *counts, long *per_user_err, double *per_user_ndcg) {
     double sum_error = 0.0, ndcg_sum = 0.0;
     long total_count = 0, total_pair_d1 = 0, tot_err = 0, tot_cmp = 0;
     for (long i = 0; i < d1; ++i) {
         long start = index[i], end = index[i + 1] - 1, len = end - start + 1;
         if (per_user_err) per_user_err[i] = 0;
+        if (per_user_ndcg) per_user_ndcg[i] = 0.0;
         if (len == 0) continue; else total_count += 1;
-        double *score = (double *)malloc(sizeof(double) * (size_t)len);
-        for (long k = 0; k < len; ++k) score[k] = dot_rev(U + i * r, V + rows[start + k] * r, r);
+        const double *score = scores + start;
         long error_comps_i = 0, num_comps_i = 0;
         for (long j = start; j < end; ++j) {
             double val_j = vals[j];
@@ -549,11 +550,24 @@ void orc_eval(long d1, long d2, long nnz, const long *index, const long *rows, c
             dcg_max += (pow(2.0, vals[start + id2]) - 1.0) / log2((double)k + 1.0);
         }
         ndcg_sum += dcg / dcg_max;
-        free(score); free(bs); free(bv);
+        if (per_user_ndcg) per_user_ndcg[i] = dcg / dcg_max;
+        free(bs); free(bv);
     }
     out[0] = sum_error / (double)total_pair_d1;
     out[1] = ndcg_sum / (double)total_count;
     if (counts) { counts[0] = tot_err; counts[1] = tot_cmp; counts[2] = total_pair_d1; counts[3] = total_count; }
+}
+
+/* compute_pairwise_error_ndcg util.cpp:434-542 at the factors (U, V): the scores are U_i . V_j (dot_rev), then as above */
+void orc_eval(long d1, long d2, long nnz, const long *index, const long *rows, const double *vals,
+              const double *U, const double *V, int r, int ndcg_k, double *out, long *counts, long *per_user_err,
+              double *per_user_ndcg) {
+    (void)d2;
+    double *score = (double *)malloc(sizeof(double) * (size_t)(nnz > 0 ? nnz : 1));
+    for (long i = 0; i < d1; ++i)
+        for (long e = index[i]; e < index[i + 1]; ++e) score[e] = dot_rev(U + i * r, V + rows[e] * r, r);
+    orc_eval_scores(d1, index, vals, score, ndcg_k, out, counts, per_user_err, per_user_ndcg);
+    free(score);
 }
 
 /* ---------------------------------------------------------------- Primal-CR (pcr.cpp), O(len^2) pair loops */
@@ -859,10 +873,10 @@ void orc_train(int solver, long d1, long d2, long nnz, const long *index, const 
             e[0] = e[1] = e[2] = e[3] = 0.0;
             if (do_predict) {
                 double o[2];
-                orc_eval(d1, d2, nnz, index, rows, vals, U, V, r, ndcg_k, o, NULL, NULL);
+                orc_eval(d1, d2, nnz, index, rows, vals, U, V, r, ndcg_k, o, NULL, NULL, NULL);
                 e[0] = o[0]; e[1] = o[1];
                 if (nnz_t != 0) {
-                    orc_eval(d1, d2, nnz_t, index_t, rows_t, vals_t, U, V, r, ndcg_k, o, NULL, NULL);
+                    orc_eval(d1, d2, nnz_t, index_t, rows_t, vals_t, U, V, r, ndcg_k, o, NULL, NULL, NULL);
                     e[2] = o[0]; e[3] = o[1];
                 }
             }

@@ -94,7 +94,7 @@ def lib():
     for name in ("initial_objective", "objective", "update_V", "update_U", "outer_iteration"):
         getattr(L, "primalcr_" + name).argtypes = [vp, C.POINTER(C.c_double)]
     L.primalcr_eval.argtypes = [vp, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]
-    L.primalcr_eval_error_counts.argtypes = [vp, C.c_int, C.c_int, vp, C.POINTER(C.c_double), C.POINTER(C.c_double)]
+    L.primalcr_eval_error_counts.argtypes = [vp, C.c_int, C.c_int, vp, vp, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.primalcr_run.argtypes = [vp, LOG_FN, vp]
     L.primalcr_get_counters.argtypes = [vp, C.POINTER(Counters)]
     L.primalcr_scores.argtypes = [vp, f64p]
@@ -411,12 +411,17 @@ class Engine:
         self._check(self._L.primalcr_eval(self._h, which, C.byref(a), C.byref(b)))
         return a.value, b.value
 
-    def eval_error_counts(self, which: int = 0, method: int = 0):
-        """(pairwise error, NDCG, integer pair-error count per user); method 0 all pairs, 1 sorted state (Primal-CR++ train set)."""
+    def eval_error_counts(self, which: int = 0, method: int = 0, ndcg_per_user: bool = False):
+        """(pairwise error, NDCG, integer pair-error count per user[, NDCG per user]); method 0 all pairs, 1 sorted state
+        (Primal-CR++ train set).  A user's NDCG is 0 for an empty row and NaN when its ideal DCG is 0."""
         n = self.d1
         cnt = np.zeros(max(n, 1), np.int64)
+        nd = np.zeros(max(n, 1)) if ndcg_per_user else None
         a, b = C.c_double(), C.c_double()
-        self._check(self._L.primalcr_eval_error_counts(self._h, which, method, cnt.ctypes.data, C.byref(a), C.byref(b)))
+        self._check(self._L.primalcr_eval_error_counts(self._h, which, method, cnt.ctypes.data,
+                                                       None if nd is None else nd.ctypes.data, C.byref(a), C.byref(b)))
+        if ndcg_per_user:
+            return a.value, b.value, cnt[:n], nd[:n]
         return a.value, b.value, cnt[:n]
 
     def run(self, log=print):

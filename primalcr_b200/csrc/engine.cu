@@ -565,7 +565,7 @@ struct Engine {
         PCR_REQUIRE(has_train, "load the training set first");
         put_matrix(Uh, d1, U); put_matrix(Vh, d2, V);
         sync();
-        has_factors = true; scores_valid = false; meta_valid = false; loss_matches_m = false; last_m_is_stale = false;
+        has_factors = true; scores_valid = false; meta_valid = false; loss_matches_m = false; last_m_is_stale = false; v_trial_pending = false;
     }
     void get_factors(double *Uh, double *Vh) {
         bind();
@@ -821,14 +821,26 @@ struct Engine {
         counters.v_cg_iters = its; counters.v_ls_trials = trials; counters.v_ls_accepted = accepted;
         v_accepted = accepted;
         last_m_is_stale = !accepted;
+        v_trial_pending = !accepted;
         return now_obj;
     }
     bool last_m_is_stale = false;
+    // update_V rejected every trial and no update_U or write has run since: Vnew still holds the last trial's V.  A read-only
+    // call may replace m (ensure_scores, primalcr_scores) in the meantime; update_U then rebuilds that trial's state from
+    // (U, Vnew) -- the same kernels on the same inputs, so the same bits -- and consumes it as if nothing had been read.
+    bool v_trial_pending = false;
     bool loss_matches_m = false;   // us.loss == per-user losses of the scores in m (set by update_V's last trial)
 
     // ------------------------------------------------------------------ update_U(_new), batched over users
     double update_U() {
         require_ready();
+        if (v_trial_pending && !last_m_is_stale) {      // what update_V's last trial left behind, see there
+            scores(U, Vnew, m, nullptr);
+            if (cfg.solver == 2) prepare(m, nullptr);
+            user_losses(m, nullptr);
+            scores_valid = false; loss_matches_m = true; last_m_is_stale = true;
+        }
+        v_trial_pending = false;
         if (!scores_valid && !last_m_is_stale) { scores(U, V, m, nullptr); scores_valid = true; meta_valid = false; loss_matches_m = false; }
         if (cfg.solver == 2 && !meta_valid) prepare(m, nullptr);
         // m holds scores(U, V) for every user (not the scores of a rejected V trial): then what the line search leaves
@@ -916,7 +928,7 @@ struct Engine {
         return which == 0 && cfg.solver == 2 && scores_valid && meta_valid && ratings_integer && T <= 8;
     }
     // method: -1 automatic, 0 all-pairs kernel (the reference's O(len^2) loop util.cpp:467-479), 1 sorted-state count
-    void eval(int which, double *err, double *ndcg, int method = -1, i64 *err_user_host = nullptr) {
+    void eval(int which, double *err, double *ndcg, int method = -1, i64 *err_user_host = nullptr, double *ndcg_user_host = nullptr) {
         require_ready();
         DevCsr &C = which == 0 ? X : XT;
         PCR_REQUIRE(which == 0 || has_test, "no test set loaded");
@@ -937,6 +949,7 @@ struct Engine {
             if (!sorted) k_eval_item_to_user(ctx, C, ev_err_item, ev_err_user);
             if (C.d1) PCR_CUDA(cudaMemcpyAsync(err_user_host, ev_err_user, sizeof(i64) * (size_t)C.d1, cudaMemcpyDeviceToHost, stream));
         }
+        if (ndcg_user_host && C.d1) PCR_CUDA(cudaMemcpyAsync(ndcg_user_host, ev_b, sizeof(double) * (size_t)C.d1, cudaMemcpyDeviceToHost, stream));
         k_sum(ctx, ev_a, C.d1, red_partials, slots + 0);
         k_sum(ctx, ev_b, C.d1, red_partials, slots + 1);
         k_sum(ctx, ev_c, C.d1, red_partials, slots + 2);
@@ -1098,7 +1111,7 @@ int primalcr_initial_objective(primalcr_engine *e, double *obj) {
     CHECK_E(e) API_BEGIN
     Engine *E = e->impl;
     E->require_ready();
-    E->scores_valid = false; E->meta_valid = false;
+    E->scores_valid = false; E->meta_valid = false; E->v_trial_pending = false;
     const double o = E->objective_current();
     E->sync();
     if (obj) *obj = o;
@@ -1148,11 +1161,12 @@ int primalcr_eval(primalcr_engine *e, int which, double *pairwise_error, double 
     API_END
 }
 
-int primalcr_eval_error_counts(primalcr_engine *e, int which, int method, int64_t *err_per_user, double *pairwise_error, double *ndcg) {
+int primalcr_eval_error_counts(primalcr_engine *e, int which, int method, int64_t *err_per_user, double *ndcg_per_user,
+                               double *pairwise_error, double *ndcg) {
     CHECK_E(e) API_BEGIN
     PCR_REQUIRE(method == 0 || method == 1, "method must be 0 (all pairs) or 1 (sorted state)");
     double a = 0, b = 0;
-    e->impl->eval(which, &a, &b, method, (pcr::i64 *)err_per_user);
+    e->impl->eval(which, &a, &b, method, (pcr::i64 *)err_per_user, ndcg_per_user);
     e->impl->sync();
     if (pairwise_error) *pairwise_error = a;
     if (ndcg) *ndcg = b;
@@ -1191,7 +1205,7 @@ int primalcr_set_scores(primalcr_engine *e, const double *m) {
     PCR_REQUIRE(m != nullptr || E->X.nnz == 0, "null scores");
     if (E->X.nnz) PCR_CUDA(cudaMemcpyAsync(E->m, m, sizeof(double) * (size_t)E->X.nnz, cudaMemcpyHostToDevice, E->stream));
     E->sync();
-    E->scores_valid = true; E->meta_valid = false; E->last_m_is_stale = false; E->loss_matches_m = false;
+    E->scores_valid = true; E->meta_valid = false; E->last_m_is_stale = false; E->loss_matches_m = false; E->v_trial_pending = false;
     API_END
 }
 

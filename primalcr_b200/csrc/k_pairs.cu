@@ -270,7 +270,7 @@ void k_eval_sorted(Ctx &c, const DevCsr &X, const SortedMeta &meta, int T, i64 *
                    double *err_ratio_user, double *ndcg_user, double *has_pair_user, double *has_any_user) {
     if (X.d1 <= 0) return;
     const unsigned grid = (unsigned)((X.d1 + 7) / 8);
-#define ES(TT) LAUNCH(c, "eval_sorted", 0.0, eval_sorted_kernel<TT>, grid, 256, 0, X.row_ptr, X.d1, meta.s, meta.lev, err_user, meta.pos, X.rating, \
+#define ES(TT) LAUNCH(c, "eval_sorted_T" #TT, 0.0, eval_sorted_kernel<TT>, grid, 256, 0, X.row_ptr, X.d1, meta.s, meta.lev, err_user, meta.pos, X.rating, \
                       level_vals, ndcg_k, err_ratio_user, ndcg_user, has_pair_user, has_any_user)
     if (T <= 5) ES(5); else ES(8);
 #undef ES
