@@ -174,6 +174,35 @@ int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2,
                        int topn, int32_t *items_out, double *scores_out,       /* [n_users x topn] row-major; scores_out may be NULL */
                        int device);
 
+/* ---- similar items / users: for each query row q of M (n x k, row-major host array: V for items, U for users), the topn
+   rows of M most similar to it under `measure`.  The kernel is primalcr_recommend's, with U = V = M.
+   - Candidates of query q: every row i != q that is not in q's exclusion row.  A row is never its own neighbour; other rows
+     with identical vectors are ordinary candidates.
+   - Scores.  dot(q, i) is primalcr_recommend's fma chain acc = fma(M[q][j], M[i][j], acc), j = 0..k-1, from +0.0, and
+     |x| = sqrt(acc) of the chain acc = fma(x[j], x[j], acc) in the same order.  PRIMALCR_SIM_DOT scores dot(q, i);
+     PRIMALCR_SIM_COSINE scores dot(q, i) / (|M[q]| * |M[i]|): one rounded product, then one IEEE division, so a zero row
+     gets NaN scores.  Scores are returned as primalcr_recommend returns them: -0.0 as +0.0, every NaN as the default
+     quiet NaN.
+   - Order: primalcr_recommend's.  Score descending, ties to the smaller id, +0.0 == -0.0, NaN below -inf.  A query with
+     fewer than topn candidates gets the tail of its row padded with id -1 and score NaN.
+   - A query's row is bit-identical from call to call and does not depend on the other queries of the batch.  With
+     PRIMALCR_SIM_DOT it equals primalcr_recommend(M, n, M, n, k, E, ..., users = {q}, topn) bit for bit, where E is q's
+     exclusion row with q merged in.
+   - 1 <= topn <= 256, 1 <= k <= 256, n <= INT32_MAX.
+   - An unknown measure, ids out of range, an exclusion row whose ids do not ascend (repeats are allowed, and q itself may
+     appear), excl_row_ptr without excl_id, a NULL ids_out when there are queries or any other bad argument returns
+     PRIMALCR_EARG before any kernel runs; without a device the call returns PRIMALCR_ECUDA.
+   - The library owns the stream and device memory of the call and releases them before returning; M is uploaded once.
+   Several GPUs: split the queries over devices, one call per device. */
+#define PRIMALCR_SIM_DOT    0   /* score = M[q] . M[i]                         */
+#define PRIMALCR_SIM_COSINE 1   /* score = (M[q] . M[i]) / (|M[q]| * |M[i]|)   */
+int primalcr_similar(const double *M, int64_t n, int k, int measure,
+                     const int64_t *excl_row_ptr, const int32_t *excl_id,   /* n+1 / row_ptr[n], indexed by query id; both NULL: none */
+                     const int32_t *queries, int64_t n_queries,            /* 0-based row ids, any order, repeats allowed;
+                                                                              NULL: 0..n-1, and n_queries must be n */
+                     int topn, int32_t *ids_out, double *scores_out,       /* [n_queries x topn] row-major; scores_out may be NULL */
+                     int device);
+
 /* ---- held-out ranking evaluation: the exact catalog rank of every held-out entry (normally the test set), scored and
    ordered as primalcr_recommend scores and orders, with every user's items of an optional exclusion CSR (normally the
    training set) removed from its candidates.  U, V, k and the exclusion CSR are as for primalcr_recommend.

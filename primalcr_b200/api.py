@@ -54,6 +54,7 @@ SYMBOLS = [
     "primalcr_profile_reset", "primalcr_profile_count", "primalcr_profile_get", "primalcr_device_bytes",
     "primalcr_reference_init", "primalcr_write_text_matrix", "primalcr_predict", "primalcr_load_dir", "primalcr_dataset_info",
     "primalcr_dataset_csr", "primalcr_dataset_free", "primalcr_recommend", "primalcr_rank_heldout", "primalcr_rank_metrics",
+    "primalcr_similar",
 ]
 
 _lib = None
@@ -119,6 +120,7 @@ def lib():
     L.primalcr_predict.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i32p, i32p, C.c_int64, f64p, C.c_int]
     L.primalcr_recommend.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i64p, i32p, i32p, C.c_int64, C.c_int, i32p,
                                      f64p, C.c_int]
+    L.primalcr_similar.argtypes = [f64p, C.c_int64, C.c_int, C.c_int, i64p, i32p, i32p, C.c_int64, C.c_int, i32p, f64p, C.c_int]
     L.primalcr_rank_heldout.argtypes = [f64p, C.c_int64, f64p, C.c_int64, C.c_int, i64p, i32p, i64p, i32p, i32p, f64p, C.c_int]
     L.primalcr_rank_metrics.argtypes = [C.c_int64, C.c_int64, i64p, i32p, i64p, i32p, f64p, i32p, C.c_double, i32p, C.c_int,
                                         f64p, f64p, f64p, C.POINTER(C.c_double), C.POINTER(C.c_double),
@@ -231,6 +233,37 @@ def recommend(U, V, n: int, exclude: Ratings | None = None, users=None, device: 
     if rc != 0:
         raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
     return items, scores
+
+
+SIMILARITY = {"dot": 0, "cosine": 1}     # PRIMALCR_SIM_DOT, PRIMALCR_SIM_COSINE
+
+
+def similar(M, n: int, measure: str = "cosine", exclude: Ratings | None = None, queries=None, device: int = 0):
+    """The n rows of M most similar to each query row -> (ids int32 (n_queries, n), scores float64 (n_queries, n)).
+
+    M is V for similar items, U for similar users.  measure "cosine": M[q].M[i] / (|M[q]| |M[i]|) (NaN for a zero row);
+    "dot": M[q].M[i].  A row is never its own neighbour; `exclude` (rows x rows, indexed by query id) removes more.  Rows are
+    ordered as api.recommend orders them and padded with id -1 / score NaN.  queries: 0-based ids in any order, repeats
+    allowed (default: every row)."""
+    if measure not in SIMILARITY:
+        raise PrimalCRError("measure must be one of %s, got %r" % (sorted(SIMILARITY), measure))
+    M = np.ascontiguousarray(M, np.float64)
+    if M.ndim != 2:
+        raise PrimalCRError("M must be 2-D, got shape %s" % (M.shape,))
+    rows, k = M.shape
+    rp = it = None
+    if exclude is not None:
+        rp, it = _csr_arrays(exclude, rows, rows, "exclude")
+    if queries is not None:
+        queries = np.ascontiguousarray(queries, np.int32).reshape(-1)
+    n_q = rows if queries is None else len(queries)
+    ids = np.empty((n_q, max(int(n), 0)), np.int32)
+    scores = np.empty((n_q, max(int(n), 0)), np.float64)
+    rc = lib().primalcr_similar(M.ctypes.data, rows, k, SIMILARITY[measure], _ptr(rp), _ptr(it), _ptr(queries), n_q,
+                                int(n), ids.ctypes.data, scores.ctypes.data, device)
+    if rc != 0:
+        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    return ids, scores
 
 
 def _csr_arrays(R: Ratings, d1: int, d2: int, name: str):

@@ -1388,10 +1388,12 @@ static void upload_exclusion(pcr::DevPool &pool, cudaStream_t st, int64_t d1, co
     if (ex_nnz) PCR_CUDA(cudaMemcpyAsync(exi_d, excl_item, sizeof(int32_t) * (size_t)ex_nnz, cudaMemcpyHostToDevice, st));
 }
 
-int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
-                       const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn, int32_t *items_out,
-                       double *scores_out, int device) {
-    API_BEGIN
+// Argument checks of a top-N call (primalcr_recommend, primalcr_similar): rows users[0..n_users) of U (d1 x k; users NULL:
+// every row) against the d2 rows of V (d2 x k), with an optional d1 x d2 exclusion CSR.  Throws before any device work;
+// returns the exclusion's nnz.
+static int64_t check_topn(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
+                          const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn,
+                          const int32_t *items_out, int device) {
     PCR_REQUIRE(k >= 1 && k <= 256, "rank k out of range [1, 256]");
     PCR_REQUIRE(topn >= 1 && topn <= 256, "topn out of range [1, 256]");
     PCR_REQUIRE(d1 >= 0 && d2 >= 0 && d1 <= INT32_MAX && d2 <= INT32_MAX, "d1 / d2 out of range");
@@ -1410,8 +1412,18 @@ int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2,
         for (int64_t t = 0; t < n_users; ++t) bad_user = bad_user || users[t] < 0 || users[t] >= d1;
     }
     PCR_REQUIRE(!bad_user, "user id out of range");
-    const int64_t ex_nnz = check_exclusion(d1, d2, excl_row_ptr, excl_item);
-    if (n_users == 0) return PRIMALCR_OK;
+    return check_exclusion(d1, d2, excl_row_ptr, excl_item);
+}
+
+// A checked top-N call on a stream and device memory of its own, all released before it returns: uploads U, V (V_is_U:
+// V is U, uploaded once), the row ids and the exclusion CSR, runs launch(ctx, pool, Ud, Vd, exp_d, exi_d, ud, itd, scd)
+// and copies the [n_users x topn] rows back.
+extern "C++" {      // a template: C++ linkage inside the extern "C" block
+template <class Launch>
+static void serve_topn(const double *U, int64_t d1, const double *V, int64_t d2, bool V_is_U, int k,
+                       const int64_t *excl_row_ptr, const int32_t *excl_item, int64_t ex_nnz, const int32_t *users,
+                       int64_t n_users, int topn, int32_t *items_out, double *scores_out, int device, Launch launch) {
+    if (n_users == 0) return;
     PCR_CUDA(cudaSetDevice(device));
     pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
     // declared after the pool, so on every exit the stream is drained and destroyed before the buffers are freed
@@ -1420,19 +1432,49 @@ int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2,
     cudaStream_t st = sg.s;
     cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
     ctx.stream = st; ctx.prof = &prof; ctx.sms = prop.multiProcessorCount; ctx.ticket = nullptr;
-    double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = pool.alloc<double>((size_t)d2 * k);
+    double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = V_is_U ? Ud : pool.alloc<double>((size_t)d2 * k);
     int32_t *ud = pool.alloc<int32_t>((size_t)n_users), *itd = pool.alloc<int32_t>((size_t)n_users * topn);
     double *scd = scores_out ? pool.alloc<double>((size_t)n_users * topn) : nullptr;
     int64_t *exp_d; int32_t *exi_d;
     if (d1) PCR_CUDA(cudaMemcpyAsync(Ud, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
-    if (d2) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
+    if (d2 && !V_is_U) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
     if (users) PCR_CUDA(cudaMemcpyAsync(ud, users, sizeof(int32_t) * (size_t)n_users, cudaMemcpyHostToDevice, st));
     else pcr::k_iota32(ctx, ud, n_users);
     upload_exclusion(pool, st, d1, excl_row_ptr, excl_item, ex_nnz, exp_d, exi_d);
-    pcr::k_topn(ctx, Ud, Vd, d2, k, (const pcr::i64 *)exp_d, exi_d, ud, n_users, topn, itd, scd);
+    launch(ctx, pool, (const double *)Ud, (const double *)Vd, (const pcr::i64 *)exp_d, (const int32_t *)exi_d,
+           (const int32_t *)ud, itd, scd);
     PCR_CUDA(cudaMemcpyAsync(items_out, itd, sizeof(int32_t) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
     if (scores_out) PCR_CUDA(cudaMemcpyAsync(scores_out, scd, sizeof(double) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
     PCR_CUDA(cudaStreamSynchronize(st));
+}
+}  // extern "C++"
+
+int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
+                       const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn, int32_t *items_out,
+                       double *scores_out, int device) {
+    API_BEGIN
+    const int64_t ex_nnz = check_topn(U, d1, V, d2, k, excl_row_ptr, excl_item, users, n_users, topn, items_out, device);
+    serve_topn(U, d1, V, d2, false, k, excl_row_ptr, excl_item, ex_nnz, users, n_users, topn, items_out, scores_out, device,
+               [&](pcr::Ctx &ctx, pcr::DevPool &, const double *Ud, const double *Vd, const pcr::i64 *exp_d,
+                   const int32_t *exi_d, const int32_t *ud, int32_t *itd, double *scd) {
+                   pcr::k_topn(ctx, Ud, Vd, d2, k, exp_d, exi_d, ud, n_users, topn, itd, scd);
+               });
+    API_END
+}
+
+// ---- similar items / users ---------------------------------------------------------------------------------------
+int primalcr_similar(const double *M, int64_t n, int k, int measure, const int64_t *excl_row_ptr, const int32_t *excl_id,
+                     const int32_t *queries, int64_t n_queries, int topn, int32_t *ids_out, double *scores_out, int device) {
+    API_BEGIN
+    PCR_REQUIRE(measure == PRIMALCR_SIM_DOT || measure == PRIMALCR_SIM_COSINE, "unknown similarity measure");
+    const int64_t ex_nnz = check_topn(M, n, M, n, k, excl_row_ptr, excl_id, queries, n_queries, topn, ids_out, device);
+    serve_topn(M, n, M, n, true, k, excl_row_ptr, excl_id, ex_nnz, queries, n_queries, topn, ids_out, scores_out, device,
+               [&](pcr::Ctx &ctx, pcr::DevPool &pool, const double *Md, const double *, const pcr::i64 *exp_d,
+                   const int32_t *exi_d, const int32_t *qd, int32_t *itd, double *scd) {
+                   const bool cosine = measure == PRIMALCR_SIM_COSINE;
+                   double *norms = cosine ? pool.alloc<double>((size_t)n) : nullptr;
+                   pcr::k_similar(ctx, Md, n, k, cosine, norms, exp_d, exi_d, qd, n_queries, topn, itd, scd);
+               });
     API_END
 }
 

@@ -12,6 +12,11 @@
 // below -inf (NaNs tie, so the item decides).  Every score is the fma chain acc = fma(U[u][j], V[i][j], acc), j = 0..k-1,
 // from +0.0 -- the same for every class and batch -- and the top-N under a total order is unique, so a user's row does not
 // depend on the batch it is computed in.
+//
+// Similar rows (similar_kernel: topn_kernel with SELF, and COS for cosine) rank the rows of one matrix M against query rows
+// of the same M: U = V = M.  SELF adds each query's own row to its tile exclusion mask; COS divides every register score
+// by (|M[q]| * |M[i]|), norms from row_norms staged in shared memory, before it meets the filter, so the buffers and the
+// merge only ever see final scores.
 #include "kernels.h"
 
 namespace pcr {
@@ -82,9 +87,10 @@ __device__ __forceinline__ void tile_load(double *Vs, double *Us, const double *
 
 // Scores of item tile t into acc: acc[r][c] = U[uid[ug*8+r]] . V[t*BI + ig + IG*c], the fma chain over k from +0.0.  With
 // `masked`, first the tile's rows x items exclusion bitmask, from each row's cursor cur[r] into its ascending exclusion row
-// (ending at cend[r]); the cursors advance past the tile.  Chunk 0 of tile t must have been loaded into buffer buf; the
-// first chunk of tile t+1 is prefetched.  Ends synchronised, with buf the buffer of that prefetch.
-template <int UG>
+// (ending at cend[r]); the cursors advance past the tile.  SELF (which needs `masked`): item uid[r] is masked in row r too.
+// Chunk 0 of tile t must have been loaded into buffer buf; the first chunk of tile t+1 is prefetched.  Ends synchronised,
+// with buf the buffer of that prefetch.
+template <int UG, bool SELF = false>
 __device__ __forceinline__ void score_tile(double (&acc)[8][8], double *Vs, double *Us, unsigned *mask, i64 *cur,
                                            const i64 *cend, const double *__restrict__ U, const double *__restrict__ V,
                                            i64 d2, int k, bool masked, const int32_t *__restrict__ ex_item, const int *uid,
@@ -115,7 +121,11 @@ __device__ __forceinline__ void score_tile(double (&acc)[8][8], double *Vs, doub
                     p += n;
                     if (n < 32) break;
                 }
-                if (lane == 0) cur[r] = p;
+                if (lane == 0) {
+                    cur[r] = p;
+                    if (SELF && uid[r] >= base && uid[r] < lim)
+                        atomicOr(&mask[r * MW + (int)((uid[r] - base) >> 5)], 1u << ((uid[r] - base) & 31));
+                }
             }
         }
     }
@@ -147,7 +157,8 @@ __device__ __forceinline__ void score_tile(double (&acc)[8][8], double *Vs, doub
 }
 
 // NMAX: largest topn of the class; UG: the tile (BU = 8 UG users); CAP: candidates buffered per user between merges.
-template <int NMAX, int UG, int CAP>
+// COS: room for the norms of the BU query rows and of the BI rows of the current tile.
+template <int NMAX, int UG, int CAP, bool COS = false>
 struct TopnCfg : TileCfg<UG> {
     typedef TileCfg<UG> T;
     static constexpr int SCR = NMAX > CAP ? NMAX : CAP;
@@ -155,19 +166,22 @@ struct TopnCfg : TileCfg<UG> {
     // 8-byte arrays first, then 4-byte ones
     static constexpr size_t o_vs = 0, o_us = o_vs + 2 * T::VS, o_lkey = o_us + 2 * T::US, o_ckey = o_lkey + BU * NMAX,
                             o_skey = o_ckey + BU * CAP, o_thr = o_skey + WARPS * SCR, o_cur = o_thr + BU, o_end = o_cur + BU,
-                            n8 = o_end + BU;
+                            o_qn = o_end + BU, o_tn = o_qn + (COS ? BU : 0), n8 = o_tn + (COS ? T::BI : 0);
     static constexpr size_t o_litem = 0, o_citem = o_litem + BU * NMAX, o_sitem = o_citem + BU * CAP,
                             o_thri = o_sitem + WARPS * SCR, o_lcnt = o_thri + BU, o_ccnt = o_lcnt + BU, o_uid = o_ccnt + BU,
                             o_mask = o_uid + BU, n4 = o_mask + BU * MW;
     static constexpr size_t smem = n8 * 8 + n4 * 4;
+    static_assert(smem <= 227 * 1024, "shared memory of one CTA");
 };
 
-template <int NMAX, int UG, int CAP>
+// SELF: a row's own id (users[q], an index into V) is never its candidate.  COS: scores are divided by
+// (norms[users[q]] * norms[item]); norms is unused otherwise.
+template <int NMAX, int UG, int CAP, bool SELF = false, bool COS = false>
 __global__ void __launch_bounds__(256, 1)
 topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, int k, const i64 *__restrict__ ex_ptr,
             const int32_t *__restrict__ ex_item, const int32_t *__restrict__ users, i64 n_users, int topn,
-            int32_t *__restrict__ items_out, double *__restrict__ scores_out) {
-    typedef TopnCfg<NMAX, UG, CAP> C;
+            int32_t *__restrict__ items_out, double *__restrict__ scores_out, const double *__restrict__ norms) {
+    typedef TopnCfg<NMAX, UG, CAP, COS> C;
     constexpr int BU = C::BU, BI = C::BI, KC = C::KC, IG = C::IG, MW = C::MW, SCR = C::SCR;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double *Vs = reinterpret_cast<double *>(smem_raw) + C::o_vs;
@@ -178,6 +192,8 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
     u64 *thr_key = reinterpret_cast<u64 *>(smem_raw) + C::o_thr;
     i64 *cur = reinterpret_cast<i64 *>(smem_raw) + C::o_cur;
     i64 *cend = reinterpret_cast<i64 *>(smem_raw) + C::o_end;
+    double *qnorm = reinterpret_cast<double *>(smem_raw) + C::o_qn;     // COS only
+    double *tnorm = reinterpret_cast<double *>(smem_raw) + C::o_tn;
     int *i4 = reinterpret_cast<int *>(smem_raw + C::n8 * 8);
     int *litem = i4 + C::o_litem, *citem = i4 + C::o_citem, *sitem_all = i4 + C::o_sitem, *thr_item = i4 + C::o_thri;
     int *lcnt = i4 + C::o_lcnt, *ccnt = i4 + C::o_ccnt, *uid = i4 + C::o_uid;
@@ -195,11 +211,13 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
         uid[r] = u; lcnt[r] = 0; ccnt[r] = 0; thr_key[r] = 0ull; thr_item[r] = 0;
         cur[r] = (ex_ptr && r < nrows) ? ex_ptr[u] : 0;
         cend[r] = (ex_ptr && r < nrows) ? ex_ptr[u + 1] : 0;
+        if (COS) qnorm[r] = r < nrows ? norms[u] : 1.0;
     }
     __syncthreads();
 
     const int nkc = (k + KC - 1) / KC;
     const int ntiles = (int)((d2 + BI - 1) / BI);
+    const bool masked = SELF || ex_ptr != nullptr;
 
     // merge every user's candidates into its sorted top-N (warp per user); caller synchronises before and after
     auto merge_all = [&]() {
@@ -247,7 +265,18 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
     if (ntiles > 0) tile_load<UG>(Vs, Us, U, V, d2, k, uid, nrows, 0, 0, 0);
     for (int t = 0; t < ntiles; ++t) {
         const i64 base = (i64)t * BI;
-        score_tile<UG>(acc, Vs, Us, mask, cur, cend, U, V, d2, k, ex_ptr != nullptr, ex_item, uid, nrows, t, ntiles, nkc, buf);
+        // the tile's norms, read after score_tile's barriers; the previous tile's reads all precede a barrier of its selection
+        if (COS)
+            for (int i = tid; i < BI; i += C::THREADS) tnorm[i] = base + i < d2 ? norms[base + i] : 1.0;
+        score_tile<UG, SELF>(acc, Vs, Us, mask, cur, cend, U, V, d2, k, masked, ex_item, uid, nrows, t, ntiles, nkc, buf);
+        if (COS) {
+#pragma unroll
+            for (int r = 0; r < 8; ++r) {
+                const double qn = qnorm[ug * 8 + r];
+#pragma unroll
+                for (int c = 0; c < 8; ++c) acc[r][c] = acc[r][c] / (qn * tnorm[ig + IG * c]);
+            }
+        }
 
         // ---- selection of this tile's scores
         u64 pend = ~0ull;
@@ -263,7 +292,7 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
                     const int il = ig + IG * c;
                     const u64 bit = 1ull << (r * 8 + c);
                     if (!(pend & bit) || base + il >= d2) continue;
-                    if (ex_ptr && ((mask[row * MW + (il >> 5)] >> (il & 31)) & 1u)) continue;
+                    if (masked && ((mask[row * MW + (il >> 5)] >> (il & 31)) & 1u)) continue;
                     if (better(score_key(acc[r][c]), (int)(base + il), tk, ti)) keep |= bit;
                 }
             }
@@ -306,32 +335,73 @@ topn_kernel(const double *__restrict__ U, const double *__restrict__ V, i64 d2, 
     }
 }
 
-template <int NMAX, int UG, int CAP>
+template <int NMAX, int UG, int CAP, bool SELF, bool COS>
 static void launch_topn(Ctx &c, const char *name, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr,
                         const int32_t *ex_item, const int32_t *users, i64 n_users, int topn, int32_t *items_out,
-                        double *scores_out) {
-    typedef TopnCfg<NMAX, UG, CAP> C;
-    auto kern = topn_kernel<NMAX, UG, CAP>;
+                        double *scores_out, const double *norms) {
+    typedef TopnCfg<NMAX, UG, CAP, COS> C;
+    auto kern = topn_kernel<NMAX, UG, CAP, SELF, COS>;
     PCR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
     const i64 grid = (n_users + C::BU - 1) / C::BU;
     const double bytes = (double)grid * d2 * k * 8.0 + (double)n_users * (k * 8.0 + topn * 12.0);
     c.prof->begin(name, c.stream, bytes);
     kern<<<(unsigned)grid, C::THREADS, C::smem, c.stream>>>(U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out,
-                                                             scores_out);
+                                                             scores_out, norms);
     c.prof->end(c.stream);
     PCR_CUDA(cudaGetLastError());
 }
 
-void k_topn(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr, const int32_t *ex_item,
-            const int32_t *users, i64 n_users, int topn, int32_t *items_out, double *scores_out) {
+// the class of topn: names[0] for topn <= 32, names[1] for <= 128, names[2] for <= 256
+template <bool SELF, bool COS>
+static void dispatch_topn(Ctx &c, const char *const (&names)[3], const double *U, const double *V, i64 d2, int k,
+                          const i64 *ex_ptr, const int32_t *ex_item, const int32_t *users, i64 n_users, int topn,
+                          int32_t *items_out, double *scores_out, const double *norms) {
     PCR_REQUIRE(topn >= 1 && topn <= 256 && k >= 1 && k <= 256, "topn / k out of range [1, 256]");
     if (n_users <= 0) return;
     if (topn <= 32)
-        launch_topn<32, 8, 64>(c, "pcr::topn_kernel<32,8,64>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+        launch_topn<32, 8, 64, SELF, COS>(c, names[0], U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out, norms);
     else if (topn <= 128)
-        launch_topn<128, 8, 64>(c, "pcr::topn_kernel<128,8,64>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+        launch_topn<128, 8, 64, SELF, COS>(c, names[1], U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out, norms);
     else
-        launch_topn<256, 4, 128>(c, "pcr::topn_kernel<256,4,128>", U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out);
+        launch_topn<256, 4, 128, SELF, COS>(c, names[2], U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out, norms);
+}
+
+void k_topn(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr, const int32_t *ex_item,
+            const int32_t *users, i64 n_users, int topn, int32_t *items_out, double *scores_out) {
+    static const char *const names[3] = {"pcr::topn_kernel<32,8,64>", "pcr::topn_kernel<128,8,64>", "pcr::topn_kernel<256,4,128>"};
+    dispatch_topn<false, false>(c, names, U, V, d2, k, ex_ptr, ex_item, users, n_users, topn, items_out, scores_out, nullptr);
+}
+
+// |M[i]| = sqrt of the fma chain acc = fma(M[i][j], M[i][j], acc), j = 0..k-1, from +0.0
+__global__ void row_norms_kernel(const double *__restrict__ M, i64 n, int k, double *__restrict__ out) {
+    for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
+        const double *m = M + i * k;
+        double acc = 0.0;
+        for (int j = 0; j < k; ++j) acc = fma(m[j], m[j], acc);
+        out[i] = sqrt(acc);
+    }
+}
+
+void k_similar(Ctx &c, const double *M, i64 n, int k, bool cosine, double *norms, const i64 *ex_ptr,
+               const int32_t *ex_item, const int32_t *queries, i64 n_queries, int topn, int32_t *ids_out,
+               double *scores_out) {
+    PCR_REQUIRE(topn >= 1 && topn <= 256 && k >= 1 && k <= 256, "topn / k out of range [1, 256]");
+    if (n_queries <= 0) return;
+    if (cosine) {
+        i64 blocks = (n + 255) / 256;
+        if (blocks > (i64)c.sms * 16) blocks = (i64)c.sms * 16;
+        c.prof->begin("pcr::row_norms", c.stream, (double)n * (k + 1) * 8.0);
+        row_norms_kernel<<<(unsigned)(blocks > 0 ? blocks : 1), 256, 0, c.stream>>>(M, n, k, norms);
+        c.prof->end(c.stream);
+        PCR_CUDA(cudaGetLastError());
+        static const char *const names[3] = {"pcr::similar_kernel<32,8,64,cos>", "pcr::similar_kernel<128,8,64,cos>",
+                                              "pcr::similar_kernel<256,4,128,cos>"};
+        dispatch_topn<true, true>(c, names, M, M, n, k, ex_ptr, ex_item, queries, n_queries, topn, ids_out, scores_out, norms);
+    } else {
+        static const char *const names[3] = {"pcr::similar_kernel<32,8,64,dot>", "pcr::similar_kernel<128,8,64,dot>",
+                                              "pcr::similar_kernel<256,4,128,dot>"};
+        dispatch_topn<true, false>(c, names, M, M, n, k, ex_ptr, ex_item, queries, n_queries, topn, ids_out, scores_out, nullptr);
+    }
 }
 
 // ---- held-out ranks: the exact catalog rank of every held-out entry, under the same scores and order as topn_kernel

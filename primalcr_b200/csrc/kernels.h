@@ -125,6 +125,11 @@ void k_eval_users(Ctx &c, const DevCsr &X, const double *score, const i64 *err_i
 // rows with fewer eligible items are padded with item -1 / score NaN.  scores_out may be nullptr.  1 <= topn, k <= 256.
 void k_topn(Ctx &c, const double *U, const double *V, i64 d2, int k, const i64 *ex_ptr, const int32_t *ex_item,
             const int32_t *users, i64 n_users, int topn, int32_t *items_out, double *scores_out);
+// similar rows: k_topn with U = V = M (n x k) and each query's own row never a candidate.  cosine: scores are
+// dot / (|M[q]| * |M[i]|), the norms computed into norms[n] first (nullptr when !cosine).  1 <= topn, k <= 256.
+void k_similar(Ctx &c, const double *M, i64 n, int k, bool cosine, double *norms, const i64 *ex_ptr,
+               const int32_t *ex_item, const int32_t *queries, i64 n_queries, int topn, int32_t *ids_out,
+               double *scores_out);
 // held-out ranks: unit q is user unit_user[q] and held-out entries [unit_beg[q], unit_beg[q+1]) (at most RANK_UNIT of them,
 // items ho_item[e]).  rank_out[e] = 1 + the number of the user's eligible items that rank before (score, item) of entry e in
 // k_topn's order, or 0 when the item is in the user's exclusion row; score_out[e] (may be nullptr) is the score as k_topn
