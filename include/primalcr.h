@@ -150,7 +150,10 @@ int     primalcr_profile_get(primalcr_engine *e, int idx, const char **name, dou
 int64_t primalcr_device_bytes(primalcr_engine *e);                /* device memory held by the engine    */
 
 /* ---- prediction: the loop of omp-pmf-predict pmf-predict.cpp:57-64 as one batch on the GPU ------------------------
-   out[t] = U[user[t]] . V[item[t]] for n (0-based) pairs; U is d1 x k, V is d2 x k row-major host arrays. */
+   out[t] = U[user[t]] . V[item[t]] for n (0-based) pairs; U is d1 x k, V is d2 x k row-major host arrays, k >= 1.
+   - Ids out of range, a bad device ordinal or any other bad argument returns PRIMALCR_EARG before any kernel runs; without
+     a device the call returns PRIMALCR_ECUDA.
+   - The library owns the stream and device memory of the call and releases them before returning. */
 int primalcr_predict(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int32_t *user,
                      const int32_t *item, int64_t n, double *out, int device);
 

@@ -142,6 +142,20 @@ def _ptr(a):
     return a.data_ptr()   # torch tensor (pinned host memory in bench.py)
 
 
+def _check(rc):
+    """Raises the library's last error when a C-ABI call returned a nonzero code."""
+    if rc != 0:
+        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+
+
+def _factors(U, V):
+    """U (d1 x k) and V (d2 x k) as C-contiguous float64 arrays -> (U, V, d1, d2, k)."""
+    U = np.ascontiguousarray(U, np.float64); V = np.ascontiguousarray(V, np.float64)
+    if U.ndim != 2 or V.ndim != 2 or U.shape[1] != V.shape[1]:
+        raise PrimalCRError("U and V must be 2-D with the same number of columns, got %s and %s" % (U.shape, V.shape))
+    return U, V, U.shape[0], V.shape[0], U.shape[1]
+
+
 def _require_factor(a, rows: int, k: int, name: str):
     """The C ABI reads / writes rows*k doubles through a raw pointer: insist on a C-contiguous float64 (rows, k) buffer."""
     if isinstance(a, np.ndarray):
@@ -165,9 +179,7 @@ def reference_init(n: int, k: int) -> np.ndarray:
 def write_text_matrix(path: str, M: np.ndarray) -> None:
     """U.txt / V.txt as the reference CLI writes them (pmf-train.cpp:276-295), formatted in parallel on the host."""
     M = np.ascontiguousarray(M, np.float64)
-    rc = lib().primalcr_write_text_matrix(path.encode(), M.ctypes.data, M.shape[0], M.shape[1])
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    _check(lib().primalcr_write_text_matrix(path.encode(), M.ctypes.data, M.shape[0], M.shape[1]))
 
 
 def load_dir(path: str, threads: int = 0):
@@ -175,9 +187,7 @@ def load_dir(path: str, threads: int = 0):
     from .data import Dataset
     L = lib()
     h = C.c_void_p()
-    rc = L.primalcr_load_dir(path.encode(), threads, C.byref(h))
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, L.primalcr_last_error().decode()))
+    _check(L.primalcr_load_dir(path.encode(), threads, C.byref(h)))
     try:
         d1, d2, n0, n1 = C.c_int64(), C.c_int64(), C.c_int64(), C.c_int64()
         L.primalcr_dataset_info(h, C.byref(d1), C.byref(d2), C.byref(n0), C.byref(n1))
@@ -196,13 +206,13 @@ def load_dir(path: str, threads: int = 0):
 
 def predict(U, V, users, items, device: int = 0) -> np.ndarray:
     """omp-pmf-predict's loop (pmf-predict.cpp:57-64) as one GPU batch: out[t] = U[users[t]] . V[items[t]] (0-based)."""
-    U = np.ascontiguousarray(U, np.float64); V = np.ascontiguousarray(V, np.float64)
+    U, V, d1, d2, k = _factors(U, V)
     users = np.ascontiguousarray(users, np.int32); items = np.ascontiguousarray(items, np.int32)
+    if users.ndim != 1 or items.ndim != 1 or len(users) != len(items):
+        raise PrimalCRError("users and items must be 1-D of the same length, got %s and %s" % (users.shape, items.shape))
     out = np.empty(len(users))
-    rc = lib().primalcr_predict(U.ctypes.data, U.shape[0], V.ctypes.data, V.shape[0], U.shape[1], users.ctypes.data,
-                                items.ctypes.data, len(users), out.ctypes.data, device)
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    _check(lib().primalcr_predict(U.ctypes.data, d1, V.ctypes.data, d2, k, users.ctypes.data, items.ctypes.data,
+                                  len(users), out.ctypes.data, device))
     return out
 
 
@@ -212,26 +222,17 @@ def recommend(U, V, n: int, exclude: Ratings | None = None, users=None, device: 
 
     Rows are sorted best first, ties to the smaller item id, NaN scores last; a user with fewer than n eligible items is
     padded with item -1 / score NaN.  users: 0-based ids in any order, repeats allowed (default: every user)."""
-    U = np.ascontiguousarray(U, np.float64); V = np.ascontiguousarray(V, np.float64)
-    if U.ndim != 2 or V.ndim != 2 or U.shape[1] != V.shape[1]:
-        raise PrimalCRError("U and V must be 2-D with the same number of columns, got %s and %s" % (U.shape, V.shape))
-    d1, d2, k = U.shape[0], V.shape[0], U.shape[1]
+    U, V, d1, d2, k = _factors(U, V)
     rp = it = None
     if exclude is not None:
-        if exclude.d1 != d1 or exclude.d2 != d2:
-            raise PrimalCRError("exclude is %d x %d, the factors are %d x %d" % (exclude.d1, exclude.d2, d1, d2))
-        rp = np.ascontiguousarray(exclude.row_ptr, np.int64); it = np.ascontiguousarray(exclude.item, np.int32)
-        if len(rp) != d1 + 1 or len(it) < rp[-1]:
-            raise PrimalCRError("exclude: row_ptr needs d1+1 entries and item row_ptr[d1]")
+        rp, it = _csr_arrays(exclude, d1, d2, "exclude")
     if users is not None:
         users = np.ascontiguousarray(users, np.int32).reshape(-1)
     n_users = d1 if users is None else len(users)
     items = np.empty((n_users, max(int(n), 0)), np.int32)
     scores = np.empty((n_users, max(int(n), 0)), np.float64)
-    rc = lib().primalcr_recommend(U.ctypes.data, d1, V.ctypes.data, d2, k, _ptr(rp), _ptr(it), _ptr(users), n_users,
-                                  int(n), items.ctypes.data, scores.ctypes.data, device)
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    _check(lib().primalcr_recommend(U.ctypes.data, d1, V.ctypes.data, d2, k, _ptr(rp), _ptr(it), _ptr(users), n_users,
+                                    int(n), items.ctypes.data, scores.ctypes.data, device))
     return items, scores
 
 
@@ -259,10 +260,8 @@ def similar(M, n: int, measure: str = "cosine", exclude: Ratings | None = None, 
     n_q = rows if queries is None else len(queries)
     ids = np.empty((n_q, max(int(n), 0)), np.int32)
     scores = np.empty((n_q, max(int(n), 0)), np.float64)
-    rc = lib().primalcr_similar(M.ctypes.data, rows, k, SIMILARITY[measure], _ptr(rp), _ptr(it), _ptr(queries), n_q,
-                                int(n), ids.ctypes.data, scores.ctypes.data, device)
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    _check(lib().primalcr_similar(M.ctypes.data, rows, k, SIMILARITY[measure], _ptr(rp), _ptr(it), _ptr(queries), n_q,
+                                  int(n), ids.ctypes.data, scores.ctypes.data, device))
     return ids, scores
 
 
@@ -282,20 +281,15 @@ def heldout_ranks(U, V, heldout: Ratings, exclude: Ratings | None = None, device
     rank = 1 + the number of the user's items outside `exclude` (normally the training set) that api.recommend would put
     before the entry's item; 0 when the item itself is excluded.  So an entry of rank r <= n is at position r-1 of
     api.recommend(U, V, n, exclude)'s row for that user, with the same score bit for bit."""
-    U = np.ascontiguousarray(U, np.float64); V = np.ascontiguousarray(V, np.float64)
-    if U.ndim != 2 or V.ndim != 2 or U.shape[1] != V.shape[1]:
-        raise PrimalCRError("U and V must be 2-D with the same number of columns, got %s and %s" % (U.shape, V.shape))
-    d1, d2, k = U.shape[0], V.shape[0], U.shape[1]
+    U, V, d1, d2, k = _factors(U, V)
     hp, hi = _csr_arrays(heldout, d1, d2, "heldout")
     rp = it = None
     if exclude is not None:
         rp, it = _csr_arrays(exclude, d1, d2, "exclude")
     nnz = int(hp[-1])
     ranks = np.empty(max(nnz, 0), np.int32); scores = np.empty(max(nnz, 0), np.float64)
-    rc = lib().primalcr_rank_heldout(U.ctypes.data, d1, V.ctypes.data, d2, k, _ptr(rp), _ptr(it), hp.ctypes.data,
-                                     hi.ctypes.data, ranks.ctypes.data, scores.ctypes.data, device)
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    _check(lib().primalcr_rank_heldout(U.ctypes.data, d1, V.ctypes.data, d2, k, _ptr(rp), _ptr(it), hp.ctypes.data,
+                                       hi.ctypes.data, ranks.ctypes.data, scores.ctypes.data, device))
     return ranks, scores
 
 
@@ -317,12 +311,10 @@ def ranking_metrics(ranks, heldout: Ratings, exclude: Ratings | None = None, cut
     nc = len(cuts)
     rec, prec, ndcg = np.empty(nc), np.empty(nc), np.empty(nc)
     mrr, auc, n_users = C.c_double(), C.c_double(), C.c_int64()
-    rc = lib().primalcr_rank_metrics(d1, d2, _ptr(rp), _ptr(it), hp.ctypes.data, hi.ctypes.data, hr.ctypes.data,
-                                     ranks.ctypes.data, -np.inf if min_rating is None else float(min_rating),
-                                     cuts.ctypes.data, nc, rec.ctypes.data, prec.ctypes.data, ndcg.ctypes.data,
-                                     C.byref(mrr), C.byref(auc), C.byref(n_users))
-    if rc != 0:
-        raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+    _check(lib().primalcr_rank_metrics(d1, d2, _ptr(rp), _ptr(it), hp.ctypes.data, hi.ctypes.data, hr.ctypes.data,
+                                       ranks.ctypes.data, -np.inf if min_rating is None else float(min_rating),
+                                       cuts.ctypes.data, nc, rec.ctypes.data, prec.ctypes.data, ndcg.ctypes.data,
+                                       C.byref(mrr), C.byref(auc), C.byref(n_users)))
     out = {}
     for j, n in enumerate(cuts):
         out["recall@%d" % n] = float(rec[j]); out["precision@%d" % n] = float(prec[j]); out["ndcg@%d" % n] = float(ndcg[j])
@@ -364,8 +356,7 @@ class Engine:
         self._keep = []
 
     def _check(self, rc):
-        if rc != 0:
-            raise PrimalCRError("primalcr error %d: %s" % (rc, self._L.primalcr_last_error().decode()))
+        _check(rc)
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -418,9 +409,7 @@ class Engine:
     @staticmethod
     def nccl_unique_id() -> bytes:
         buf = C.create_string_buffer(128)
-        rc = lib().primalcr_nccl_unique_id(buf)
-        if rc != 0:
-            raise PrimalCRError("primalcr error %d: %s" % (rc, lib().primalcr_last_error().decode()))
+        _check(lib().primalcr_nccl_unique_id(buf))
         return buf.raw
 
     def comm_init(self, rank: int, world: int, uid: bytes | None):

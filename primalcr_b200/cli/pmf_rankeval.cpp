@@ -4,15 +4,13 @@
 // The training ratings of data_dir are excluded from every user's candidates and its test ratings are the held-out set;
 // test ratings >= min_rating are relevant (default: all).  Prints one "name value" line per metric ("%.17g"):
 // recall@N, precision@N and ndcg@N per cutoff, then mrr, auc and n_users (the number of evaluated users).
-#include "../host/loader.hpp"
+#include "../host/cli.hpp"
 #include "../host/model.hpp"
 #include "primalcr.h"
 
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
-#include <cstring>
-#include <string>
 #include <vector>
 
 static void usage() {
@@ -53,13 +51,7 @@ int main(int argc, char **argv) {
     long d1 = 0, k = 0, d2 = 0;
     if (!pcrhost::read_model(model_path, W, d1, H, d2, k)) { fprintf(stderr, "can't read model file %s\n", model_path); return 1; }
     pcrhost::DataDir data;
-    try { data = pcrhost::load_dir(data_dir); }
-    catch (const std::exception &ex) { fprintf(stderr, "can't load %s: %s\n", data_dir, ex.what()); return 1; }
-    if (data.train.d1 != d1 || data.train.d2 != d2) {
-        fprintf(stderr, "%s is %lld x %lld, the model is %ld x %ld\n", data_dir, (long long)data.train.d1,
-                (long long)data.train.d2, d1, d2);
-        return 1;
-    }
+    if (!pcrhost::load_model_dir(data_dir, d1, d2, data)) return 1;
     if (!data.has_test) { fprintf(stderr, "%s has no test set to evaluate\n", data_dir); return 1; }
 
     const pcrhost::Csr &X = data.train, &T = data.test;

@@ -5,6 +5,7 @@
 // -q: one 1-based item / user id per line (default: every one).
 // Writes one "query neighbour score" line per neighbour: 1-based ids, "%.17g" scores (the doubles round-trip), queries in
 // request order, best first; a query is never its own neighbour, and padding entries (fewer than topN rows) are not written.
+#include "../host/cli.hpp"
 #include "../host/model.hpp"
 #include "primalcr.h"
 
@@ -53,16 +54,7 @@ int main(int argc, char **argv) {
     const long n = users_side ? d1 : d2;
 
     std::vector<int32_t> queries;
-    if (ids_file) {
-        FILE *fp = fopen(ids_file, "r");
-        if (!fp) { fprintf(stderr, "can't open ids file %s\n", ids_file); return 1; }
-        long q;
-        while (fscanf(fp, "%ld", &q) == 1) {
-            if (q < 1 || q > n) { fprintf(stderr, "id %ld out of range [1, %ld]\n", q, n); fclose(fp); return 1; }
-            queries.push_back((int32_t)(q - 1));
-        }
-        fclose(fp);
-    }
+    if (ids_file && !pcrhost::read_ids(ids_file, n, "id", queries)) return 1;
     const int64_t n_queries = ids_file ? (int64_t)queries.size() : (int64_t)n;
 
     std::vector<int32_t> ids((size_t)n_queries * (topn > 0 ? topn : 0));
@@ -71,16 +63,6 @@ int main(int argc, char **argv) {
                                     n_queries, topn, ids.data(), scores.data(), device);
     if (rc != 0) { fprintf(stderr, "primalcr_similar failed (%d): %s\n", rc, primalcr_last_error()); return 1; }
 
-    FILE *out = fopen(out_path, "wb");
-    if (!out) { fprintf(stderr, "can't open output file %s\n", out_path); return 1; }
-    for (int64_t t = 0; t < n_queries; ++t) {
-        const long q = ids_file ? (long)queries[t] + 1 : (long)t + 1;
-        for (int j = 0; j < topn; ++j) {
-            const size_t e = (size_t)t * topn + j;
-            if (ids[e] < 0) break;
-            fprintf(out, "%ld %d %.17g\n", q, ids[e] + 1, scores[e]);
-        }
-    }
-    fclose(out);
+    if (!pcrhost::write_topn(out_path, ids_file ? queries.data() : nullptr, n_queries, topn, ids, scores)) return 1;
     return 0;
 }

@@ -13,6 +13,9 @@ namespace pcr {
 
 typedef long long i64;
 
+// leading dimension of every factor-shaped array: rows start on 128-byte lines (a 128-byte row chunk never straddles two)
+inline int ceil16(int k) { return (k + 15) & ~15; }
+
 // ------------------------------------------------------------------ errors
 struct Error : public std::runtime_error {
     int code;

@@ -1,5 +1,5 @@
 // engine.cu -- host orchestration of the Primal-CR / Primal-CR++ alternating Newton-CG loop on one GPU,
-// and the C ABI declared in include/primalcr.h.
+// and the C ABI declared in include/primalcr.h (the one-shot queries are in queries.cu).
 //
 // Control flow mirrors the reference exactly (SURVEY.md 3.2 / 3.3):
 //   update_V  : pcrpp.cpp:415-444 (pcr.cpp:279-330) with solve_delta_new :335-358
@@ -7,9 +7,8 @@
 //   driver    : pcrpp.cpp:841-901 / pcr.cpp:616-704
 // Arithmetic runs in the kernels of k_core.cu / k_pairs.cu.  There is no CPU implementation of any stage.
 #include "kernels.h"
-#include "../../include/primalcr.h"
+#include "abi.h"
 #include "../host/loader.hpp"
-#include "../host/rankmetrics.hpp"
 #include "../host/textio.hpp"
 
 #include <algorithm>
@@ -61,10 +60,7 @@ struct CommKey { int device, rank, world; bool operator<(const CommKey &o) const
 static std::map<CommKey, pcr_ncclComm_t> g_comm_cache;
 static std::mutex g_comm_mutex;
 
-static thread_local std::string g_last_error;
-
-// leading dimension of every factor-shaped array: rows start on 128-byte lines (a 128-byte row chunk never straddles two)
-static int ceil16(int k) { return (k + 15) & ~15; }
+thread_local std::string g_last_error;
 
 struct Engine {
     primalcr_config cfg;
@@ -1001,11 +997,6 @@ using pcr::Engine;
 
 struct primalcr_engine { Engine *impl; };
 
-#define API_BEGIN try {
-#define API_END                                                                  \
-    } catch (const pcr::Error &e) { pcr::g_last_error = e.what(); return e.code; } \
-    catch (const std::exception &e) { pcr::g_last_error = e.what(); return PRIMALCR_EINTERNAL; } \
-    return PRIMALCR_OK;
 #define CHECK_E(e) if (!(e) || !(e)->impl) { pcr::g_last_error = "null engine"; return PRIMALCR_EARG; }
 
 extern "C" {
@@ -1337,221 +1328,6 @@ int primalcr_profile_get(primalcr_engine *e, int idx, const char **name, double 
     API_END
 }
 int64_t primalcr_device_bytes(primalcr_engine *e) { return (e && e->impl) ? e->impl->pool.bytes : -1; }
-
-// ---- prediction (pmf-predict.cpp:57-64) ---------------------------------------------------------------
-int primalcr_predict(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int32_t *user,
-                     const int32_t *item, int64_t n, double *out, int device) {
-    API_BEGIN
-    PCR_REQUIRE(U && V && (n == 0 || (user && item && out)) && k >= 1 && d1 >= 0 && d2 >= 0, "bad argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        throw pcr::Error(PRIMALCR_ECUDA, "no CUDA device available: libprimalcr_b200 has no CPU fallback");
-    for (int64_t t = 0; t < n; ++t)
-        PCR_REQUIRE(user[t] >= 0 && user[t] < d1 && item[t] >= 0 && item[t] < d2, "user/item id out of range");
-    PCR_CUDA(cudaSetDevice(device));
-    const int ld = pcr::ceil16(k);
-    pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
-    cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
-    cudaStream_t st; PCR_CUDA(cudaStreamCreate(&st));
-    ctx.stream = st; ctx.prof = &prof; ctx.sms = prop.multiProcessorCount; ctx.ticket = pool.alloc<unsigned long long>(1);
-    double *Uc = pool.alloc<double>((size_t)d1 * k), *Vc = pool.alloc<double>((size_t)d2 * k);
-    double *Ud = pool.alloc<double>((size_t)d1 * ld), *Vd = pool.alloc<double>((size_t)d2 * ld), *od = pool.alloc<double>((size_t)n);
-    int32_t *ud = pool.alloc<int32_t>((size_t)n), *id = pool.alloc<int32_t>((size_t)n);
-    PCR_CUDA(cudaMemcpyAsync(Uc, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
-    PCR_CUDA(cudaMemcpyAsync(Vc, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
-    PCR_CUDA(cudaMemcpyAsync(ud, user, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-    PCR_CUDA(cudaMemcpyAsync(id, item, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-    pcr::k_pad_copy(ctx, Uc, d1, k, ld, Ud); pcr::k_pad_copy(ctx, Vc, d2, k, ld, Vd);
-    pcr::k_dots(ctx, Ud, ud, Vd, id, n, ld, k, nullptr, od, 0.0);
-    if (n) PCR_CUDA(cudaMemcpyAsync(out, od, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    PCR_CUDA(cudaStreamSynchronize(st));
-    cudaStreamDestroy(st);
-    API_END
-}
-
-// ---- top-N recommendation ---------------------------------------------------------------------------------------
-// the exclusion CSR of primalcr_recommend / primalcr_rank_heldout: both pointers or neither, ascending rows -> its nnz
-static int64_t check_exclusion(int64_t d1, int64_t d2, const int64_t *excl_row_ptr, const int32_t *excl_item) {
-    if (!excl_row_ptr) return 0;
-    const std::string err = pcrhost::csr_error("exclusion", d1, d2, excl_row_ptr, excl_item, true);
-    PCR_REQUIRE(err.empty(), err);
-    return excl_row_ptr[d1];
-}
-
-// exclusion CSR to the device (both nullptr when there is none)
-static void upload_exclusion(pcr::DevPool &pool, cudaStream_t st, int64_t d1, const int64_t *excl_row_ptr,
-                             const int32_t *excl_item, int64_t ex_nnz, int64_t *&exp_d, int32_t *&exi_d) {
-    exp_d = nullptr; exi_d = nullptr;
-    if (!excl_row_ptr) return;
-    exp_d = pool.alloc<int64_t>((size_t)d1 + 1); exi_d = pool.alloc<int32_t>((size_t)ex_nnz);
-    PCR_CUDA(cudaMemcpyAsync(exp_d, excl_row_ptr, sizeof(int64_t) * ((size_t)d1 + 1), cudaMemcpyHostToDevice, st));
-    if (ex_nnz) PCR_CUDA(cudaMemcpyAsync(exi_d, excl_item, sizeof(int32_t) * (size_t)ex_nnz, cudaMemcpyHostToDevice, st));
-}
-
-// Argument checks of a top-N call (primalcr_recommend, primalcr_similar): rows users[0..n_users) of U (d1 x k; users NULL:
-// every row) against the d2 rows of V (d2 x k), with an optional d1 x d2 exclusion CSR.  Throws before any device work;
-// returns the exclusion's nnz.
-static int64_t check_topn(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
-                          const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn,
-                          const int32_t *items_out, int device) {
-    PCR_REQUIRE(k >= 1 && k <= 256, "rank k out of range [1, 256]");
-    PCR_REQUIRE(topn >= 1 && topn <= 256, "topn out of range [1, 256]");
-    PCR_REQUIRE(d1 >= 0 && d2 >= 0 && d1 <= INT32_MAX && d2 <= INT32_MAX, "d1 / d2 out of range");
-    PCR_REQUIRE((U || d1 == 0) && (V || d2 == 0), "null factor matrix");
-    PCR_REQUIRE(n_users >= 0 && (users || n_users == d1), "users == NULL requires n_users == d1");
-    PCR_REQUIRE(n_users == 0 || items_out, "null items_out");
-    PCR_REQUIRE((excl_row_ptr == nullptr) == (excl_item == nullptr), "excl_row_ptr and excl_item must both be given or both be NULL");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        throw pcr::Error(PRIMALCR_ECUDA, "no CUDA device available: libprimalcr_b200 has no CPU fallback");
-    PCR_REQUIRE(device >= 0 && device < ndev, "bad device ordinal");
-    // every id the kernel reads through is checked here, before anything runs
-    bool bad_user = false;
-    if (users) {
-#pragma omp parallel for reduction(|| : bad_user) schedule(static)
-        for (int64_t t = 0; t < n_users; ++t) bad_user = bad_user || users[t] < 0 || users[t] >= d1;
-    }
-    PCR_REQUIRE(!bad_user, "user id out of range");
-    return check_exclusion(d1, d2, excl_row_ptr, excl_item);
-}
-
-// A checked top-N call on a stream and device memory of its own, all released before it returns: uploads U, V (V_is_U:
-// V is U, uploaded once), the row ids and the exclusion CSR, runs launch(ctx, pool, Ud, Vd, exp_d, exi_d, ud, itd, scd)
-// and copies the [n_users x topn] rows back.
-extern "C++" {      // a template: C++ linkage inside the extern "C" block
-template <class Launch>
-static void serve_topn(const double *U, int64_t d1, const double *V, int64_t d2, bool V_is_U, int k,
-                       const int64_t *excl_row_ptr, const int32_t *excl_item, int64_t ex_nnz, const int32_t *users,
-                       int64_t n_users, int topn, int32_t *items_out, double *scores_out, int device, Launch launch) {
-    if (n_users == 0) return;
-    PCR_CUDA(cudaSetDevice(device));
-    pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
-    // declared after the pool, so on every exit the stream is drained and destroyed before the buffers are freed
-    struct StreamGuard { cudaStream_t s = nullptr; ~StreamGuard() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } } } sg;
-    PCR_CUDA(cudaStreamCreateWithFlags(&sg.s, cudaStreamNonBlocking));
-    cudaStream_t st = sg.s;
-    cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
-    ctx.stream = st; ctx.prof = &prof; ctx.sms = prop.multiProcessorCount; ctx.ticket = nullptr;
-    double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = V_is_U ? Ud : pool.alloc<double>((size_t)d2 * k);
-    int32_t *ud = pool.alloc<int32_t>((size_t)n_users), *itd = pool.alloc<int32_t>((size_t)n_users * topn);
-    double *scd = scores_out ? pool.alloc<double>((size_t)n_users * topn) : nullptr;
-    int64_t *exp_d; int32_t *exi_d;
-    if (d1) PCR_CUDA(cudaMemcpyAsync(Ud, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
-    if (d2 && !V_is_U) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
-    if (users) PCR_CUDA(cudaMemcpyAsync(ud, users, sizeof(int32_t) * (size_t)n_users, cudaMemcpyHostToDevice, st));
-    else pcr::k_iota32(ctx, ud, n_users);
-    upload_exclusion(pool, st, d1, excl_row_ptr, excl_item, ex_nnz, exp_d, exi_d);
-    launch(ctx, pool, (const double *)Ud, (const double *)Vd, (const pcr::i64 *)exp_d, (const int32_t *)exi_d,
-           (const int32_t *)ud, itd, scd);
-    PCR_CUDA(cudaMemcpyAsync(items_out, itd, sizeof(int32_t) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
-    if (scores_out) PCR_CUDA(cudaMemcpyAsync(scores_out, scd, sizeof(double) * (size_t)n_users * topn, cudaMemcpyDeviceToHost, st));
-    PCR_CUDA(cudaStreamSynchronize(st));
-}
-}  // extern "C++"
-
-int primalcr_recommend(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
-                       const int32_t *excl_item, const int32_t *users, int64_t n_users, int topn, int32_t *items_out,
-                       double *scores_out, int device) {
-    API_BEGIN
-    const int64_t ex_nnz = check_topn(U, d1, V, d2, k, excl_row_ptr, excl_item, users, n_users, topn, items_out, device);
-    serve_topn(U, d1, V, d2, false, k, excl_row_ptr, excl_item, ex_nnz, users, n_users, topn, items_out, scores_out, device,
-               [&](pcr::Ctx &ctx, pcr::DevPool &, const double *Ud, const double *Vd, const pcr::i64 *exp_d,
-                   const int32_t *exi_d, const int32_t *ud, int32_t *itd, double *scd) {
-                   pcr::k_topn(ctx, Ud, Vd, d2, k, exp_d, exi_d, ud, n_users, topn, itd, scd);
-               });
-    API_END
-}
-
-// ---- similar items / users ---------------------------------------------------------------------------------------
-int primalcr_similar(const double *M, int64_t n, int k, int measure, const int64_t *excl_row_ptr, const int32_t *excl_id,
-                     const int32_t *queries, int64_t n_queries, int topn, int32_t *ids_out, double *scores_out, int device) {
-    API_BEGIN
-    PCR_REQUIRE(measure == PRIMALCR_SIM_DOT || measure == PRIMALCR_SIM_COSINE, "unknown similarity measure");
-    const int64_t ex_nnz = check_topn(M, n, M, n, k, excl_row_ptr, excl_id, queries, n_queries, topn, ids_out, device);
-    serve_topn(M, n, M, n, true, k, excl_row_ptr, excl_id, ex_nnz, queries, n_queries, topn, ids_out, scores_out, device,
-               [&](pcr::Ctx &ctx, pcr::DevPool &pool, const double *Md, const double *, const pcr::i64 *exp_d,
-                   const int32_t *exi_d, const int32_t *qd, int32_t *itd, double *scd) {
-                   const bool cosine = measure == PRIMALCR_SIM_COSINE;
-                   double *norms = cosine ? pool.alloc<double>((size_t)n) : nullptr;
-                   pcr::k_similar(ctx, Md, n, k, cosine, norms, exp_d, exi_d, qd, n_queries, topn, itd, scd);
-               });
-    API_END
-}
-
-// ---- held-out ranking evaluation --------------------------------------------------------------------------------
-int primalcr_rank_heldout(const double *U, int64_t d1, const double *V, int64_t d2, int k, const int64_t *excl_row_ptr,
-                          const int32_t *excl_item, const int64_t *ho_row_ptr, const int32_t *ho_item, int32_t *rank_out,
-                          double *score_out, int device) {
-    API_BEGIN
-    PCR_REQUIRE(k >= 1 && k <= 256, "rank k out of range [1, 256]");
-    PCR_REQUIRE(d1 >= 0 && d2 >= 0 && d1 <= INT32_MAX && d2 <= INT32_MAX, "d1 / d2 out of range");
-    PCR_REQUIRE((U || d1 == 0) && (V || d2 == 0), "null factor matrix");
-    PCR_REQUIRE(ho_row_ptr, "null ho_row_ptr");
-    PCR_REQUIRE((excl_row_ptr == nullptr) == (excl_item == nullptr), "excl_row_ptr and excl_item must both be given or both be NULL");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        throw pcr::Error(PRIMALCR_ECUDA, "no CUDA device available: libprimalcr_b200 has no CPU fallback");
-    PCR_REQUIRE(device >= 0 && device < ndev, "bad device ordinal");
-    // every id the kernel reads through is checked here, before anything runs
-    const int64_t nnz = ho_row_ptr[d1];
-    PCR_REQUIRE(nnz == 0 || (ho_item && rank_out), "null ho_item or rank_out");
-    const std::string err = pcrhost::csr_error("held-out", d1, d2, ho_row_ptr, ho_item, false);
-    PCR_REQUIRE(err.empty(), err);
-    const int64_t ex_nnz = check_exclusion(d1, d2, excl_row_ptr, excl_item);
-    if (nnz == 0) return PRIMALCR_OK;
-    // units: a user and at most RANK_UNIT consecutive entries of its row; they tile [0, nnz) in order
-    std::vector<int32_t> unit_user;
-    std::vector<int64_t> unit_beg;
-    for (int64_t u = 0; u < d1; ++u)
-        for (int64_t e = ho_row_ptr[u]; e < ho_row_ptr[u + 1]; e += pcr::RANK_UNIT) { unit_user.push_back((int32_t)u); unit_beg.push_back(e); }
-    unit_beg.push_back(nnz);
-    const int64_t n_units = (int64_t)unit_user.size();
-    PCR_CUDA(cudaSetDevice(device));
-    pcr::DevPool pool; pcr::Profiler prof; pcr::Ctx ctx;
-    // declared after the pool, so on every exit the stream is drained and destroyed before the buffers are freed
-    struct StreamGuard { cudaStream_t s = nullptr; ~StreamGuard() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } } } sg;
-    PCR_CUDA(cudaStreamCreateWithFlags(&sg.s, cudaStreamNonBlocking));
-    cudaStream_t st = sg.s;
-    cudaDeviceProp prop; PCR_CUDA(cudaGetDeviceProperties(&prop, device));
-    ctx.stream = st; ctx.prof = &prof; ctx.sms = prop.multiProcessorCount; ctx.ticket = nullptr;
-    double *Ud = pool.alloc<double>((size_t)d1 * k), *Vd = pool.alloc<double>((size_t)d2 * k);
-    int32_t *hid = pool.alloc<int32_t>((size_t)nnz), *rkd = pool.alloc<int32_t>((size_t)nnz);
-    int32_t *uud = pool.alloc<int32_t>((size_t)n_units);
-    int64_t *ubd = pool.alloc<int64_t>((size_t)n_units + 1);
-    double *scd = score_out ? pool.alloc<double>((size_t)nnz) : nullptr;
-    int64_t *exp_d; int32_t *exi_d;
-    if (d1) PCR_CUDA(cudaMemcpyAsync(Ud, U, sizeof(double) * (size_t)d1 * k, cudaMemcpyHostToDevice, st));
-    if (d2) PCR_CUDA(cudaMemcpyAsync(Vd, V, sizeof(double) * (size_t)d2 * k, cudaMemcpyHostToDevice, st));
-    PCR_CUDA(cudaMemcpyAsync(hid, ho_item, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-    PCR_CUDA(cudaMemcpyAsync(uud, unit_user.data(), sizeof(int32_t) * (size_t)n_units, cudaMemcpyHostToDevice, st));
-    PCR_CUDA(cudaMemcpyAsync(ubd, unit_beg.data(), sizeof(int64_t) * ((size_t)n_units + 1), cudaMemcpyHostToDevice, st));
-    upload_exclusion(pool, st, d1, excl_row_ptr, excl_item, ex_nnz, exp_d, exi_d);
-    pcr::k_rank_heldout(ctx, Ud, Vd, d2, k, (const pcr::i64 *)exp_d, exi_d, hid, uud, (const pcr::i64 *)ubd, n_units, rkd, scd);
-    PCR_CUDA(cudaMemcpyAsync(rank_out, rkd, sizeof(int32_t) * (size_t)nnz, cudaMemcpyDeviceToHost, st));
-    if (score_out) PCR_CUDA(cudaMemcpyAsync(score_out, scd, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToHost, st));
-    PCR_CUDA(cudaStreamSynchronize(st));
-    API_END
-}
-
-int primalcr_rank_metrics(int64_t d1, int64_t d2, const int64_t *excl_row_ptr, const int32_t *excl_item,
-                          const int64_t *ho_row_ptr, const int32_t *ho_item, const double *ho_rating, const int32_t *rank,
-                          double min_rating, const int32_t *cutoffs, int n_cutoffs, double *recall, double *precision,
-                          double *ndcg, double *mrr, double *auc, int64_t *n_users) {
-    API_BEGIN
-    pcrhost::RankMetrics m;
-    const std::string err = pcrhost::rank_metrics(d1, d2, excl_row_ptr, excl_item, ho_row_ptr, ho_item, ho_rating, rank,
-                                                  min_rating, cutoffs, n_cutoffs, m);
-    PCR_REQUIRE(err.empty(), err);
-    for (int c = 0; c < n_cutoffs; ++c) {
-        if (recall) recall[c] = m.recall[(size_t)c];
-        if (precision) precision[c] = m.precision[(size_t)c];
-        if (ndcg) ndcg[c] = m.ndcg[(size_t)c];
-    }
-    if (mrr) *mrr = m.mrr;
-    if (auc) *auc = m.auc;
-    if (n_users) *n_users = m.n_users;
-    API_END
-}
 
 // ---- host loader ------------------------------------------------------------------------------------------
 struct primalcr_dataset { pcrhost::DataDir d; };
