@@ -116,8 +116,9 @@ int primalcr_get_counters(primalcr_engine *e, primalcr_counters *out);
 /* ---- per-stage entry points (parity tests call these through the same library) ----------------- */
 /* comp_m_new pcrpp.cpp:17 : scores of every training rating, CSR order */
 int primalcr_scores(primalcr_engine *e, double *m_out);
-/* load externally supplied scores (so sort / counts can be compared bit-exactly on identical inputs); training-set
-   evaluation (which = 0) then evaluates the loaded scores until the factors or the scores change */
+/* load externally supplied scores (so sort / counts can be compared bit-exactly on identical inputs).  Until the factors
+   or the scores change, they stand in for the scores of the current factors in every call: training-set evaluation
+   (which = 0), the objective and stage outputs, and the next update_V or update_U, which consume them. */
 int primalcr_set_scores(primalcr_engine *e, const double *m);
 /* get_sorted_mm pcrpp.cpp:52 + the window pointers of the sweep pcrpp.cpp:214-229, for all users:
    per rating, in (user, ascending score) order: sorted score, local index of that score inside its user,

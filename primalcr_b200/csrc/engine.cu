@@ -92,7 +92,16 @@ struct Engine {
     // per-rating work buffers
     double *m = nullptr, *b = nullptr, *cbuf = nullptr;
     SortedMeta meta;
-    bool scores_valid = false, meta_valid = false;
+    // What m, the sorted state `meta` and the per-user losses us.loss hold.  Only the methods under "what m holds",
+    // prepare, and update_V / update_U when they commit write it.  CURRENT: comp_m(U, V) for every user, or the scores
+    // loaded by load_scores.  V_TRIAL: comp_m(U, Vnew) of update_V's last, rejected, line-search trial.
+    enum class MHolds { NOTHING, CURRENT, V_TRIAL };
+    struct ScoreState {
+        MHolds m = MHolds::NOTHING;
+        bool sorted = false;            // meta is the Primal-CR++ sorted state of m
+        bool losses = false;            // us.loss holds the per-user losses of m
+        bool v_trial_pending = false;   // update_V rejected every trial, no update_U or write ran since: Vnew holds it
+    } held;
     // heavy-user scratch of the one-CTA-per-user kernels (allocated on demand: T > 8, or the score-order outputs for tests)
     double *h_v = nullptr, *h_p1 = nullptr, *h_p2 = nullptr, *h_acc = nullptr; int32_t *h_cnt = nullptr;
     HeavyLM hv;                       // chunk-parallel heavy-user path (k_heavy.cu)
@@ -113,7 +122,6 @@ struct Engine {
     // comm
     int rank = 0, world = 1; pcr_ncclComm_t comm = nullptr;
     primalcr_counters counters;
-    int v_accepted = 1;
 
     explicit Engine(const primalcr_config &c) : cfg(c) {
         memset(&counters, 0, sizeof(counters));
@@ -180,6 +188,15 @@ struct Engine {
         return d;
     }
     template <typename Tp> Tp *upload_vec(const std::vector<Tp> &v) { return upload(v.data(), v.size()); }
+    // the int flag that `check(flag)` sets on the device: zeroed before the launch, read once the stream has drained
+    template <typename F> int device_flag(F check) {
+        int *flag = (int *)pool.raw_alloc(sizeof(int));
+        PCR_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), stream));
+        check(flag);
+        PCR_CUDA(cudaMemcpyAsync(h_counters, flag, sizeof(int), cudaMemcpyDeviceToHost, stream));
+        sync(); pool.raw_free(flag);
+        return h_counters[0];
+    }
 
     // ------------------------------------------------------------------ data
     void build_csr_common(DevCsr &C, i64 d1_, i64 nnz, const i64 *row_ptr, const int32_t *item, const double *rating) {
@@ -191,14 +208,8 @@ struct Engine {
         C.item = upload(item, (size_t)nnz);
         C.rating = upload(rating, (size_t)nnz);
         C.user = pool.alloc<int32_t>((size_t)nnz);
-        {   // item ids are used as array indices by every kernel: validate them first
-            int *bad = pool.alloc<int>(1);
-            PCR_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), stream));
-            k_check_range(ctx, C.item, nnz, d2, bad);
-            PCR_CUDA(cudaMemcpyAsync(h_counters, bad, sizeof(int), cudaMemcpyDeviceToHost, stream));
-            PCR_CUDA(cudaStreamSynchronize(stream));
-            PCR_REQUIRE(h_counters[0] == 0, "item id out of range [0, d2)");
-        }
+        // item ids are used as array indices by every kernel: validate them first
+        PCR_REQUIRE(device_flag([&](int *bad) { k_check_range(ctx, C.item, nnz, d2, bad); }) == 0, "item id out of range [0, d2)");
         for (i64 u = 0; u < d1_; ++u) PCR_REQUIRE(C.h_row_ptr[u + 1] >= C.h_row_ptr[u], "row_ptr must be non-decreasing");
         k_expand_users(ctx, C.row_ptr, d1_, nnz, C.user);
         // pair-tile work items
@@ -252,10 +263,19 @@ struct Engine {
         PCR_REQUIRE(!has_train, "training set already loaded (one data set per engine)");
         PCR_REQUIRE(d1_ >= 0 && d2_ >= 1 && nnz >= 0, "bad sizes");
         d1 = d1_; d2 = d2_;
-        build_csr_common(X, d1_, nnz, row_ptr, item, rating);
-        lap("upload CSR + pair tiles");
-        // ---- rating levels (find_levels pcrpp.cpp:38-49, as one global order-preserving table).  Primal-CR (-s 1) never
-        // looks at levels (pcr.cpp compares the exact ratings), so any rating scale is accepted there.
+        build_csr_common(X, d1_, nnz, row_ptr, item, rating);   lap("upload CSR + pair tiles");
+        build_levels(rating);                                   lap("levels");
+        const std::vector<int32_t> heavy = build_classes_and_tiles();
+        build_heavy_plans(heavy);
+        build_user_units();                                     lap("classes, tiles, user units");
+        build_csc_and_item_units(lap);                          lap("item units (user blocks)");
+        alloc_work_buffers();                                   lap("work buffers");
+        has_train = true;
+    }
+    // ---- rating levels (find_levels pcrpp.cpp:38-49, as one global order-preserving table).  Primal-CR (-s 1) never
+    // looks at levels (pcr.cpp compares the exact ratings), so any rating scale is accepted there.
+    void build_levels(const double *rating) {
+        const i64 nnz = X.nnz;
         X.level = pool.alloc<uint8_t>((size_t)nnz);
         if (cfg.solver == 1) {
             levels.assign(1, 0); T = 1;
@@ -292,25 +312,18 @@ struct Engine {
                 levels = distinct;
             }
             T = (int)levels.size();
-            {
-                std::vector<double> lv(std::max<size_t>(levels.size(), 8), 0.0);
-                for (size_t q = 0; q < levels.size(); ++q) lv[q] = (double)levels[q];
-                level_vals = upload_vec(lv);
-            }
+            std::vector<double> lv(std::max<size_t>(levels.size(), 8), 0.0);
+            for (size_t q = 0; q < levels.size(); ++q) lv[q] = (double)levels[q];
+            level_vals = upload_vec(lv);
             i64 *tab = upload_vec(levels);
-            int *bad = pool.alloc<int>(1);
-            PCR_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), stream));
-            k_levels(ctx, X.rating, nnz, tab, T, X.level, bad);
-            PCR_CUDA(cudaMemcpyAsync(h_counters, bad, sizeof(int), cudaMemcpyDeviceToHost, stream));
-            sync();
-            PCR_REQUIRE((h_counters[0] & 1) == 0, "a rating rounds to a level that is not in the level table");
-            ratings_integer = (h_counters[0] & 2) == 0;
+            const int bad = device_flag([&](int *flag) { k_levels(ctx, X.rating, nnz, tab, T, X.level, flag); });
+            PCR_REQUIRE((bad & 1) == 0, "a rating rounds to a level that is not in the level table");
+            ratings_integer = (bad & 2) == 0;
         }
-        lap("levels");
-        // ---- size classes, heavy scratch
+    }
+    // ---- size classes and tiles; returns the users of the heavy class
+    std::vector<int32_t> build_classes_and_tiles() {
         std::vector<int32_t> cls[3];
-        std::vector<i64> hoff((size_t)d1, -1), hb, he;
-        i64 htot = 0;
         use_tiles = T <= 8;
         // tiles: runs of consecutive users; geometry 0 takes users with len <= TILE_CAP, geometry 1 users with
         // TILE_CAP < len <= TILE_CAP_M, geometry 2 users with TILE_CAP_M < len <= TILE_CAP_L; anything longer is heavy
@@ -329,7 +342,7 @@ struct Engine {
             if (len == 0) continue;
             if (len <= S_CAP) cls[0].push_back((int32_t)u);
             else if (len <= L_CAP) cls[1].push_back((int32_t)u);
-            else { cls[2].push_back((int32_t)u); hoff[u] = htot; htot += len + 1; hb.push_back(X.h_row_ptr[u]); he.push_back(X.h_row_ptr[u + 1]); }
+            else cls[2].push_back((int32_t)u);
         }
         for (int gq = 0; gq < 3; ++gq) {
             tb[gq].close();
@@ -344,56 +357,61 @@ struct Engine {
             sync();
         }
         for (int q = 0; q < 3; ++q) { X.n_cls[q] = (int)cls[q].size(); X.cls_users[q] = upload_vec(cls[q]); }
+        sync();
+        return cls[2];
+    }
+    // ---- the heavy users' scratch layout (users len + 1 apart).  Their segmented sort (k_hsort.cu, any T) and, on the
+    // tile path, their chunk-parallel sweeps (k_heavy.cu) walk one work list: chunks of HEAVY_CHUNK ratings as (index
+    // of the heavy user, first rating inside it).
+    void build_heavy_plans(const std::vector<int32_t> &heavy) {
+        std::vector<i64> hoff((size_t)d1, -1), hb, he, off, soff; std::vector<int32_t> cu, clo, c0;
+        i64 htot = 0, run = 0, maxlen = 0;
+        for (size_t q = 0; q < heavy.size(); ++q) {
+            const i64 u = heavy[q], len = X.h_row_ptr[u + 1] - X.h_row_ptr[u];
+            hb.push_back(X.h_row_ptr[u]); he.push_back(X.h_row_ptr[u + 1]);
+            off.push_back(htot); hoff[u] = htot; htot += len + 1;
+            soff.push_back(run); run += len; maxlen = std::max(maxlen, len);
+            c0.push_back((int32_t)cu.size());
+            for (i64 lo = 0; lo < len; lo += HEAVY_CHUNK) { cu.push_back((int32_t)q); clo.push_back((int32_t)lo); }
+        }
+        c0.push_back((int32_t)cu.size());
         X.heavy_off = upload_vec(hoff); X.heavy_total = htot;
         X.heavy_begin = upload_vec(hb); X.heavy_end = upload_vec(he);
-        if (!cls[2].empty()) {            // work list of the heavy-user sort: the same chunks of 2048 ratings, any T
-            std::vector<i64> soff; std::vector<int32_t> scu, sclo;
-            i64 run = 0, maxlen = 0;
-            for (size_t q = 0; q < cls[2].size(); ++q) {
-                const i64 len = he[q] - hb[q];
-                soff.push_back(run); run += len; maxlen = std::max(maxlen, len);
-                for (i64 lo = 0; lo < len; lo += HEAVY_CHUNK) { scu.push_back((int32_t)q); sclo.push_back((int32_t)lo); }
-            }
-            hsort.n_users = (int)cls[2].size(); hsort.n_chunks = (int)scu.size();
-            hsort.max_passes = 0;
-            while (((i64)HEAVY_CHUNK << hsort.max_passes) < maxlen) ++hsort.max_passes;
-            hsort.begin = X.heavy_begin; hsort.end = X.heavy_end;
-            hsort.off = upload_vec(soff); hsort.chunk_user = upload_vec(scu); hsort.chunk_lo = upload_vec(sclo);
-            hsort.tmp_s = pool.alloc<double>((size_t)run); hsort.tmp_pos = pool.alloc<int32_t>((size_t)run);
-            sync();
-        }
-        heavy_chunked = use_tiles && !cls[2].empty();
+        heavy_chunked = use_tiles && !heavy.empty();
+        if (heavy.empty()) { sync(); return; }
+        const int32_t *chunk_user = upload_vec(cu), *chunk_lo = upload_vec(clo);
+        hsort.n_users = (int)heavy.size(); hsort.n_chunks = (int)cu.size();
+        hsort.max_passes = 0;
+        while (((i64)HEAVY_CHUNK << hsort.max_passes) < maxlen) ++hsort.max_passes;
+        hsort.begin = X.heavy_begin; hsort.end = X.heavy_end;
+        hsort.off = upload_vec(soff); hsort.chunk_user = chunk_user; hsort.chunk_lo = chunk_lo;
+        hsort.tmp_s = pool.alloc<double>((size_t)run); hsort.tmp_pos = pool.alloc<int32_t>((size_t)run);
         if (heavy_chunked) {
-            std::vector<i64> hoff_h; std::vector<int32_t> cu, clo, c0;
-            for (size_t q = 0; q < cls[2].size(); ++q) {
-                hoff_h.push_back(hoff[cls[2][q]]);
-                c0.push_back((int32_t)cu.size());
-                for (i64 lo = 0; lo < he[q] - hb[q]; lo += HEAVY_CHUNK) { cu.push_back((int32_t)q); clo.push_back((int32_t)lo); }
-            }
-            c0.push_back((int32_t)cu.size());
-            hv.n_users = (int)cls[2].size(); hv.n_chunks = (int)cu.size(); hv.htot = htot;
+            hv.n_users = hsort.n_users; hv.n_chunks = hsort.n_chunks; hv.htot = htot;
             hv.users = X.cls_users[2]; hv.begin = X.heavy_begin; hv.end = X.heavy_end;
-            hv.off = upload_vec(hoff_h); hv.chunk_user = upload_vec(cu); hv.chunk_lo = upload_vec(clo); hv.chunk0 = upload_vec(c0);
+            hv.off = upload_vec(off); hv.chunk_user = chunk_user; hv.chunk_lo = chunk_lo; hv.chunk0 = upload_vec(c0);
             hv.ccnt = pool.alloc<int32_t>((size_t)hv.n_chunks * 8); hv.B = pool.alloc<int32_t>((size_t)hv.n_users * 9);
             hv.idx = pool.alloc<int32_t>((size_t)std::max(T - 1, 1) * (size_t)htot);
             hv.G = pool.alloc<double>((size_t)htot); hv.G2 = pool.alloc<double>((size_t)htot);
             hv.pos = pool.alloc<int32_t>((size_t)htot); hv.lo = pool.alloc<int32_t>((size_t)htot); hv.hi = pool.alloc<int32_t>((size_t)htot);
             hv.lev = pool.alloc<uint8_t>((size_t)htot);
             hv.csum = pool.alloc<double>((size_t)hv.n_chunks * 2);
-            sync();
         } else {
             alloc_heavy_cta_scratch();
         }
-        // ---- row-sum work units over the CSR
-        {
-            std::vector<int32_t> useg; std::vector<i64> ustart, supt;
-            make_units(X.h_row_ptr, useg, ustart, supt);
-            X.n_units = (i64)useg.size();
-            X.un_seg = upload_vec(useg); X.un_start = upload_vec(ustart); X.seg_unit_ptr = upload_vec(supt);
-            sync();
-        }
-        lap("classes, tiles, user units");
-        // ---- CSC by item + its work units
+        sync();
+    }
+    // ---- row-sum work units over the CSR
+    void build_user_units() {
+        std::vector<int32_t> useg; std::vector<i64> ustart, supt;
+        make_units(X.h_row_ptr, useg, ustart, supt);
+        X.n_units = (i64)useg.size();
+        X.un_seg = upload_vec(useg); X.un_start = upload_vec(ustart); X.seg_unit_ptr = upload_vec(supt);
+        sync();
+    }
+    // ---- CSC by item, and the work units of the item-major row sum over it
+    void build_csc_and_item_units(Lap &lap) {
+        const i64 nnz = X.nnz;
         col_ptr = pool.alloc<i64>((size_t)d2 + 1);
         csc2csr = pool.alloc<int32_t>((size_t)nnz); csc_user = pool.alloc<int32_t>((size_t)nnz);
         k_build_csc(ctx, pool, X.item, X.user, nnz, d2, col_ptr, csc2csr, csc_user);
@@ -405,51 +423,49 @@ struct Engine {
         // Work units of the item-major row sum, ordered USER-BLOCK-major: every unit only touches U rows of one block
         // of <= ~40 MB, so while the persistent grid walks the unit list the gathered rows stay L2-resident
         // (users ascend inside a column, so a column's entries of one block are contiguous).
-        {
-            const double blk_bytes = getenv("PRIMALCR_UBLOCK_MB") ? atof(getenv("PRIMALCR_UBLOCK_MB")) * 1e6 : 24e6;
-            const double u_bytes = (double)d1 * ld * 8.0;
-            int nb = (int)std::ceil(u_bytes / blk_bytes);
-            // ... but never so many blocks that an (item, user block) unit averages fewer than ~32 ratings: with many
-            // items (Yahoo / power-law shapes, d2 >= 500 k) the tiny units and their partial rows cost more than the L2
-            // misses of a larger block (measured: 24 MB -> ~100 MB blocks, -8 % per iteration on both shapes)
-            if (getenv("PRIMALCR_UBLOCK_MB") == nullptr) {
-                const i64 nb_max = std::max<i64>(1, nnz / (32 * std::max<i64>(d2, 1)));
-                if (nb > nb_max) nb = (int)nb_max;
-            }
-            if (nb < 1) nb = 1;
-            if (nb > 64) nb = 64;
-            const i64 bu = (d1 + nb - 1) / nb > 0 ? (d1 + nb - 1) / nb : 1;
-            n_user_blocks = nb;
-            std::vector<i64> bpos((size_t)d2 * (nb + 1));
-            i64 *bpos_d = nullptr;
-            bpos_d = (i64 *)pool.raw_alloc(sizeof(i64) * bpos.size());
-            k_csc_block_bounds(ctx, col_ptr, csc_user, d2, nb, bu, bpos_d);
-            PCR_CUDA(cudaMemcpyAsync(bpos.data(), bpos_d, sizeof(i64) * bpos.size(), cudaMemcpyDeviceToHost, stream));
-            sync();
-            pool.raw_free(bpos_d);
-            std::vector<int32_t> cseg, cidx; std::vector<i64> cstart, cend, csup((size_t)d2 + 1, 0);
-            for (int blk = 0; blk < nb; ++blk)
-                for (i64 pcol = 0; pcol < d2; ++pcol) {
-                    const i64 lo = bpos[(size_t)pcol * (nb + 1) + blk], hi = blk + 1 == nb ? h_col[pcol + 1] : bpos[(size_t)pcol * (nb + 1) + blk + 1];
-                    // popular items get longer units so that no item has more than ~48 + nb partial sums to add up
-                    const i64 collen = h_col[pcol + 1] - h_col[pcol];
-                    const i64 chunk = std::max<i64>(ROWSUM_CHUNK, (collen + 47) / 48);
-                    for (i64 bb = lo; bb < hi; bb += chunk) {
-                        cseg.push_back((int32_t)pcol); cstart.push_back(bb); cend.push_back(std::min(bb + chunk, hi));
-                        csup[pcol + 1] += 1;
-                    }
-                }
-            n_cunits = (i64)cseg.size();
-            for (i64 pcol = 0; pcol < d2; ++pcol) csup[pcol + 1] += csup[pcol];
-            cidx.resize(cseg.size());
-            std::vector<i64> fill(csup.begin(), csup.end() - 1);
-            for (size_t uu = 0; uu < cseg.size(); ++uu) cidx[fill[cseg[uu]]++] = (int32_t)uu;
-            cu_seg = upload_vec(cseg); cu_start = upload_vec(cstart); cu_end = upload_vec(cend);
-            col_unit_ptr = upload_vec(csup); col_unit_idx = upload_vec(cidx);
-            sync();
+        const double blk_bytes = getenv("PRIMALCR_UBLOCK_MB") ? atof(getenv("PRIMALCR_UBLOCK_MB")) * 1e6 : 24e6;
+        const double u_bytes = (double)d1 * ld * 8.0;
+        int nb = (int)std::ceil(u_bytes / blk_bytes);
+        // ... but never so many blocks that an (item, user block) unit averages fewer than ~32 ratings: with many
+        // items (Yahoo / power-law shapes, d2 >= 500 k) the tiny units and their partial rows cost more than the L2
+        // misses of a larger block (measured: 24 MB -> ~100 MB blocks, -8 % per iteration on both shapes)
+        if (getenv("PRIMALCR_UBLOCK_MB") == nullptr) {
+            const i64 nb_max = std::max<i64>(1, nnz / (32 * std::max<i64>(d2, 1)));
+            if (nb > nb_max) nb = (int)nb_max;
         }
-        lap("item units (user blocks)");
-        // ---- work buffers
+        if (nb < 1) nb = 1;
+        if (nb > 64) nb = 64;
+        const i64 bu = (d1 + nb - 1) / nb > 0 ? (d1 + nb - 1) / nb : 1;
+        n_user_blocks = nb;
+        std::vector<i64> bpos((size_t)d2 * (nb + 1));
+        i64 *bpos_d = (i64 *)pool.raw_alloc(sizeof(i64) * bpos.size());
+        k_csc_block_bounds(ctx, col_ptr, csc_user, d2, nb, bu, bpos_d);
+        PCR_CUDA(cudaMemcpyAsync(bpos.data(), bpos_d, sizeof(i64) * bpos.size(), cudaMemcpyDeviceToHost, stream));
+        sync();
+        pool.raw_free(bpos_d);
+        std::vector<int32_t> cseg, cidx; std::vector<i64> cstart, cend, csup((size_t)d2 + 1, 0);
+        for (int blk = 0; blk < nb; ++blk)
+            for (i64 pcol = 0; pcol < d2; ++pcol) {
+                const i64 lo = bpos[(size_t)pcol * (nb + 1) + blk], hi = blk + 1 == nb ? h_col[pcol + 1] : bpos[(size_t)pcol * (nb + 1) + blk + 1];
+                // popular items get longer units so that no item has more than ~48 + nb partial sums to add up
+                const i64 collen = h_col[pcol + 1] - h_col[pcol];
+                const i64 chunk = std::max<i64>(ROWSUM_CHUNK, (collen + 47) / 48);
+                for (i64 bb = lo; bb < hi; bb += chunk) {
+                    cseg.push_back((int32_t)pcol); cstart.push_back(bb); cend.push_back(std::min(bb + chunk, hi));
+                    csup[pcol + 1] += 1;
+                }
+            }
+        n_cunits = (i64)cseg.size();
+        for (i64 pcol = 0; pcol < d2; ++pcol) csup[pcol + 1] += csup[pcol];
+        cidx.resize(cseg.size());
+        std::vector<i64> fill(csup.begin(), csup.end() - 1);
+        for (size_t uu = 0; uu < cseg.size(); ++uu) cidx[fill[cseg[uu]]++] = (int32_t)uu;
+        cu_seg = upload_vec(cseg); cu_start = upload_vec(cstart); cu_end = upload_vec(cend);
+        col_unit_ptr = upload_vec(csup); col_unit_idx = upload_vec(cidx);
+        sync();
+    }
+    void alloc_work_buffers() {
+        const i64 nnz = X.nnz;
         m = pool.alloc<double>((size_t)nnz); b = pool.alloc<double>((size_t)nnz); cbuf = pool.alloc<double>((size_t)nnz);
         meta.s = pool.alloc<double>((size_t)nnz); meta.pos = pool.alloc<int32_t>((size_t)nnz);
         meta.lev = pool.alloc<uint8_t>((size_t)nnz);
@@ -491,8 +507,6 @@ struct Engine {
         obj_item = pool.alloc<double>((size_t)X.n_pt);
         ensure_eval_buffers(X);
         sync();
-        lap("work buffers");
-        has_train = true;
     }
 
     void alloc_heavy_cta_scratch() {
@@ -561,7 +575,8 @@ struct Engine {
         PCR_REQUIRE(has_train, "load the training set first");
         put_matrix(Uh, d1, U); put_matrix(Vh, d2, V);
         sync();
-        has_factors = true; scores_valid = false; meta_valid = false; loss_matches_m = false; last_m_is_stale = false; v_trial_pending = false;
+        has_factors = true;
+        forget();
     }
     void get_factors(double *Uh, double *Vh) {
         bind();
@@ -591,11 +606,7 @@ struct Engine {
     }
     double pass_bytes(i64 n, i64 prows) const { return (double)n * (8.0 * k + 12.0) + 8.0 * k * (double)prows; }
 
-    // scores of all training ratings under (Um, Vm): comp_m_new pcrpp.cpp:17-35
-    void scores(const double *Um, const double *Vm, double *out, const uint8_t *active) {
-        train_dots(Um, Vm, out, active);
-    }
-    // out[e] = P[user(e)] . Q[item(e)] over the training set
+    // out[e] = P[user(e)] . Q[item(e)] over the training set (the scores comp_m_new pcrpp.cpp:17-35 for P = U, Q = V)
     void train_dots(const double *P, const double *Q, double *out, const uint8_t *active) {
         const double bytes = active ? 0.0 : pass_bytes(X.nnz, d1);
         k_dots_units(ctx, X.un_seg, X.un_start, nullptr, X.n_units, P, Q, X.item, ld, k, active, out, bytes);
@@ -618,7 +629,7 @@ struct Engine {
         }
         if (heavy_chunked) join_aux();
         heavy_windows_valid = false;
-        meta_valid = true;
+        held.sorted = true;
     }
     void sweep_coeff(int mode, const uint8_t *active, const double *bsrc) {
         if (heavy_chunked) { fork_aux(); k_heavy_sweep(ctx_aux, mode, hv, active, meta, bsrc, cbuf, nullptr, T); }
@@ -700,30 +711,65 @@ struct Engine {
         PCR_REQUIRE(has_train && has_factors, "engine needs a training set and factors");
         bind();
     }
-    void ensure_scores() {
-        if (scores_valid) return;
-        scores(U, V, m, nullptr);
-        scores_valid = true; meta_valid = false; loss_matches_m = false;
-        last_m_is_stale = false;      // m is comp_m(U, V) again, no longer the scores of a rejected V trial
+    // ------------------------------------------------------------------ what m holds (see `held`)
+    void forget() { held = ScoreState(); }
+    void score_current() { train_dots(U, V, m, nullptr); held.m = MHolds::CURRENT; held.sorted = held.losses = false; }
+    // externally supplied scores stand in for comp_m(U, V) until the factors or the scores change
+    void load_scores(const double *h) {
+        require_ready();
+        PCR_REQUIRE(h != nullptr || X.nnz == 0, "null scores");
+        if (X.nnz) PCR_CUDA(cudaMemcpyAsync(m, h, sizeof(double) * (size_t)X.nnz, cudaMemcpyHostToDevice, stream));
+        sync();
+        forget(); held.m = MHolds::CURRENT;
     }
-    void ensure_meta() { ensure_scores(); if (cfg.solver == 2 && !meta_valid) prepare(m, nullptr); }
+    // comp_m_new + get_sorted_mm + objective_new of the line-search trial (U, Vnew)   pcrpp.cpp:429-431
+    void score_v_trial() {
+        train_dots(U, Vnew, m, nullptr); held.m = MHolds::V_TRIAL; held.sorted = false;
+        if (cfg.solver == 2) prepare(m, nullptr);
+        user_losses(m, nullptr); held.losses = true;
+    }
+    void ensure_scores() { if (held.m != MHolds::CURRENT) score_current(); }
+    void ensure_meta() { ensure_scores(); if (cfg.solver == 2 && !held.sorted) prepare(m, nullptr); }
 
     // ------------------------------------------------------------------ stage entry points
+    double initial_objective() { require_ready(); forget(); return objective_current(); }   // from the factors alone
     double objective_current() {   // objective_new(m, U, V) / objective(m, U, V)
         require_ready(); ensure_meta();
         user_losses(m, nullptr);
         return total_objective(U, V);
     }
-    void grad_V(double *out_dev) { // obtain_g_new / obtain_g
+    void scores_stage() { require_ready(); score_current(); }
+    void sort_segments() {         // rebuilds the sorted state of the current scores even when it exists
+        require_ready(); PCR_REQUIRE(cfg.solver == 2, "sorted state exists only for Primal-CR++");
+        ensure_scores();
+        prepare(m, nullptr);
+        ensure_heavy_windows();
+    }
+    // count_left / count_right of every rating and level: host arrays of [nnz x T], either may be null
+    void level_counts(int32_t *cnt_left, int32_t *cnt_right) {
+        require_ready(); PCR_REQUIRE(cfg.solver == 2, "sorted state exists only for Primal-CR++");
+        ensure_meta();
+        ensure_heavy_windows();
+        const size_t n = (size_t)X.nnz * T;
+        int32_t *dl = (int32_t *)pool.raw_alloc(sizeof(int32_t) * n), *dr = (int32_t *)pool.raw_alloc(sizeof(int32_t) * n);
+        k_level_counts(ctx, X.row_ptr, d1, meta, T, dl, dr);
+        sync();
+        if (n && cnt_left) PCR_CUDA(cudaMemcpy(cnt_left, dl, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
+        if (n && cnt_right) PCR_CUDA(cudaMemcpy(cnt_right, dr, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
+        pool.raw_free(dl); pool.raw_free(dr);
+    }
+    void grad_V() {                // obtain_g_new / obtain_g into g
         require_ready(); ensure_meta();
         coeffs(0, nullptr);
-        rowsum_items(V, out_dev);
+        rowsum_items(V, g);
     }
-    void hv_V(const double *a_dev, double *out_dev) {   // compute_Ha_new / compute_Ha
-        require_ready(); ensure_meta();
-        train_dots(U, a_dev, b, nullptr);
+    void hv_V(const double *a) {   // compute_Ha_new / compute_Ha of the host direction a [d2 x k] into Hp
+        require_ready(); PCR_REQUIRE(a != nullptr, "null direction");
+        put_matrix(a, d2, p);
+        ensure_meta();
+        train_dots(U, p, b, nullptr);
         coeffs(1, nullptr);
-        rowsum_items(a_dev, out_dev);
+        rowsum_items(p, Hp);
     }
 
     // ------------------------------------------------------------------ update_V(_new)
@@ -732,15 +778,12 @@ struct Engine {
         const i64 vn = d2 * ld;
         // comp_m_new + get_sorted_mm (:417-418).  After an update_U the scores, the sorted state and the per-user losses of
         // every user's LAST line-search trial are exactly those of the committed (U, V) -- same kernels, same inputs --
-        // so they are reused instead of being recomputed (update_U sets the three flags only when that holds).
-        if (!(scores_valid && (cfg.solver != 2 || meta_valid))) {
-            scores(U, V, m, nullptr); scores_valid = true; meta_valid = false; loss_matches_m = false;
-            if (cfg.solver == 2) prepare(m, nullptr);
-        }
+        // so they are reused instead of being recomputed (update_U leaves them marked current only when that holds).
+        ensure_meta();
         coeffs(0, nullptr);
         if (sharded_cg) rowsum_items_rs(V, g); else rowsum_items(V, g);
         // prev_obj = objective(m, U, V): m and the sorted state do not change during CG, so evaluate it now
-        if (!loss_matches_m) user_losses(m, nullptr);
+        if (!held.losses) user_losses(m, nullptr);
         const double prev_obj = total_objective(U, V);
         // ---- solve_delta(_new): pcrpp.cpp:335-358
         int its = 0;
@@ -803,56 +846,40 @@ struct Engine {
         int trials = 0, accepted = 0;
         for (int iter = 0; iter < 20; ++iter) {
             k_axpby(ctx, Vnew, 1.0, V, -stepsize, delta, vn);
-            scores(U, Vnew, m, nullptr);
-            if (cfg.solver == 2) prepare(m, nullptr);
-            user_losses(m, nullptr);
+            score_v_trial();
             now_obj = total_objective(U, Vnew);
             ++trials;
-            if (now_obj < prev_obj) { std::swap(V, Vnew); accepted = 1; break; }
+            if (now_obj < prev_obj) { std::swap(V, Vnew); held.m = MHolds::CURRENT; accepted = 1; break; }
             stepsize /= 2.0;
         }
         // m (and the sorted state) are those of the LAST trial, accepted or not -- as in the reference (:443)
-        scores_valid = accepted != 0;   // if rejected, m belongs to a V that was thrown away
-        loss_matches_m = true;
+        held.v_trial_pending = !accepted;
         counters.v_cg_iters = its; counters.v_ls_trials = trials; counters.v_ls_accepted = accepted;
-        v_accepted = accepted;
-        last_m_is_stale = !accepted;
-        v_trial_pending = !accepted;
         return now_obj;
     }
-    bool last_m_is_stale = false;
-    // update_V rejected every trial and no update_U or write has run since: Vnew still holds the last trial's V.  A read-only
-    // call may replace m (ensure_scores, primalcr_scores) in the meantime; update_U then rebuilds that trial's state from
-    // (U, Vnew) -- the same kernels on the same inputs, so the same bits -- and consumes it as if nothing had been read.
-    bool v_trial_pending = false;
-    bool loss_matches_m = false;   // us.loss == per-user losses of the scores in m (set by update_V's last trial)
 
     // ------------------------------------------------------------------ update_U(_new), batched over users
     double update_U() {
         require_ready();
-        if (v_trial_pending && !last_m_is_stale) {      // what update_V's last trial left behind, see there
-            scores(U, Vnew, m, nullptr);
-            if (cfg.solver == 2) prepare(m, nullptr);
-            user_losses(m, nullptr);
-            scores_valid = false; loss_matches_m = true; last_m_is_stale = true;
-        }
-        v_trial_pending = false;
-        if (!scores_valid && !last_m_is_stale) { scores(U, V, m, nullptr); scores_valid = true; meta_valid = false; loss_matches_m = false; }
-        if (cfg.solver == 2 && !meta_valid) prepare(m, nullptr);
+        // update_V rejected every trial and a read has replaced its scores since: rebuild that trial's state from (U, Vnew)
+        // -- the same kernels on the same inputs, so the same bits -- and consume it as if nothing had been read
+        if (held.v_trial_pending && held.m != MHolds::V_TRIAL) score_v_trial();
+        held.v_trial_pending = false;
+        if (held.m != MHolds::V_TRIAL) ensure_scores();
+        if (cfg.solver == 2 && !held.sorted) prepare(m, nullptr);
         // m holds scores(U, V) for every user (not the scores of a rejected V trial): then what the line search leaves
         // behind is valid for the next update_V (see there)
-        const bool m_covers_all_users = scores_valid && cfg.solver == 2;
+        const bool m_covers_all_users = held.m == MHolds::CURRENT && cfg.solver == 2;
         // gradient coefficients from m (stale m included, as precompute_ui / obtain_g_u do)
         coeffs(0, nullptr);
         // prev_obj: Primal-CR++ takes it from the same sorted state (objective_u_new :785); Primal-CR recomputes
         // the scores with the current (u_i, V) (compute_mm pcr.cpp:549), which differs only if V's search failed
-        if (cfg.solver == 1 && last_m_is_stale) {
+        if (cfg.solver == 1 && held.m == MHolds::V_TRIAL) {
             train_dots(U, V, b, nullptr);
             user_losses(b, nullptr);
-        } else if (!loss_matches_m) {
+        } else if (!held.losses) {
             user_losses(m, nullptr);      // else: us.loss still holds the losses of these very scores (last V trial)
         }
-        loss_matches_m = false;
         rowsum_users(U, us.g, nullptr, 1);
         zero_counters();
         k_u_init(ctx, us, U, X.row_ptr, cfg.solver == 1 ? has_pairs : nullptr, d1, ld, cfg.lambda);
@@ -886,8 +913,8 @@ struct Engine {
         k_u_commit(ctx, us, U, d1, ld);
         // Primal-CR++: every user that moved went through trial 0 at least, so m / the sorted state / us.loss are those
         // of its last trial = its committed row; users that were skipped kept their row and their entries.
-        scores_valid = m_covers_all_users; meta_valid = m_covers_all_users; loss_matches_m = m_covers_all_users;
-        last_m_is_stale = false;
+        held.m = m_covers_all_users ? MHolds::CURRENT : MHolds::NOTHING;
+        held.sorted = held.losses = m_covers_all_users;
         // now_obj = sum_i obj_u + lambda/2 ||V||^2   (pcrpp.cpp:832-836)
         k_sum(ctx, us.obj_new, d1, red_partials, slots + 0);
         k_dot(ctx, V, V, d2 * ld, red_partials, slots + 1);
@@ -910,18 +937,20 @@ struct Engine {
         zero_counters();
         k_u_init(ctx, us, U, X.row_ptr, cfg.solver == 1 ? has_pairs : nullptr, d1, ld, cfg.lambda);
     }
-    void hv_U_stage(const double *S_dev, double *out_dev) {
-        require_ready(); ensure_meta();
-        train_dots(S_dev, V, b, nullptr);
+    void hv_U_stage(const double *S) {     // of the host direction S [d1 x k] into us.Hp
+        require_ready(); PCR_REQUIRE(S != nullptr, "null direction");
+        put_matrix(S, d1, us.p);
+        ensure_meta();
+        train_dots(us.p, V, b, nullptr);
         coeffs(1, nullptr);
-        rowsum_users(S_dev, out_dev, nullptr, 0);
+        rowsum_users(us.p, us.Hp, nullptr, 0);
     }
 
     // ------------------------------------------------------------------ compute_pairwise_error_ndcg util.cpp:434-542
     // pair errors from the sorted state (O(len * T)) are possible for the training set of Primal-CR++ whenever the
     // sorted state of the CURRENT scores exists and the ratings are integers (levels == exact ratings), T <= 8
     bool eval_sorted_ok(int which) const {
-        return which == 0 && cfg.solver == 2 && scores_valid && meta_valid && ratings_integer && T <= 8;
+        return which == 0 && cfg.solver == 2 && held.m == MHolds::CURRENT && held.sorted && ratings_integer && T <= 8;
     }
     // method: -1 automatic, 0 all-pairs kernel (the reference's O(len^2) loop util.cpp:467-479), 1 sorted-state count
     void eval(int which, double *err, double *ndcg, int method = -1, i64 *err_user_host = nullptr, double *ndcg_user_host = nullptr) {
@@ -932,8 +961,8 @@ struct Engine {
         PCR_REQUIRE(method != 1 || eval_sorted_ok(which), "sorted-state evaluation needs the Primal-CR++ training set with integer ratings and <= 8 levels");
         const bool sorted = method == 1 || (method < 0 && eval_sorted_ok(which));
         double *sc = which == 0 ? b : ev_score_t;
-        if (which == 0 && scores_valid) sc = m;                      // m already holds U_i . V_j of the current factors
-        else if (which == 0) train_dots(U, V, sc, nullptr);           // user-major units kernel (2x the generic one)
+        if (which == 0 && held.m == MHolds::CURRENT) sc = m;    // m already holds U_i . V_j of the current factors
+        else if (which == 0) train_dots(U, V, sc, nullptr);     // user-major units kernel (2x the generic one)
         else k_dots(ctx, U, C.user, V, C.item, C.nnz, ld, k, nullptr, sc, 0.0);
         if (sorted) {       // pair errors AND NDCG@k of every user from the sorted state, one kernel
             k_eval_sorted(ctx, C, meta, T, ev_err_user, level_vals, cfg.ndcg_k, ev_a, ev_b, ev_c, ev_d);
@@ -1100,11 +1129,8 @@ int primalcr_comm_init(primalcr_engine *e, int rank, int world, const void *id12
 
 int primalcr_initial_objective(primalcr_engine *e, double *obj) {
     CHECK_E(e) API_BEGIN
-    Engine *E = e->impl;
-    E->require_ready();
-    E->scores_valid = false; E->meta_valid = false; E->v_trial_pending = false;
-    const double o = E->objective_current();
-    E->sync();
+    const double o = e->impl->initial_objective();
+    e->impl->sync();
     if (obj) *obj = o;
     API_END
 }
@@ -1182,8 +1208,7 @@ int primalcr_get_counters(primalcr_engine *e, primalcr_counters *out) {
 int primalcr_scores(primalcr_engine *e, double *m_out) {
     CHECK_E(e) API_BEGIN
     Engine *E = e->impl;
-    E->require_ready();
-    E->scores(E->U, E->V, E->m, nullptr); E->scores_valid = true; E->meta_valid = false; E->last_m_is_stale = false; E->loss_matches_m = false;
+    E->scores_stage();
     if (m_out && E->X.nnz) PCR_CUDA(cudaMemcpyAsync(m_out, E->m, sizeof(double) * (size_t)E->X.nnz, cudaMemcpyDeviceToHost, E->stream));
     E->sync();
     API_END
@@ -1191,12 +1216,7 @@ int primalcr_scores(primalcr_engine *e, double *m_out) {
 
 int primalcr_set_scores(primalcr_engine *e, const double *m) {
     CHECK_E(e) API_BEGIN
-    Engine *E = e->impl;
-    E->require_ready();
-    PCR_REQUIRE(m != nullptr || E->X.nnz == 0, "null scores");
-    if (E->X.nnz) PCR_CUDA(cudaMemcpyAsync(E->m, m, sizeof(double) * (size_t)E->X.nnz, cudaMemcpyHostToDevice, E->stream));
-    E->sync();
-    E->scores_valid = true; E->meta_valid = false; E->last_m_is_stale = false; E->loss_matches_m = false; E->v_trial_pending = false;
+    e->impl->load_scores(m);
     API_END
 }
 
@@ -1209,11 +1229,7 @@ int primalcr_sort_segments(primalcr_engine *e, double *sorted, int32_t *perm, in
                            int32_t *cnt_lo, int32_t *cnt_hi) {
     CHECK_E(e) API_BEGIN
     Engine *E = e->impl;
-    E->require_ready();
-    PCR_REQUIRE(E->cfg.solver == 2, "sorted state exists only for Primal-CR++");
-    E->ensure_scores();
-    E->prepare(E->m, nullptr);
-    E->ensure_heavy_windows();
+    E->sort_segments();
     E->sync();
     const size_t n = (size_t)E->X.nnz;
     if (n) {
@@ -1239,27 +1255,14 @@ int primalcr_sort_segments(primalcr_engine *e, double *sorted, int32_t *perm, in
 
 int primalcr_level_counts(primalcr_engine *e, int32_t *cnt_left, int32_t *cnt_right) {
     CHECK_E(e) API_BEGIN
-    Engine *E = e->impl;
-    E->require_ready();
-    PCR_REQUIRE(E->cfg.solver == 2, "sorted state exists only for Primal-CR++");
-    E->ensure_meta();
-    E->ensure_heavy_windows();
-    const size_t n = (size_t)E->X.nnz * E->T;
-    int32_t *dl = nullptr, *dr = nullptr;
-    dl = (int32_t *)E->pool.raw_alloc(sizeof(int32_t) * (n ? n : 1));
-    dr = (int32_t *)E->pool.raw_alloc(sizeof(int32_t) * (n ? n : 1));
-    pcr::k_level_counts(E->ctx, E->X.row_ptr, E->d1, E->meta, E->T, dl, dr);
-    E->sync();
-    if (n && cnt_left) PCR_CUDA(cudaMemcpy(cnt_left, dl, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
-    if (n && cnt_right) PCR_CUDA(cudaMemcpy(cnt_right, dr, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
-    E->pool.raw_free(dl); E->pool.raw_free(dr);
+    e->impl->level_counts(cnt_left, cnt_right);
     API_END
 }
 
 int primalcr_grad_V(primalcr_engine *e, double *g_out) {
     CHECK_E(e) API_BEGIN
     Engine *E = e->impl;
-    E->grad_V(E->g);
+    E->grad_V();
     if (g_out) E->get_matrix(E->g, E->d2, g_out);
     E->sync();
     API_END
@@ -1268,10 +1271,7 @@ int primalcr_grad_V(primalcr_engine *e, double *g_out) {
 int primalcr_hv_V(primalcr_engine *e, const double *a, double *Ha_out) {
     CHECK_E(e) API_BEGIN
     Engine *E = e->impl;
-    E->require_ready();
-    PCR_REQUIRE(a != nullptr, "null direction");
-    E->put_matrix(a, E->d2, E->p);
-    E->hv_V(E->p, E->Hp);
+    E->hv_V(a);
     if (Ha_out) E->get_matrix(E->Hp, E->d2, Ha_out);
     E->sync();
     API_END
@@ -1290,10 +1290,7 @@ int primalcr_grad_U(primalcr_engine *e, double *g_out, double *obj_u_out) {
 int primalcr_hv_U(primalcr_engine *e, const double *S, double *HS_out) {
     CHECK_E(e) API_BEGIN
     Engine *E = e->impl;
-    E->require_ready();
-    PCR_REQUIRE(S != nullptr, "null direction");
-    E->put_matrix(S, E->d1, E->us.p);
-    E->hv_U_stage(E->us.p, E->us.Hp);
+    E->hv_U_stage(S);
     if (HS_out) E->get_matrix(E->us.Hp, E->d1, HS_out);
     E->sync();
     API_END
